@@ -50,7 +50,17 @@ def parse_args():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--comm", choices=["auto", "ipc", "nccl"], default="auto",
                     help="exchange backend of the N > 1 ranks: CUDA IPC windows + shared-memory rendezvous (one box, NVLink), or NCCL send/recv")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float64): rounds (per round: round, n_in, "
+                         "parse_len, n_phrases, dict_syms, tot_phrases, n_pre_runs), the last level (last_rule_l, last_rule_r, last_has_hocc, "
+                         "last_pre_sym, last_pre_len) and final_parse; an array longer than 2^20 values is replaced by the values at the sorted "
+                         "positions numpy.random.default_rng(0).integers(0, length, 2^20)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
+    return args
 
 
 def c2_workload_desc(reads):
@@ -252,6 +262,34 @@ def split_range(total, world, rank):
     return first, per + (1 if rank < extra else 0)
 
 
+DUMP_VALUES = 1 << 20   # per array: the seven float64 arrays of --dump-outputs stay under 64 MB
+
+
+def dump_outputs(out_dir, ctx, rounds, final_cells, rank, world, dist, host_group):
+    """--dump-outputs: what the last step left in the context (the level of its last round and the final parse; N ranks: every rank's
+    part, in rank order) and the figures of its rounds. float64 holds every value exactly: the bench's texts are DNA, so symbols,
+    ranks and counts stay far below 2^53."""
+    import numpy as np
+    names = ("rule_l", "rule_r", "has_hocc", "pre_sym", "pre_len")
+    if world == 1:
+        level, parse = ctx.fetch_level(), ctx.fetch_parse()
+    else:
+        parts = [None] * world if rank == 0 else None
+        dist.gather_object((ctx.mg_fetch_slice(), ctx.fetch_parse_local(final_cells)), parts, dst=0, group=host_group)
+        if rank != 0:
+            return
+        level = {k: np.concatenate([p[0][k] for p in parts]) for k in names}
+        parse = np.concatenate([p[1] for p in parts])
+    keys = ("round", "n_in", "parse_len", "n_phrases", "dict_syms", "tot_phrases", "n_pre_runs")
+    arrays = {"rounds": np.array([[r[k] for k in keys] for r in rounds]), "final_parse": parse}
+    arrays.update({"last_" + k: level[k] for k in names})
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if a.size > DUMP_VALUES:
+            a = a[np.sort(np.random.default_rng(0).integers(0, a.size, DUMP_VALUES))]
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64))
+
+
 def run_ours(args, rank, world, local_rank):
     import hashlib
     import numpy as np
@@ -392,9 +430,10 @@ def run_ours(args, rank, world, local_rank):
     ci0 = comm.info() if comm is not None else None
     l0 = ctx.launch_count()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    last_rounds = []
     e0.record(stream)
-    for _ in range(args.steps):
-        step_resident()
+    for i in range(args.steps):
+        step_resident(last_rounds if args.dump_outputs and i == args.steps - 1 else None)
     e1.record(stream)
     barrier()
     launches = ctx.launch_count() - l0
@@ -414,6 +453,8 @@ def run_ours(args, rank, world, local_rank):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms_total = float(t.item())
     value = n_total * args.steps / 1e6 / (ms_total / 1e3)
+    if args.dump_outputs:   # before the e2e steps reuse the context
+        dump_outputs(args.dump_outputs, ctx, last_rounds, final_cells[0], rank, world, dist, host_group)
 
     # ---- e2e: host buffers through the C ABI (pinned text -> device; this rank's levels + final parse -> pinned host) ----
     e2e = None

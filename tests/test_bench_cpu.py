@@ -28,6 +28,12 @@ def test_reference_arm_other_ranks_exit_quietly():
     assert r.returncode == 0 and r.stdout.strip() == ""
 
 
+def test_bad_arguments_are_rejected():
+    for bad in (["--steps", "0"], ["--warmup", "-1"], ["--impl", "reference", "--dump-outputs", "out"]):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + bad, capture_output=True, text=True, cwd=ROOT, timeout=600)
+        assert r.returncode == 2 and bad[0] in r.stderr, (bad, r.stderr[-300:])
+
+
 def test_our_arm_refuses_to_run_without_a_device():
     import torch
     if torch.cuda.is_available():

@@ -1,6 +1,8 @@
 """CPU suite: the .rl_bwt consumer tools (grl2plain, grlbwt2rle, reverse_bwt, bwt_stats, split_runs) -- SURVEY.md 8(f)-4.
-Round trip text -> BWT (oracle) -> .rl_bwt -> reverse_bwt == text; parity with the reference's own scripts where they build
-without SDSL (oracle/_ref/*_ref, compiled from /root/reference/scripts by oracle/Makefile)."""
+Round trip text -> BWT (oracle) -> .rl_bwt -> reverse_bwt == text; parity with the reference's own scripts that build
+without SDSL, through their outputs stored in tests/golden/tools_golden.json."""
+import hashlib
+import json
 import os
 import subprocess
 
@@ -132,14 +134,13 @@ def test_rl_bwt_writer_matches_the_format(tmp_path, sb, fb):
 
 
 # ---------------------------------------------------------------- parity with the reference's scripts
-REF_DIR = os.path.join(G.ROOT if hasattr(G, "ROOT") else os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref")
+# what the reference's scripts produce on these files, stored by tests/golden/make_tools_golden.py
+with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "tools_golden.json")) as _f:
+    REF_OUT = json.load(_f)["cases"]
 
 
-def ref_tool(name):
-    path = os.path.join(REF_DIR, name + "_ref")
-    if not os.path.exists(path):
-        pytest.skip(f"{path} not built (needs /root/reference at build time)")
-    return path
+def sha256_file(path):
+    return hashlib.sha256(open(path, "rb").read()).hexdigest()
 
 
 def _bwt_file(all_cases, tmp_path, name):
@@ -150,6 +151,7 @@ def _bwt_file(all_cases, tmp_path, name):
     o.close()
     rl = tmp_path / f"{name}.rl_bwt"
     rl.write_bytes(O.rl_bwt_bytes(syms, lens, sb, fb))
+    assert sha256_file(rl) == REF_OUT[name]["rl_bwt_sha256"], name
     return rl, syms, lens, sb, fb
 
 
@@ -165,18 +167,17 @@ def _records(raw):
 def test_tools_match_the_reference_scripts(all_cases, tmp_path, name):
     """grl2plain and grlbwt2rle: the same bytes as scripts/grl2plain.cpp / grlbwt2rle.cpp; bwt_stats: the same report"""
     rl, syms, lens, sb, fb = _bwt_file(all_cases, tmp_path, name)
-    for ours, theirs, outs in (("grl2plain", "grl2plain", ["{}"]), ("grlbwt2rle", "grlbwt2rle", ["{}.syms", "{}.len"])):
-        a, b = tmp_path / ("ref_" + ours), tmp_path / ("our_" + ours)
-        r1 = subprocess.run([ref_tool(theirs), str(rl), str(a)], capture_output=True, text=True)
+    want = REF_OUT[name]
+    for ours, outs in (("grl2plain", {"{}": "grl2plain_sha256"}), ("grlbwt2rle", {"{}.syms": "grlbwt2rle_syms_sha256", "{}.len": "grlbwt2rle_len_sha256"})):
+        b = tmp_path / ("our_" + ours)
         r2 = subprocess.run([tool(ours), str(rl), str(b)], capture_output=True, text=True)
-        assert r1.returncode == 0 and r2.returncode == 0, (r1.stderr, r2.stderr)
-        for o_ in outs:
-            assert open(o_.format(a), "rb").read() == open(o_.format(b), "rb").read(), (ours, o_)
+        assert r2.returncode == 0, r2.stderr
+        for o_, key in outs.items():
+            assert sha256_file(o_.format(b)) == want[key], (ours, o_)
     if len(syms) >= 20:   # (the reference reads one past its sorted lengths when there are fewer than 10 runs)
-        r1 = subprocess.run([ref_tool("bwt_stats"), str(rl)], capture_output=True, text=True)
         r2 = subprocess.run([tool("bwt_stats"), str(rl)], capture_output=True, text=True)
-        want = r1.stdout.splitlines()
-        assert r2.stdout.splitlines()[: len(want)] == want
+        report = want["bwt_stats_report"]
+        assert r2.stdout.splitlines()[: len(report)] == report
 
 
 @pytest.mark.parametrize("name", ["rep_50x200k", "homopolymers_multi", "mixed_reads"])
@@ -202,14 +203,8 @@ def test_split_runs(all_cases, tmp_path, name):
             assert dist[:, 1].sum() == per_block.size == -(-n_syms // n)
             assert np.array_equal(np.bincount(per_block, minlength=dist.shape[0])[: dist.shape[0]], dist[:, 1].astype(np.int64))
         if n and n >= 64:   # the reference: asserts (or worse) on tiny blocks and on n = 0
-            ref_out = tmp_path / f"r_{bits}_{n}"
-            rr = subprocess.run([ref_tool("split_runs"), str(rl), str(bits), str(n), str(ref_out)], capture_output=True, text=True)
-            if rr.returncode == 0 and ref_out.exists():
-                rsb, rfb, s3, l3 = _records(ref_out.read_bytes())
-                keep = l3 > 0
-                assert (rsb, rfb) == (osb, ofb) and np.array_equal(s3[keep], s2) and np.array_equal(l3[keep], l2), (bits, n)
-                if keep.all():   # no zero-length records: the distribution files agree too
-                    assert open(str(ref_out) + ".dist").read() == open(str(out) + ".dist").read(), (bits, n)
+            ref = REF_OUT[name]["split_runs"][f"{bits}_{n}"]
+            assert sha256_file(out) == ref["sha256"] and sha256_file(str(out) + ".dist") == ref["dist_sha256"], (bits, n)
 
 
 def test_parse_rl_bwt_helper(tmp_path):
