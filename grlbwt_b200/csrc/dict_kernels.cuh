@@ -375,50 +375,29 @@ static __global__ void __launch_bounds__(256) pack_ginfo_dense_kernel(const u32*
 // metasymbol of every whole phrase (exact_par_phase.cpp:174-176, :437-444) and is_suffix of the next round (:443): a group
 // of equal suffixes holds at most one whole phrase, whose destination group_reduce left in gfull
 static __global__ void __launch_bounds__(256) full_apply_kernel(const u32* __restrict__ gcnt, const u32* __restrict__ rflag, const u32* __restrict__ rrank,
-                                                                const u64* __restrict__ gfull, u64 G, u64 rank_base, ulonglong2* table, u64* __restrict__ ph_meta,
-                                                                u8* __restrict__ is_suffix_next) {
+                                                                const u64* __restrict__ gfull, u64 G, ulonglong2* table, u8* __restrict__ is_suffix_next) {
     const u64 g = (u64)blockIdx.x * blockDim.x + threadIdx.x;
     if (g >= G || !rflag[g] || !(gcnt[g] >> 31)) return;
-    const u64 r = (u64)rrank[g] + rank_base, f = gfull[g];
-    const u64 meta = (r << 1) | (f & 1ULL);
-    if (ph_meta) ph_meta[f >> 2] = meta;  // multi-GPU: the dictionary is global, the tables are per rank
-    else table[f >> 2].y = meta;
+    const u64 r = rrank[g], f = gfull[g];
+    table[f >> 2].y = (r << 1) | (f & 1ULL);
     is_suffix_next[r] = (u8)((f >> 1) & 1ULL);
 }
 // rank marks of the entries of hocc groups (phr_marks + new_phrases_ht, :190-207), pass in sorted order
 static __global__ void __launch_bounds__(256) group_apply_kernel(const u32* __restrict__ order, const u32* __restrict__ head_bits, const u32* __restrict__ head_pref,
-                                                                 const u32* __restrict__ ginfo, u64 nE, u64 rank_base, u32 erank_bias, u32* __restrict__ erank) {
+                                                                 const u32* __restrict__ ginfo, u64 nE, u32* __restrict__ erank) {
     const u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= nE) return;
     const u32 hw = head_bits[i >> 5];
     const u32 g = head_pref[i >> 5] + __popc(hw & (0xffffffffu >> (31 - (i & 31)))) - 1;
     const u32 gi = ginfo[g];
     if ((gi & 3u) != 3u) return;  // only ranked groups with more than one entry
-    erank[order[i]] = (u32)((u64)(gi >> 2) + rank_base) + erank_bias;  // bias 1 in distributed rounds (0 = none, merged by all-reduce MAX)
+    erank[order[i]] = gi >> 2;
 }
 
 // ---- distributed ranking: every rank owns the suffix entries whose first key falls in its range [lo, hi) ----
 static __global__ void __launch_bounds__(256) key_sample_kernel(const u64* __restrict__ keys, u64 n, u64 stride, u64 n_samples, u64* __restrict__ out, u32* __restrict__ vals) {
     const u64 s = (u64)blockIdx.x * blockDim.x + threadIdx.x;
     if (s < n_samples) { const u64 i = s * stride; out[s] = keys[i < n ? i : n - 1]; vals[s] = (u32)s; }
-}
-static __global__ void __launch_bounds__(256) key_range_flags_kernel(const u64* __restrict__ keys, u64 n, u64 lo, u64 hi, int hi_open, u32* __restrict__ flags) {
-    const u64 e = (u64)blockIdx.x * blockDim.x + threadIdx.x;
-    if (e < n) flags[e] = (keys[e] >= lo && (hi_open || keys[e] < hi)) ? 1u : 0u;
-}
-static __global__ void __launch_bounds__(256) key_range_compact_kernel(const u64* __restrict__ keys, const u32* __restrict__ vals, const u32* __restrict__ flags,
-                                                                       const u32* __restrict__ excl, u64 n, u64* __restrict__ okeys, u32* __restrict__ ovals) {
-    const u64 e = (u64)blockIdx.x * blockDim.x + threadIdx.x;
-    if (e < n && flags[e]) { okeys[excl[e]] = keys[e]; ovals[excl[e]] = vals[e]; }
-}
-// hocc marks travel between ranks as rank+1 (0 = none) so that an all-reduce(MAX) merges them; decode in place
-static __global__ void __launch_bounds__(256) erank_decode_kernel(u32* __restrict__ erank, u64 n) {
-    const u64 e = (u64)blockIdx.x * blockDim.x + threadIdx.x;
-    if (e < n) erank[e] = erank[e] ? erank[e] - 1 : 0xffffffffu;
-}
-static __global__ void __launch_bounds__(256) u8_to_u64max_kernel(const u64* __restrict__ in, u64 n, u8* __restrict__ out) {
-    const u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) out[i] = in[i] ? 1 : 0;
 }
 
 static __global__ void __launch_bounds__(256) popc_words_kernel(const u32* __restrict__ bits, u64 n_words, u32* __restrict__ cnt) {

@@ -178,10 +178,6 @@ static __global__ void adjacent_max_diff_kernel(const u64* __restrict__ ptrs, u6
     m = warp_max(m);
     if (lane_id() == 0 && m) atomicMax(out, m);
 }
-static __global__ void fill_u32_kernel(u32* __restrict__ p, u64 n, u32 v) {
-    const u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) p[i] = v;
-}
 static __global__ void u32_to_u64_kernel(const u32* __restrict__ in, u64 n, u64* __restrict__ out) {
     const u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) out[i] = in[i];
@@ -208,8 +204,7 @@ struct Round {
     u64 nS = 0;
     DevBuf<u64> keys;
     DevBuf<u32> vals;
-    const void* dict_text = nullptr;  // text the dictionary's ph_pos point into (default: the context's text)
-    u64* ph_meta = nullptr;           // if set, metasymbols go here (per phrase) instead of into the table
+    const void* dict_text = nullptr;  // multi-GPU partition: the received phrase cells its ph_pos point into
     explicit Round(grlgpu_ctx* ctx) : c(ctx), st(ctx->st), n(ctx->n) {}
 };
 
@@ -394,22 +389,22 @@ void dict_offsets(Round& R) {
 }
 
 template <class CellT, bool FIRST, class SymT>
-void stage_gather(Round& R, bool force_ext = false) {
+void stage_gather(Round& R) {
     grlgpu_ctx* c = R.c;
     R.sym_bits = bit_width64(c->alphabet + 1);
     R.K = std::max(1, 64 / R.sym_bits);
     // refinement by key extension needs ceil((longest phrase + 1) / K) passes at most; beyond 64 passes (or when a test
     // forces it) the groups are refined by prefix doubling on position-based ranks instead
-    R.ext_mode = force_ext || (!(c->flags & GRLGPU_FLAG_FORCE_DOUBLING) && (R.max_len + 1 + (u64)R.K - 1) / (u64)R.K <= 64);
+    R.ext_mode = !(c->flags & GRLGPU_FLAG_FORCE_DOUBLING) && (R.max_len + 1 + (u64)R.K - 1) / (u64)R.K <= 64;
     R.spare = (R.ext_mode && R.sym_bits * R.K < 64) ? 64 - R.sym_bits * R.K : 0;
-    const CellT* dtext = (const CellT*)(R.dict_text ? R.dict_text : c->text);
+    const CellT* text = (const CellT*)c->text;
     DevBuf<u32> voff;
     R.nS = R.nE;
     if (R.ext_mode) {
         voff.alloc(R.d + 1, R.st);
         DevBuf<u32> tot(1, R.st);
         IsSuffix isuf0{c->is_suffix.p, c->sep, c->first};
-        GRL_LAUNCH("phrase_vlen", R.d * 48, (phrase_vlen_kernel<CellT, FIRST>), grid_for(R.d, 256), 256, 0, R.st, dtext, R.ph_pos.p, R.ph_len.p, R.d, isuf0, voff.p);
+        GRL_LAUNCH("phrase_vlen", R.d * 48, (phrase_vlen_kernel<CellT, FIRST>), grid_for(R.d, 256), 256, 0, R.st, text, R.ph_pos.p, R.ph_len.p, R.d, isuf0, voff.p);
         exclusive_scan<u32, u32>(voff.p, voff.p, R.d, voff.p + R.d, R.st);
         R.nS = d2h_scalar(voff.p + R.d, R.st);
         R.keys.alloc(R.nS, R.st);
@@ -420,31 +415,24 @@ void stage_gather(Round& R, bool force_ext = false) {
     R.rem.alloc(R.nE, R.st);
     R.einfo.alloc(R.nE, R.st);
     IsSuffix isuf{R.c->is_suffix.p, R.c->sep, R.c->first};
-    // metasymbols go to the phrase's table slot, or to the global per-phrase array in multi-GPU rounds
-    GRL_LAUNCH("dict_gather", R.nE * (sizeof(CellT) + sizeof(SymT) + 20) + R.nS * 12 + R.d * 32, (dict_gather_kernel<CellT, FIRST, SymT>), grid_for(R.d, 256), 256, 0, R.st, dtext,
-               R.ph_pos.p, R.ph_len.p, R.ph_off.p, R.ph_freq.p, R.ph_meta ? (const u32*)nullptr : (const u32*)R.occ_slots.p, R.d, isuf, (SymT*)R.D_raw.p, R.phr_of.p, R.rem.p,
+    // metasymbols go to the phrase's table slot
+    GRL_LAUNCH("dict_gather", R.nE * (sizeof(CellT) + sizeof(SymT) + 20) + R.nS * 12 + R.d * 32, (dict_gather_kernel<CellT, FIRST, SymT>), grid_for(R.d, 256), 256, 0, R.st, text,
+               R.ph_pos.p, R.ph_len.p, R.ph_off.p, R.ph_freq.p, R.occ_slots.p, R.d, isuf, (SymT*)R.D_raw.p, R.phr_of.p, R.rem.p,
                R.einfo.p, (const u32*)voff.p, c->alphabet + 1, R.sym_bits, R.K, R.spare, R.keys.p, R.vals.p);
 }
 
 // One refinement depth of the suffix order: the active elements (slot j: extension key nk[j], gflag[j] = first of its group)
 // are sorted by key inside their groups. -> perm[q] = active index of the element that belongs at slot q, flags[q] = 1 where
 // a new (sub)group starts. Tile-local segmented sort for the groups that fit a window; the flagged rest goes through two
-// device-wide radix sorts (by key, then stably by group), as every element did before.
+// device-wide radix sorts (by key, then stably by group).
 void refine_sort_groups(cudaStream_t st, const u64* nk, const u32* gflag, u64 nA, int key_bits, DevBuf<u32>& perm, DevBuf<u32>& flags) {
     perm.alloc(nA, st);
     flags.alloc(nA, st);
     if (nA == 0) return;
-    const bool local = getenv("GRL_NO_LOCAL_SORT") == nullptr;
     DevBuf<u32> lflag(nA, st), lexcl(nA, st), cnt(1, st);
-    u64 nLft = nA;
-    if (local) {
-        GRL_LAUNCH("ext_local_sort", nA * 24, ext_local_sort_kernel, (unsigned)div_up(nA, LS_WIN), LS_THREADS, 0, st, nk, gflag, nA, perm.p, flags.p, lflag.p);
-        exclusive_scan<u32, u32>(lflag.p, lexcl.p, nA, cnt.p, st);
-        nLft = d2h_scalar(cnt.p, st);
-    } else {
-        GRL_LAUNCH("fill_ones", nA * 4, fill_u32_kernel, grid_for(nA, 256), 256, 0, st, lflag.p, nA, 1u);
-        exclusive_scan<u32, u32>(lflag.p, lexcl.p, nA, cnt.p, st);
-    }
+    GRL_LAUNCH("ext_local_sort", nA * 24, ext_local_sort_kernel, (unsigned)div_up(nA, LS_WIN), LS_THREADS, 0, st, nk, gflag, nA, perm.p, flags.p, lflag.p);
+    exclusive_scan<u32, u32>(lflag.p, lexcl.p, nA, cnt.p, st);
+    const u64 nLft = d2h_scalar(cnt.p, st);
     if (getenv("GRLGPU_TRACE")) fprintf(stderr, "[grlgpu]   refine sort: %llu active, %llu through the device-wide path\n", nA, nLft);
     if (nLft == 0) return;
     DevBuf<u32> lpos(nLft, st), lv(nLft, st), lv_alt(nLft, st), lg(nLft, st), gexcl(nLft, st), lf(nLft, st);
@@ -628,12 +616,12 @@ void stage_dict(Round& R) {
     is_suffix_next.zero();
     DevBuf<u32> erank(nE, st);
     erank.fill_ff();
-    GRL_LAUNCH("full_apply", G * 20 + R.d * 40, full_apply_kernel, grid_for(G, 256), 256, 0, st, gcnt.p, rflag.p, rrank.p, gfull.p, G, (u64)0, R.table.p, R.ph_meta, is_suffix_next.p);
+    GRL_LAUNCH("full_apply", G * 20 + R.d * 40, full_apply_kernel, grid_for(G, 256), 256, 0, st, gcnt.p, rflag.p, rrank.p, gfull.p, G, R.table.p, is_suffix_next.p);
     gfull.release();
     if (ext_mode) {  // hocc marks in sorted order: group info is read sequentially, entries need no rank of their own
         DevBuf<u32> ginfo(G, st);
         GRL_LAUNCH("pack_ginfo_dense", G * 16, pack_ginfo_dense_kernel, grid_for(G, 256), 256, 0, st, gcnt.p, rflag.p, rrank.p, G, ginfo.p);
-        GRL_LAUNCH("group_apply", nS * 12, group_apply_kernel, grid_for(nS, 256), 256, 0, st, order, head_bits.p, head_pref.p, ginfo.p, nS, (u64)0, 0u, erank.p);
+        GRL_LAUNCH("group_apply", nS * 12, group_apply_kernel, grid_for(nS, 256), 256, 0, st, order, head_bits.p, head_pref.p, ginfo.p, nS, erank.p);
     } else {
         DevBuf<u32> ginfo(nE, st);  // indexed by head position
         GRL_LAUNCH("pack_ginfo", G * 20, pack_ginfo_kernel, grid_for(G, 256), 256, 0, st, gcnt.p, rflag.p, rrank.p, ghead.p, G, ginfo.p);
@@ -649,8 +637,8 @@ void stage_dict(Round& R) {
     c->lvl_tot = tot;
     c->lvl_npre = R.n_pre;
     // every valid dictionary entry contributes its phrase's frequency to exactly one run: the lengths of a level sum to at most
-    // n + p (phrases overlap by one cell). Multi-GPU: the frequencies are global, the local sizes bound nothing.
-    c->lvl_n_in = R.ph_meta ? ~0ull : R.n + R.p;
+    // n + p (phrases overlap by one cell)
+    c->lvl_n_in = R.n + R.p;
 
     if (c->flags & GRLGPU_FLAG_KEEP_DICT) {
         c->kd_d = R.d; c->kd_nE = nE; c->kd_nS = nS;
@@ -706,7 +694,7 @@ void finish_round(grlgpu_ctx* c, Round& R, u64 tot, u64 n_pre, u64 dict_d, u64 d
     out->dict_ms = tm.dict;
     out->rewrite_ms = t_rw.ms();
 
-    if ((c->flags & GRLGPU_FLAG_KEEP_DICT) && !R.ph_meta && c->kd_meta.p) {  // metasymbol per distinct phrase, for tests
+    if ((c->flags & GRLGPU_FLAG_KEEP_DICT) && c->kd_meta.p) {  // metasymbol per distinct phrase, for tests
         std::vector<u32> slots(R.d);
         GRL_CUDA(cudaMemcpy(slots.data(), R.occ_slots.p, R.d * 4, cudaMemcpyDeviceToHost));
         std::vector<ulonglong2> tab(R.cap);

@@ -251,7 +251,7 @@ static __global__ void lms_resolve_kernel(const u8* __restrict__ block_state, u8
 // min(len, LEN_SAT), count}; a key is claimed with one 64-bit CAS and is immediately complete because it
 // points into the immutable text.
 //
-// dedup_kernel is the fused text pass: persistent CTAs walk tiles of 8192 cells staged in shared memory
+// dedup_cached_kernel is the fused text pass: persistent CTAs walk 32 KB tiles of cells staged in shared memory
 // (cells + look-ahead halo, start/end bitmap words); a thread owns one bitmap word, numbers its phrases
 // from the tile's scanned base and, for phrases of at most 15 bytes, packs the cells into a 128-bit key
 // and looks it up in a per-CTA shared-memory cache of hot phrases (key -> global slot, local count).
@@ -292,10 +292,10 @@ __device__ __forceinline__ u64 phrase_hash(const CellT* __restrict__ text, u64 s
     return mix64(h);
 }
 
-// global path: probes `table` (whose keys point into ttext) for the phrase qtext[s, s+len). INSERT: claims a
-// slot if the phrase is new (then qtext must be ttext) and adds `add` to its count; returns the slot, or
-// HT_OVERFLOW when the probe limit is hit (insert) / the phrase is absent (find).
-template <class CellT, bool INSERT>
+// global path: probes `table` (whose keys point into ttext) for the phrase qtext[s, s+len), claims a slot if the
+// phrase is new (then qtext must be ttext) and adds `add` to its count; returns the slot, or HT_OVERFLOW when the
+// probe limit is hit.
+template <class CellT>
 __device__ u32 table_probe(const CellT* __restrict__ qtext, u64 s, u64 len, const CellT* __restrict__ ttext, ulonglong2* table, u64 cap, u64 add,
                            const u32* __restrict__ start_bits, const u32* __restrict__ end_bits, u64 n, u32* overflow) {
     const u64 lenf = len < HT_LEN_SAT ? len : HT_LEN_SAT;
@@ -304,11 +304,10 @@ __device__ u32 table_probe(const CellT* __restrict__ qtext, u64 s, u64 len, cons
     for (int probes = 0; probes < HT_MAX_PROBES; probes++) {
         u64 k = *reinterpret_cast<volatile u64*>(&table[slot].x);
         if (k == HT_EMPTY) {
-            if (!INSERT) return HT_OVERFLOW;
             const u64 old = atomicCAS(&table[slot].x, HT_EMPTY, mykey);
             k = old == HT_EMPTY ? mykey : old;
         }
-        bool match = INSERT && k == mykey;
+        bool match = k == mykey;
         if (!match && (k & HT_LEN_SAT) == lenf) {
             const u64 kpos = k >> 24;
             match = true;
@@ -317,18 +316,18 @@ __device__ u32 table_probe(const CellT* __restrict__ qtext, u64 s, u64 len, cons
             if (match && lenf == HT_LEN_SAT) match = start_bits != nullptr && phrase_len_bits(start_bits, end_bits, n, kpos) == len;
         }
         if (match) {
-            if (INSERT) atomicAdd(&table[slot].y, add);
+            atomicAdd(&table[slot].y, add);
             return (u32)slot;
         }
         if (++slot == cap) slot = 0;
     }
-    if (INSERT) atomicExch(overflow, 1u);
+    atomicExch(overflow, 1u);
     return HT_OVERFLOW;
 }
 template <class CellT>
 __device__ __forceinline__ u32 table_insert_global(const CellT* __restrict__ text, u64 s, u64 len, ulonglong2* table, u64 cap, const u32* __restrict__ start_bits,
                                                    const u32* __restrict__ end_bits, u64 n, u32* overflow) {
-    return table_probe<CellT, true>(text, s, len, text, table, cap, 1ULL, start_bits, end_bits, n, overflow);
+    return table_probe<CellT>(text, s, len, text, table, cap, 1ULL, start_bits, end_bits, n, overflow);
 }
 
 // ---- thread-per-phrase variant over a compacted start array (unique-heavy rounds: maximum memory-level parallelism) ----
@@ -603,31 +602,6 @@ static __global__ void gather_u32_kernel(const u32* __restrict__ src, const u32*
     const u64 k = (u64)blockIdx.x * blockDim.x + threadIdx.x;
     if (k < m) dst[k] = src[perm[k]];
 }
-// first[g] = number of sorted keys < g, for g = 0..n_ranks
-static __global__ void owner_bounds_kernel(const u64* __restrict__ keys, u64 m, u32 n_ranks, u64* __restrict__ first) {
-    const u32 g = threadIdx.x;
-    if (g > n_ranks) return;
-    u64 lo = 0, hi = m;
-    while (lo < hi) {
-        const u64 mid = (lo + hi) >> 1;
-        if (keys[mid] < g) lo = mid + 1; else hi = mid;
-    }
-    first[g] = lo;
-}
-// out[k] = phrase perm[k] (or k) of (src_text, ph_pos, ph_len, ph_cnt); cells at offs[k]
-template <class CellT>
-__global__ void __launch_bounds__(256) pack_phrases_kernel(const CellT* __restrict__ src_text, const u64* __restrict__ ph_pos, const u32* __restrict__ ph_len,
-                                                           const u64* __restrict__ ph_cnt, const u32* __restrict__ perm, const u64* __restrict__ offs, u64 m,
-                                                           u32* __restrict__ out_lens, u64* __restrict__ out_counts, CellT* __restrict__ out_cells) {
-    const u64 k = (u64)blockIdx.x * blockDim.x + threadIdx.x;
-    if (k >= m) return;
-    const u32 i = perm ? perm[k] : (u32)k;
-    const u32 len = ph_len[i];
-    const u64 pos = ph_pos[i], o = offs[k];
-    out_lens[k] = len;
-    out_counts[k] = ph_cnt[i];
-    for (u32 t = 0; t < len; t++) out_cells[o + t] = src_text[pos + t];
-}
 // dedup of a pack into a table whose keys point into the pack's own cells; count += counts[k] (or the index k when counts == nullptr)
 template <class CellT>
 __global__ void __launch_bounds__(256) pack_insert_kernel(const CellT* __restrict__ cells, const u64* __restrict__ offs, const u32* __restrict__ lens,
@@ -636,7 +610,7 @@ __global__ void __launch_bounds__(256) pack_insert_kernel(const CellT* __restric
     const u64 k = (u64)blockIdx.x * blockDim.x + threadIdx.x;
     if (k >= m) return;
     if (*reinterpret_cast<volatile u32*>(overflow)) return;
-    const u32 slot = table_probe<CellT, true>(cells, offs[k], lens[k], cells, table, cap, counts ? counts[k] : k, nullptr, nullptr, 0, overflow);
+    const u32 slot = table_probe<CellT>(cells, offs[k], lens[k], cells, table, cap, counts ? counts[k] : k, nullptr, nullptr, 0, overflow);
     if (slot_out) slot_out[k] = slot;
 }
 // owner side of the metasymbol return: dense partition index of every table slot, then of every received phrase
@@ -657,17 +631,6 @@ static __global__ void __launch_bounds__(256) apply_reply_kernel(const u32* __re
                                                                  ulonglong2* ltable) {
     const u64 k = (u64)blockIdx.x * blockDim.x + threadIdx.x;
     if (k < d) ltable[occ_slots[perm[k]]].y = local_meta[k];
-}
-// metasymbol of every local distinct phrase: look its cells up in the global dictionary's table
-template <class CellT>
-__global__ void __launch_bounds__(256) map_local_kernel(const CellT* __restrict__ text, const u64* __restrict__ ph_pos, const u32* __restrict__ ph_len,
-                                                        const u32* __restrict__ occ_slots, u64 d, const CellT* __restrict__ gcells, ulonglong2* gtable,
-                                                        u64 gcap, const u64* __restrict__ g_meta, ulonglong2* ltable, u32* missing) {
-    const u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= d) return;
-    const u32 gs = table_probe<CellT, false>(text, ph_pos[i], ph_len[i], gcells, gtable, gcap, 0, nullptr, nullptr, 0, nullptr);
-    if (gs == HT_OVERFLOW) { atomicExch(missing, 1u); return; }
-    ltable[occ_slots[i]].y = g_meta[gtable[gs].y];
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -1,6 +1,6 @@
 // Device-wide building blocks written for this path: exclusive scan, bitmap -> position compaction,
-// LSD radix sort of (u64 key, u32 value) pairs, max-reduction. All are plain multi-kernel
-// formulations (no inter-CTA spin waits), HBM-bound, grid sized from the data.
+// LSD radix sort of (u64 or u32 key, u32 value) pairs and its one-digit partition, max-reduction.
+// All are plain multi-kernel formulations (no inter-CTA spin waits), HBM-bound, grid sized from the data.
 #pragma once
 #include "util.cuh"
 
@@ -237,12 +237,13 @@ struct BitmapCompactor {
 };
 
 // ------------------------------------------------------------------------------------------------
-// LSD radix sort of (u64 key, u32 value) pairs on key bits [0, n_bits), 8 bits per pass, stable.
+// LSD radix sort of (u64 or u32 key, u32 value) pairs on key bits [0, n_bits), 8 bits per pass, stable.
 // Per pass: per-tile digit histogram -> exclusive scan of the digit-major table -> ranked scatter
 // through shared memory (writes of one digit from one tile are contiguous).
 // ------------------------------------------------------------------------------------------------
 constexpr int RS_THREADS = 256;
 constexpr int RS_WARPS = RS_THREADS / 32;
+constexpr int RS_ITEMS = 8;  // items per thread: 59 registers, 4 CTAs/SM (measured best on B200 against 4, 12 and 16)
 template <class KeyT, int ITEMS>
 constexpr size_t rs_smem_bytes() {
     return (size_t)RS_THREADS * ITEMS * (sizeof(KeyT) + sizeof(u32)) + (size_t)RS_WARPS * 257 * sizeof(u32) + 2 * 256 * sizeof(u32) + 34 * sizeof(u32);
@@ -269,8 +270,8 @@ __global__ void __launch_bounds__(RS_THREADS) radix_hist_kernel(const KeyT* __re
     hist[(u64)threadIdx.x * tiles + blockIdx.x] = cnt[threadIdx.x];
 }
 
-template <class KeyT, int ITEMS, int MINB>
-__global__ void __launch_bounds__(RS_THREADS, MINB) radix_scatter_kernel(const KeyT* __restrict__ keys_in, const u32* __restrict__ vals_in, KeyT* __restrict__ keys_out,
+template <class KeyT, int ITEMS>
+__global__ void __launch_bounds__(RS_THREADS, 4) radix_scatter_kernel(const KeyT* __restrict__ keys_in, const u32* __restrict__ vals_in, KeyT* __restrict__ keys_out,
                                                                    u32* __restrict__ vals_out, u64 n, int shift, const u64* __restrict__ goff, u64 tiles) {
     constexpr int TILE = RS_THREADS * ITEMS, WARP_ITEMS = TILE / RS_WARPS;
     extern __shared__ __align__(16) unsigned char rs_smem[];
@@ -341,363 +342,42 @@ __global__ void __launch_bounds__(RS_THREADS, MINB) radix_scatter_kernel(const K
     }
 }
 
-// Pipelined variant: persistent CTAs; the NEXT tile of a CTA streams into shared memory with 16-byte cp.async copies while
-// the current one is ranked, permuted and written out, so every resident CTA always has a tile of loads in flight
-// (the one-tile-per-CTA kernel above is load-latency-bound: all warps of a CTA wait for the same loads). The input
-// buffer of a tile doubles as its sorted staging area once the items sit in registers: two buffers per CTA.
-template <class KeyT, int ITEMS>
-constexpr size_t rsp_smem_bytes() {
-    return 2 * (size_t)RS_THREADS * ITEMS * (sizeof(KeyT) + sizeof(u32)) + (size_t)RS_WARPS * 257 * sizeof(u32) + 256 * sizeof(u64) + 256 * sizeof(u32) + 34 * sizeof(u32);
-}
-__device__ __forceinline__ void cp_async16(void* smem_dst, const void* gsrc, u32 src_bytes) {
-    const u32 d = (u32)__cvta_generic_to_shared(smem_dst);
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;\n" ::"r"(d), "l"(gsrc), "r"(src_bytes) : "memory");
-}
-template <class T, int TILE>
-__device__ __forceinline__ void rsp_prefetch(T* sdst, const T* __restrict__ gsrc, u64 base, u64 n) {
-    constexpr int PER = 16 / sizeof(T), CHUNKS = TILE / PER;
-    const u64 left = n - base;  // items of this tile that exist (>= 1)
-    for (int c = threadIdx.x; c < CHUNKS; c += RS_THREADS) {
-        const u64 first = (u64)c * PER;
-        const u32 bytes = first >= left ? 0u : (left - first >= (u64)PER ? 16u : (u32)((left - first) * sizeof(T)));
-        cp_async16(sdst + first, gsrc + (bytes ? base + first : base), bytes);  // missing bytes are zero-filled
-    }
-}
-template <class KeyT, int ITEMS>
-__global__ void __launch_bounds__(RS_THREADS) radix_scatter_pipe_kernel(const KeyT* __restrict__ keys_in, const u32* __restrict__ vals_in, KeyT* __restrict__ keys_out,
-                                                                        u32* __restrict__ vals_out, u64 n, int shift, const u64* __restrict__ goff, u64 tiles) {
-    constexpr int TILE = RS_THREADS * ITEMS, WARP_ITEMS = TILE / RS_WARPS;
-    constexpr size_t BUF = (size_t)TILE * (sizeof(KeyT) + sizeof(u32));
-    extern __shared__ __align__(16) unsigned char rs_smem[];
-    u32* s_cnt = (u32*)(rs_smem + 2 * BUF);                 // [RS_WARPS][257]
-    u64* s_delta = (u64*)(s_cnt + RS_WARPS * 257);          // [256] global offset of digit d minus its tile-local start (8 * 257 words: 8-byte aligned)
-    u32* s_dstart = (u32*)(s_delta + 256);                  // [256]
-    u32* s_scan = s_dstart + 256;                           // 33 scratch
-
-    const u32 lane = lane_id(), warp = threadIdx.x >> 5;
-    u32* wc = s_cnt + warp * 257;
-    u64 tile = blockIdx.x;
-    if (tile >= tiles) return;
-    rsp_prefetch<KeyT, TILE>((KeyT*)rs_smem, keys_in, tile * TILE, n);
-    rsp_prefetch<u32, TILE>((u32*)(rs_smem + (size_t)TILE * sizeof(KeyT)), vals_in, tile * TILE, n);
-    asm volatile("cp.async.commit_group;\n" ::: "memory");
-    for (u32 it = 0; tile < tiles; tile += gridDim.x, it ^= 1u) {
-        KeyT* s_keys = (KeyT*)(rs_smem + it * BUF);
-        u32* s_vals = (u32*)(s_keys + TILE);
-        for (int i = threadIdx.x; i < RS_WARPS * 257; i += RS_THREADS) s_cnt[i] = 0;
-        const u64 my_goff = goff[(u64)threadIdx.x * tiles + tile];
-        asm volatile("cp.async.wait_group 0;\n" ::: "memory");
-        __syncthreads();  // this tile has landed; everyone is done with the other buffer (output of the previous tile)
-        const u64 next = tile + gridDim.x;
-        if (next < tiles) {
-            unsigned char* nb = rs_smem + (it ^ 1u) * BUF;
-            rsp_prefetch<KeyT, TILE>((KeyT*)nb, keys_in, next * TILE, n);
-            rsp_prefetch<u32, TILE>((u32*)(nb + (size_t)TILE * sizeof(KeyT)), vals_in, next * TILE, n);
-        }
-        asm volatile("cp.async.commit_group;\n" ::: "memory");
-
-        const u64 tile_base = tile * TILE;
-        KeyT key[ITEMS];
-        u32 val[ITEMS];
-        u32 rnk[ITEMS];
-#pragma unroll
-        for (int r = 0; r < ITEMS; r++) {
-            const u32 li = warp * WARP_ITEMS + r * 32 + lane;
-            const bool ok = tile_base + li < n;
-            key[r] = s_keys[li];
-            val[r] = s_vals[li];
-            const u32 d = ok ? ((u32)(key[r] >> shift) & 255u) : 256u;
-            const u32 m = __match_any_sync(0xffffffffu, d);
-            const u32 b = wc[d];
-            __syncwarp();
-            if (lane == (u32)(__ffs(m) - 1)) wc[d] = b + __popc(m);
-            __syncwarp();
-            rnk[r] = b + __popc(m & lanemask_lt());
-        }
-        __syncthreads();  // items sit in registers: the buffer is free to become the sorted staging area
-        {
-            const u32 d = threadIdx.x;
-            u32 run = 0;
-#pragma unroll
-            for (int w = 0; w < RS_WARPS; w++) {
-                const u32 t = s_cnt[w * 257 + d];
-                s_cnt[w * 257 + d] = run;
-                run += t;
-            }
-            u32 tot;
-            const u32 ex = block_exclusive_sum<u32>(run, s_scan, tot);
-            s_dstart[d] = ex;
-            s_delta[d] = my_goff - ex;
-        }
-        __syncthreads();
-#pragma unroll
-        for (int r = 0; r < ITEMS; r++) {
-            const u32 li = warp * WARP_ITEMS + r * 32 + lane;
-            if (tile_base + li < n) {
-                const u32 d = (u32)(key[r] >> shift) & 255u;
-                const u32 pos = s_dstart[d] + wc[d] + rnk[r];
-                s_keys[pos] = key[r];
-                s_vals[pos] = val[r];
-            }
-        }
-        __syncthreads();
-        const u64 rem = n - tile_base;
-        const u32 valid = rem < (u64)TILE ? (u32)rem : (u32)TILE;
-        for (u32 i = threadIdx.x; i < valid; i += RS_THREADS) {
-            const KeyT k = s_keys[i];
-            const u32 d = (u32)(k >> shift) & 255u;
-            const u64 g = s_delta[d] + i;
-            keys_out[g] = k;
-            vals_out[g] = s_vals[i];
-        }
-    }
-}
-inline int rs_pipe_setting() {  // measured on B200: the pipelined variant is slower (2.4 vs 3.5 TB/s), the shared-memory pipe is what binds
-    static int v = -1;
-    if (v < 0) { const char* e = getenv("GRL_RS_PIPE"); v = e ? atoi(e) : 0; }
-    return v;
-}
-inline int rs_minb_setting() {
-    static int v = -1;
-    if (v < 0) { const char* e = getenv("GRL_RS_MINB"); v = e ? atoi(e) : 1; }
-    return v;
-}
-
-// ------------------------------------------------------------------------------------------------
-// One-sweep variant of the LSD pass (after Adinets & Merrill's "Onesweep"): the digit histograms of ALL passes come from one
-// read of the keys up front; each pass is then a single kernel in which a tile ranks its items, publishes its per-digit
-// counts and learns its output offsets by looking back over the tiles before it (decoupled look-back) -- no per-pass
-// histogram read of the keys, no device-wide scan of a tiles x 256 table. Per pass and item: 24 B instead of 32 B of HBM
-// traffic. Forward progress: tiles are handed out by an atomic ticket, so a tile only ever waits for tiles whose CTAs are
-// already running; the wait is bounded all the same (a timed-out look-back raises *err and the host throws: a wrong size can
-// cost an error, never a hung GPU). The per-tile status words carry an epoch (the pass number), so one zero-fill serves all
-// passes of a sort.  word = epoch << 56 | state << 54 | value   state: 1 = tile aggregate, 2 = inclusive prefix
-// ------------------------------------------------------------------------------------------------
-constexpr u64 OS_VAL_MASK = (1ULL << 54) - 1ULL;
-constexpr u32 OS_SPIN_LIMIT = 1u << 26;
-
-template <class KeyT>
-__global__ void __launch_bounds__(256) radix_hist_all_kernel(const KeyT* __restrict__ keys, u64 n, int n_pass, u64* __restrict__ ghist) {
-    __shared__ u32 sh[8][256];
-    for (int p = 0; p < n_pass; p++) sh[p][threadIdx.x] = 0;
-    __syncthreads();
-    const u64 stride = (u64)gridDim.x * blockDim.x;
-    const u64 n_round = (n + 31) / 32 * 32;
-    for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < n_round; i += stride) {
-        const bool ok = i < n;
-        const u32 act = __ballot_sync(0xffffffffu, ok);
-        if (!ok) continue;
-        const KeyT k = keys[i];
-        for (int p = 0; p < n_pass; p++) {  // one shared-memory atomic per distinct digit of the warp (skewed digits would serialise)
-            const u32 d = (u32)(k >> (8 * p)) & 255u;
-            const u32 m = __match_any_sync(act, d);
-            if (lane_id() == (u32)(__ffs(m) - 1)) atomicAdd(&sh[p][d], (u32)__popc(m));
-        }
-    }
-    __syncthreads();
-    for (int p = 0; p < n_pass; p++)
-        if (sh[p][threadIdx.x]) atomicAdd(&ghist[p * 256 + threadIdx.x], (u64)sh[p][threadIdx.x]);
-}
-// per pass: exclusive scan of the 256 digit totals (one block per pass)
-static __global__ void __launch_bounds__(256) radix_base_kernel(const u64* __restrict__ ghist, u64* __restrict__ gbase) {
-    __shared__ u64 sm[33];
-    u64 tot;
-    const u64 ex = block_exclusive_sum<u64>(ghist[blockIdx.x * 256 + threadIdx.x], sm, tot);
-    gbase[blockIdx.x * 256 + threadIdx.x] = ex;
-}
-
-template <class KeyT, int ITEMS>
-__global__ void __launch_bounds__(RS_THREADS, 4) radix_onesweep_kernel(const KeyT* __restrict__ keys_in, const u32* __restrict__ vals_in, KeyT* __restrict__ keys_out,
-                                                                     u32* __restrict__ vals_out, u64 n, int shift, const u64* __restrict__ gbase,
-                                                                     volatile u64* status, u32* ticket, u64 epoch, u32* err) {
-    constexpr int TILE = RS_THREADS * ITEMS, WARP_ITEMS = TILE / RS_WARPS;
-    extern __shared__ __align__(16) unsigned char rs_smem[];
-    KeyT* s_keys = (KeyT*)rs_smem;
-    u32* s_vals = (u32*)(s_keys + TILE);
-    u32* s_cnt = s_vals + TILE;               // [RS_WARPS][257]
-    u32* s_scan = s_cnt + RS_WARPS * 257 + 256;  // 33 scratch (same layout as radix_scatter_kernel)
-    __shared__ u64 s_delta[256];
-    __shared__ u32 s_tile;
-
-    const u32 lane = lane_id(), warp = threadIdx.x >> 5;
-    if (threadIdx.x == 0) s_tile = atomicAdd(ticket, 1u);
-    for (int i = threadIdx.x; i < RS_WARPS * 257; i += RS_THREADS) s_cnt[i] = 0;
-    __syncthreads();
-    const u64 tile = s_tile;
-    const u64 tile_base = tile * TILE;
-    KeyT key[ITEMS];
-    u32 val[ITEMS];
-    u32 rnk[ITEMS];
-    u32* wc = s_cnt + warp * 257;
-#pragma unroll
-    for (int r = 0; r < ITEMS; r++) {
-        const u64 idx = tile_base + (u64)warp * WARP_ITEMS + (u64)r * 32 + lane;
-        const bool ok = idx < n;
-        key[r] = ok ? keys_in[idx] : (KeyT)~(KeyT)0;
-        val[r] = ok ? vals_in[idx] : 0u;
-        const u32 d = ok ? ((u32)(key[r] >> shift) & 255u) : 256u;
-        const u32 m = __match_any_sync(0xffffffffu, d);
-        const u32 b = wc[d];
-        __syncwarp();
-        if (lane == (u32)(__ffs(m) - 1)) wc[d] = b + __popc(m);
-        __syncwarp();
-        rnk[r] = b + __popc(m & lanemask_lt());
-    }
-    __syncthreads();
-    {
-        const u32 d = threadIdx.x;
-        u32 c[RS_WARPS], run = 0;
-#pragma unroll
-        for (int w = 0; w < RS_WARPS; w++) { c[w] = s_cnt[w * 257 + d]; run += c[w]; }
-        // publish this tile's count of digit d, then look back for the items of digit d in the tiles before
-        const u64 tag = epoch << 56;
-        status[tile * 256 + d] = tag | (1ULL << 54) | (u64)run;
-        u64 excl = 0;
-        for (u64 t = tile; t-- > 0;) {
-            u64 w64;
-            u32 spins = 0;
-            do { w64 = status[t * 256 + d]; } while (((w64 >> 56) != epoch || ((w64 >> 54) & 3ULL) == 0) && ++spins < OS_SPIN_LIMIT);
-            if (spins >= OS_SPIN_LIMIT) { atomicExch(err, 1u); break; }
-            excl += w64 & OS_VAL_MASK;
-            if (((w64 >> 54) & 3ULL) == 2ULL) break;
-        }
-        status[tile * 256 + d] = tag | (2ULL << 54) | (excl + (u64)run);
-        u32 tot;
-        u32 ex = block_exclusive_sum<u32>(run, s_scan, tot);
-        s_delta[d] = gbase[d] + excl - ex;
-#pragma unroll
-        for (int w = 0; w < RS_WARPS; w++) { s_cnt[w * 257 + d] = ex; ex += c[w]; }  // tile-local start of (warp, digit)
-    }
-    __syncthreads();
-#pragma unroll
-    for (int r = 0; r < ITEMS; r++) {
-        const u64 idx = tile_base + (u64)warp * WARP_ITEMS + (u64)r * 32 + lane;
-        if (idx < n) {
-            const u32 d = (u32)(key[r] >> shift) & 255u;
-            const u32 pos = wc[d] + rnk[r];
-            s_keys[pos] = key[r];
-            s_vals[pos] = val[r];
-        }
-    }
-    __syncthreads();
-    const u64 rem = n - tile_base;
-    const u32 valid = rem < (u64)TILE ? (u32)rem : (u32)TILE;
-    for (u32 i = threadIdx.x; i < valid; i += RS_THREADS) {
-        const KeyT k = s_keys[i];
-        const u32 d = (u32)(k >> shift) & 255u;
-        const u64 g = s_delta[d] + i;
-        keys_out[g] = k;
-        vals_out[g] = s_vals[i];
-    }
-}
-inline int rs_onesweep_setting() {
-    static int v = -1;
-    // measured on B200 (C2, 1.2e9 x 12 B items): 2.8 ms per pass against 1.6 ms for the histogram + scan + scatter passes, and the
-    // all-digit histogram costs more than the eight per-pass ones it replaces (match-any per digit); off unless GRL_RS_ONESWEEP=1
-    if (v < 0) { const char* e = getenv("GRL_RS_ONESWEEP"); v = e ? atoi(e) : 0; }
-    return v;
-}
-// all passes of one sort, one-sweep style; false if the look-back timed out (never observed; the caller reports it)
-template <class KeyT, int ITEMS>
-inline void radix_sort_onesweep(KeyT** keys, u32** vals, KeyT** keys_alt, u32** vals_alt, u64 n, int n_bits, cudaStream_t st) {
-    const int n_pass = (n_bits + 7) / 8;
-    const u64 tiles = div_up(n, RS_THREADS * ITEMS);
-    DevBuf<u64> ghist((u64)n_pass * 256, st), gbase((u64)n_pass * 256, st), status(tiles * 256, st);
-    DevBuf<u32> ctl((u64)n_pass + 1, st);  // one ticket per pass + the error flag
-    ghist.zero(); status.zero(); ctl.zero();
-    GRL_CUDA(cudaFuncSetAttribute(radix_onesweep_kernel<KeyT, ITEMS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rs_smem_bytes<KeyT, ITEMS>()));
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    GRL_LAUNCH("radix_hist_all", n * sizeof(KeyT), (radix_hist_all_kernel<KeyT>), (unsigned)std::min<u64>(div_up(n, 256), (u64)sms * 8), 256, 0, st, *keys, n, n_pass, ghist.p);
-    GRL_LAUNCH("radix_base", 0, radix_base_kernel, (unsigned)n_pass, 256, 0, st, ghist.p, gbase.p);
-    for (int p = 0; p < n_pass; p++) {
-        GRL_LAUNCH("radix_scatter", n * 2 * (sizeof(KeyT) + 4), (radix_onesweep_kernel<KeyT, ITEMS>), (unsigned)tiles, RS_THREADS, (rs_smem_bytes<KeyT, ITEMS>()), st, *keys, *vals,
-                   *keys_alt, *vals_alt, n, 8 * p, gbase.p + p * 256, status.p, ctl.p + p, (u64)(p + 1), ctl.p + n_pass);
-        KeyT* tk = *keys; *keys = *keys_alt; *keys_alt = tk;
-        u32* tv = *vals; *vals = *vals_alt; *vals_alt = tv;
-    }
-    u32 e = 0;
-    d2h_small(&e, ctl.p + n_pass, 4, st);
-    if (e) throw Error(GRLGPU_ERR_STATE, "radix sort: tile look-back timed out");
-}
-
 // one stable partition pass on the 8-bit digit at `shift` (also the building block of the LSD sort below)
-template <class KeyT, int ITEMS>
+template <class KeyT>
 inline void radix_pass(KeyT** keys, u32** vals, KeyT** keys_alt, u32** vals_alt, u64 n, int shift, DevBuf<u32>& hist, DevBuf<u64>& goff, cudaStream_t st) {
-    // per-device attributes: (re)applied for the current device, not cached process-wide
-    GRL_CUDA(cudaFuncSetAttribute(radix_scatter_kernel<KeyT, ITEMS, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rs_smem_bytes<KeyT, ITEMS>()));
-    if (rs_minb_setting() == 5) {
-        GRL_CUDA(cudaFuncSetAttribute(radix_scatter_kernel<KeyT, ITEMS, 5>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rs_smem_bytes<KeyT, ITEMS>()));
-        GRL_CUDA(cudaFuncSetAttribute(radix_scatter_kernel<KeyT, ITEMS, 5>, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
-    }
-    const u64 tiles = div_up(n, RS_THREADS * ITEMS);
-    GRL_LAUNCH("radix_hist", n * sizeof(KeyT), (radix_hist_kernel<KeyT, ITEMS>), (unsigned)tiles, RS_THREADS, 0, st, *keys, n, shift, hist.p, tiles);
+    // per-device attribute: (re)applied for the current device, not cached process-wide
+    GRL_CUDA(cudaFuncSetAttribute(radix_scatter_kernel<KeyT, RS_ITEMS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rs_smem_bytes<KeyT, RS_ITEMS>()));
+    const u64 tiles = div_up(n, RS_THREADS * RS_ITEMS);
+    GRL_LAUNCH("radix_hist", n * sizeof(KeyT), (radix_hist_kernel<KeyT, RS_ITEMS>), (unsigned)tiles, RS_THREADS, 0, st, *keys, n, shift, hist.p, tiles);
     exclusive_scan<u32, u64>(hist.p, goff.p, 256 * tiles, nullptr, st);
-    if (rs_pipe_setting()) {
-        int pipe_grid = 0;
-        {
-            GRL_CUDA(cudaFuncSetAttribute(radix_scatter_pipe_kernel<KeyT, ITEMS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rsp_smem_bytes<KeyT, ITEMS>()));
-            GRL_CUDA(cudaFuncSetAttribute(radix_scatter_pipe_kernel<KeyT, ITEMS>, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
-            int dev = 0, sms = 0, per_sm = 0;
-            GRL_CUDA(cudaGetDevice(&dev));
-            GRL_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-            GRL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, radix_scatter_pipe_kernel<KeyT, ITEMS>, RS_THREADS, rsp_smem_bytes<KeyT, ITEMS>()));
-            pipe_grid = sms * std::max(1, per_sm);
-        }
-        GRL_LAUNCH("radix_scatter", n * 2 * (sizeof(KeyT) + 4), (radix_scatter_pipe_kernel<KeyT, ITEMS>), (unsigned)std::min<u64>(tiles, (u64)pipe_grid), RS_THREADS,
-                   (rsp_smem_bytes<KeyT, ITEMS>()), st, *keys, *vals, *keys_alt, *vals_alt, n, shift, goff.p, tiles);
-    } else if (rs_minb_setting() == 5) {
-        GRL_LAUNCH("radix_scatter", n * 2 * (sizeof(KeyT) + 4), (radix_scatter_kernel<KeyT, ITEMS, 5>), (unsigned)tiles, RS_THREADS, (rs_smem_bytes<KeyT, ITEMS>()), st, *keys, *vals,
-                   *keys_alt, *vals_alt, n, shift, goff.p, tiles);
-    } else {
-        GRL_LAUNCH("radix_scatter", n * 2 * (sizeof(KeyT) + 4), (radix_scatter_kernel<KeyT, ITEMS, 4>), (unsigned)tiles, RS_THREADS, (rs_smem_bytes<KeyT, ITEMS>()), st, *keys, *vals,
-                   *keys_alt, *vals_alt, n, shift, goff.p, tiles);
-    }
+    GRL_LAUNCH("radix_scatter", n * 2 * (sizeof(KeyT) + 4), (radix_scatter_kernel<KeyT, RS_ITEMS>), (unsigned)tiles, RS_THREADS, (rs_smem_bytes<KeyT, RS_ITEMS>()), st, *keys,
+               *vals, *keys_alt, *vals_alt, n, shift, goff.p, tiles);
     KeyT* tk = *keys; *keys = *keys_alt; *keys_alt = tk;
     u32* tv = *vals; *vals = *vals_alt; *vals_alt = tv;
 }
 // Sorts in place logically: on return *keys / *vals point at the buffers holding the sorted data
 // (either the inputs or the alternates).
-template <int ITEMS>
-inline void radix_sort_pairs_t(u64** keys, u32** vals, u64** keys_alt, u32** vals_alt, u64 n, int n_bits, cudaStream_t st) {
-    if (rs_onesweep_setting() && n >= (1ull << 16) && ITEMS == 8) {  // small sorts: the launch-light 3-kernel passes below
-        radix_sort_onesweep<u64, ITEMS>(keys, vals, keys_alt, vals_alt, n, n_bits, st);
-        return;
-    }
-    const u64 tiles = div_up(n, RS_THREADS * ITEMS);
+inline void radix_sort_pairs(u64** keys, u32** vals, u64** keys_alt, u32** vals_alt, u64 n, int n_bits, cudaStream_t st) {
+    if (n <= 1 || n_bits <= 0) return;
+    const u64 tiles = div_up(n, RS_THREADS * RS_ITEMS);
     DevBuf<u32> hist(256 * tiles, st);
     DevBuf<u64> goff(256 * tiles, st);
-    for (int shift = 0; shift < n_bits; shift += 8) radix_pass<u64, ITEMS>(keys, vals, keys_alt, vals_alt, n, shift, hist, goff, st);
+    for (int shift = 0; shift < n_bits; shift += 8) radix_pass<u64>(keys, vals, keys_alt, vals_alt, n, shift, hist, goff, st);
 }
 // (u32 key, u32 value) pairs partitioned by the key's digit at `shift`: used to make a big random scatter L2-local
 inline void radix_partition_u32(u32** keys, u32** vals, u32** keys_alt, u32** vals_alt, u64 n, int shift, cudaStream_t st) {
-    const u64 tiles = div_up(n, RS_THREADS * 8);
+    const u64 tiles = div_up(n, RS_THREADS * RS_ITEMS);
     DevBuf<u32> hist(256 * tiles, st);
     DevBuf<u64> goff(256 * tiles, st);
-    radix_pass<u32, 8>(keys, vals, keys_alt, vals_alt, n, shift, hist, goff, st);
+    radix_pass<u32>(keys, vals, keys_alt, vals_alt, n, shift, hist, goff, st);
 }
 // LSD sort of (u32 key, u32 value) pairs on the low n_bits of the key
 inline void radix_sort_pairs_u32(u32** keys, u32** vals, u32** keys_alt, u32** vals_alt, u64 n, int n_bits, cudaStream_t st) {
     if (n <= 1 || n_bits <= 0) return;
-    const u64 tiles = div_up(n, RS_THREADS * 8);
+    const u64 tiles = div_up(n, RS_THREADS * RS_ITEMS);
     DevBuf<u32> hist(256 * tiles, st);
     DevBuf<u64> goff(256 * tiles, st);
-    for (int shift = 0; shift < n_bits; shift += 8) radix_pass<u32, 8>(keys, vals, keys_alt, vals_alt, n, shift, hist, goff, st);
-}
-inline int rs_items_setting() {
-    static int v = 0;
-    if (!v) { const char* e = getenv("GRL_RS_ITEMS"); v = e ? atoi(e) : 8; if (v != 4 && v != 8 && v != 12 && v != 16) v = 8; }  // 8 items/thread: 59 registers, 4 CTAs/SM (measured best on B200)
-    return v;
-}
-inline void radix_sort_pairs(u64** keys, u32** vals, u64** keys_alt, u32** vals_alt, u64 n, int n_bits, cudaStream_t st) {
-    if (n <= 1 || n_bits <= 0) return;
-    switch (rs_items_setting()) {
-        case 4: radix_sort_pairs_t<4>(keys, vals, keys_alt, vals_alt, n, n_bits, st); break;
-        case 16: radix_sort_pairs_t<16>(keys, vals, keys_alt, vals_alt, n, n_bits, st); break;
-        case 12: radix_sort_pairs_t<12>(keys, vals, keys_alt, vals_alt, n, n_bits, st); break;
-        default: radix_sort_pairs_t<8>(keys, vals, keys_alt, vals_alt, n, n_bits, st); break;
-    }
+    for (int shift = 0; shift < n_bits; shift += 8) radix_pass<u32>(keys, vals, keys_alt, vals_alt, n, shift, hist, goff, st);
 }
 
 // ------------------------------------------------------------------------------------------------
