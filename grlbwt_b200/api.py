@@ -11,6 +11,7 @@ import numpy as np
 
 LIB_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "lib")
 FLAG_SMALL_TABLE, FLAG_FORCE_SLOW_SCAN, FLAG_KEEP_DICT, FLAG_FORCE_UNCACHED, FLAG_SMALL_PILOT, FLAG_FORCE_DOUBLING = 1, 2, 4, 8, 16, 32
+FLAG_FORCE_WALK, FLAG_FORCE_JUMP = 64, 128   # tests: grlgpu_invert takes the walk per string / pointer jumping regardless of the chains
 CELL = {1: np.uint8, 2: np.uint16, 4: np.uint32, 8: np.uint64}
 
 
@@ -37,6 +38,11 @@ class Round(C.Structure):
 class Slice(C.Structure):
     _fields_ = [(k, C.c_uint64) for k in ("rank_base", "tot_local", "pre_first", "n_pre_local", "exchange_bytes", "n_in_local", "parse_len_local")] + \
                [("sym_bytes", C.c_uint32), ("reserved", C.c_uint32)]
+
+
+class Invert(C.Structure):
+    _fields_ = [(k, C.c_uint64) for k in ("n", "n_strings", "n_runs", "n_out")] + [(k, C.c_uint32) for k in ("path", "jump_rounds")] + \
+               [(k, C.c_float) for k in ("device_ms", "lf_ms", "invert_ms")]
 
 
 class BwtResult(C.Structure):
@@ -105,6 +111,7 @@ def lib_gpu():
         L.grlgpu_text_end.argtypes = [vp]
         L.grlgpu_level_park.argtypes = [vp, C.c_int, vp]
         L.grlgpu_copy_to_host.argtypes = [C.c_int, vp, vp, u64]
+        L.grlgpu_invert.argtypes = [vp, vp, u64, C.c_int, u64, vp, u64, C.POINTER(Invert)]
         L.grlgpu_selftest_scan.argtypes = [vp, u64, vp, vp]
         L.grlgpu_selftest_sort.argtypes = [vp, vp, u64, C.c_int]
         L.grlgpu_selftest_compact.argtypes = [vp, vp, u64, vp, vp]
@@ -307,6 +314,18 @@ class GrlGpu:
         self._check(self._L.grlgpu_fetch_parse(self._h, _ptr(out)))
         return out
 
+    def invert(self, image, cell_bytes: int = 1, n_seqs: int | None = None, out: np.ndarray | None = None):
+        """invert_rl_bwt on this context (its text, levels and BWT are left as they are)"""
+        raw, out = _invert_args(image, cell_bytes, n_seqs, out)
+        info = Invert()
+        rc = self._L.grlgpu_invert(self._h, _ptr(raw), raw.size, cell_bytes, (1 << 64) - 1 if n_seqs is None else int(n_seqs), _ptr(out), out.size, C.byref(info))
+        d = {k: getattr(info, k) for k, _ in Invert._fields_}
+        if rc != 0:
+            err = GrlGpuError(rc, self._L.grlgpu_strerror(rc).decode() + " | " + self._L.grlgpu_last_error(self._h).decode())
+            err.info = d
+            raise err
+        return out[: d["n_out"] * cell_bytes].view(CELL[cell_bytes]), d
+
     def profile_enable(self, on: bool = True):
         self._check(self._L.grlgpu_profile_enable(self._h, int(on)))
 
@@ -413,6 +432,36 @@ def parse_rl_bwt(image) -> tuple:
     for i in range(fb):
         lens |= rec[:, sb + i].astype(np.uint64) << np.uint64(8 * i)
     return syms, lens, sb, fb
+
+
+def _invert_args(image, cell_bytes, n_seqs, out):
+    """checks of invert_rl_bwt's arguments, before the library is called -> (uint8 image, output buffer)"""
+    if cell_bytes not in CELL:
+        raise GrlGpuError(-1, "cell_bytes must be 1, 2, 4 or 8")
+    if n_seqs is not None and int(n_seqs) < 0:
+        raise GrlGpuError(-1, "n_seqs must be >= 0")
+    if out is not None and (not isinstance(out, np.ndarray) or out.dtype != np.uint8 or out.ndim != 1 or not out.flags.c_contiguous or not out.flags.writeable):
+        raise GrlGpuError(-1, "out must be a writable contiguous 1-d uint8 array")
+    raw = np.fromfile(image, np.uint8) if isinstance(image, (str, os.PathLike)) else np.ascontiguousarray(np.frombuffer(image, np.uint8))
+    if out is None:   # the BWT length n bounds the output; a malformed header is left to the library to report
+        n = 0
+        if raw.size >= 16:
+            sb, fb = (int(x) for x in raw[:16].view(np.uint64))
+            if 1 <= sb <= 8 and 1 <= fb <= 8:
+                rec = raw[16:16 + (raw.size - 16) // (sb + fb) * (sb + fb)].reshape(-1, sb + fb)
+                n = sum(int(rec[:, sb + i].sum(dtype=np.uint64)) << (8 * i) for i in range(fb))
+        out = np.zeros(n * cell_bytes, np.uint8)
+    return raw, out
+
+
+def invert_rl_bwt(image, cell_bytes: int = 1, n_seqs: int | None = None, device: int = 0, flags: int = 0, out: np.ndarray | None = None):
+    """Inverts a BCR BWT on the device (grlgpu_invert): `image` is what parse_rl_bwt takes (a path, bytes or a uint8 array).
+    -> (the first min(n_seqs, N) strings, each followed by the separator, as cells of cell_bytes bytes; dict of grlgpu_invert_t).
+    out: optional caller-owned uint8 buffer (e.g. pinned memory) the cells are written to; the result is a view of it.
+    Errors of the call raise GrlGpuError, whose `info` holds the dict (n_out = cells needed when `out` is too small)."""
+    raw, out = _invert_args(image, cell_bytes, n_seqs, out)
+    with GrlGpu(device, flags) as ctx:
+        return ctx.invert(raw, cell_bytes, n_seqs, out)
 
 
 def build_bwt_file(inp: str, out: str, sym_bytes: int = 1, device: int = 0, n_threads: int = 1, verbose: bool = False):

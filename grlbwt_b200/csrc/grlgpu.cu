@@ -751,6 +751,7 @@ void run_round_t(grlgpu_ctx* c, grlgpu_round_t* out) {
 
 #include "mg2.cuh"
 #include "induce.cuh"
+#include "invert.cuh"
 
 void run_round(grlgpu_ctx* c, grlgpu_round_t* out) {
     if (c->first) {
@@ -1655,6 +1656,19 @@ int grlgpu_fetch_bwt_packed(grlgpu_ctx* ctx, int sb, int fb, void* out, uint64_t
         for (int q = 0; q < 2; q++) { cudaEventDestroy(packed[q]); cudaEventDestroy(copied[q]); }
         if (d2h_scalar(err.p, st)) throw Error(GRLGPU_ERR_STATE, "a symbol or a run length of the BWT does not fit the record widths");
     });
+}
+
+int grlgpu_invert(grlgpu_ctx* ctx, const void* image, uint64_t image_bytes, int cell_bytes, uint64_t n_seqs, void* out, uint64_t cap_bytes, grlgpu_invert_t* info) {
+    if (!ctx || !image || !info || !(cell_bytes == 1 || cell_bytes == 2 || cell_bytes == 4 || cell_bytes == 8)) return GRLGPU_ERR_ARG;
+    memset(info, 0, sizeof(*info));
+    if (image_bytes < 16) return GRLGPU_ERR_ARG;
+    u64 hdr[2];
+    memcpy(hdr, image, 16);
+    if (hdr[0] < 1 || hdr[0] > 8 || hdr[1] < 1 || hdr[1] > 8) return GRLGPU_ERR_ARG;
+    const u64 body = image_bytes - 16;
+    if (body == 0 || body % (hdr[0] + hdr[1])) return GRLGPU_ERR_ARG;
+    if (!out && cap_bytes) return GRLGPU_ERR_ARG;
+    return guarded(ctx, [&] { invert_image(ctx, (const u8*)image, image_bytes, cell_bytes, n_seqs, out, cap_bytes, info); });
 }
 
 int grlgpu_profile_enable(grlgpu_ctx* ctx, int on) {

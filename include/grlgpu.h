@@ -35,6 +35,8 @@ enum grlgpu_status {
 #define GRLGPU_FLAG_SMALL_PILOT 16ull /* tests: one pilot tile, so small inputs exercise pilot + remainder */
 #define GRLGPU_FLAG_FORCE_DOUBLING 32ull /* tests: refine suffix groups by prefix doubling even when key extension would do */
 #define GRLGPU_FLAG_KEEP_DICT 4ull /* tests: keep the last round's dictionary for grlgpu_fetch_dictionary */
+#define GRLGPU_FLAG_FORCE_WALK 64ull /* tests: grlgpu_invert walks every string, whatever the chain lengths */
+#define GRLGPU_FLAG_FORCE_JUMP 128ull /* tests: grlgpu_invert runs pointer jumping, whatever the chain lengths */
 
 /* = str_collection (external/cdt/include/utils.h:20-28) as filled by collection_stats (utils.cpp:100-189) */
 typedef struct {
@@ -161,6 +163,25 @@ int grlgpu_fetch_bwt(grlgpu_ctx* ctx, uint32_t* syms, uint32_t* lens);
 int grlgpu_fetch_bwt_packed(grlgpu_ctx* ctx, int sb, int fb, void* out, uint64_t cap_bytes, uint64_t* n_bytes);
 /* the same arrays as DEVICE addresses (valid until grlgpu_drop_kept / the next grlgpu_induce), for parallel grlgpu_copy_to_host */
 int grlgpu_bwt_ptrs(grlgpu_ctx* ctx, const uint32_t** d_syms, const uint32_t** d_lens, uint64_t* n_runs);
+
+/* inversion of a BCR BWT: the .rl_bwt image back to the collection (replaces scripts/reverse_bwt.cpp:5-54)
+ * image: [sb u64][fb u64] + records of sb symbol bytes and fb length bytes, little endian (what grlgpu_fetch_bwt_packed and the CLI
+ * write). The separator is the smallest symbol, N = its count; out receives the first min(n_seqs, N) strings, each followed by the
+ * separator, as cells of cell_bytes little-endian bytes: byte for byte what `reverse_bwt image out [n_seqs] -a cell_bytes` writes.
+ * GRLGPU_ERR_ARG: sb or fb outside 1..8, a partial record, no record, cell_bytes not in {1,2,4,8}, or cap_bytes smaller than
+ * n_out * cell_bytes (info->n_out is then set). GRLGPU_ERR_LIMIT: n >= 0xfffffff0 or a symbol / length >= 2^32 (the host tool
+ * reverse_bwt is the general path). GRLGPU_ERR_ILL_FORMED: the run list is not a BWT (its LF has a cycle without separator).
+ * Needs no text in the context and leaves its text, levels and BWT untouched. The path (walk per string or pointer jumping) is
+ * chosen from the chain lengths the call observes (GRLGPU_FLAG_FORCE_WALK / _JUMP force one, for tests). */
+typedef struct {
+    uint64_t n, n_strings, n_runs;   /* BWT length, separators, records of the image */
+    uint64_t n_out;                  /* cells written (or needed, when cap_bytes is too small) */
+    uint32_t path;                   /* 0 walk per string, 1 pointer jumping */
+    uint32_t jump_rounds;
+    float device_ms, lf_ms, invert_ms; /* CUDA events on the context's stream: whole call / table / inversion */
+} grlgpu_invert_t;
+int grlgpu_invert(grlgpu_ctx* ctx, const void* image, uint64_t image_bytes, int cell_bytes,
+                  uint64_t n_seqs /* UINT64_MAX: all */, void* out, uint64_t cap_bytes, grlgpu_invert_t* info);
 
 /* digest of the last round's level artefacts, computed on the device before they are fetched: four sums mod 2^64
  * {rules weighted by rank, hocc marks weighted by rank, sum of the preliminary-BWT run lengths, runs weighted by symbol}.
