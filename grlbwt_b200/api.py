@@ -45,6 +45,15 @@ class Invert(C.Structure):
                [(k, C.c_float) for k in ("device_ms", "lf_ms", "invert_ms")]
 
 
+class FmInfo(C.Structure):
+    _fields_ = [(k, C.c_uint64) for k in ("n", "n_strings", "n_runs", "sigma", "sep")] + [("load_ms", C.c_float)]
+
+
+class FmQuery(C.Structure):
+    _fields_ = [(k, C.c_uint64) for k in ("n_pat", "n_pat_syms", "n_occ")] + [(k, C.c_uint32) for k in ("path", "jump_rounds")] + \
+               [(k, C.c_float) for k in ("device_ms", "search_ms", "locate_ms")]
+
+
 class BwtResult(C.Structure):
     _fields_ = [("n_runs", C.c_uint64), ("sb", C.c_uint64), ("fb", C.c_uint64), ("syms", C.POINTER(C.c_uint64)),
                 ("lens", C.POINTER(C.c_uint64)), ("n_rounds", C.c_uint64), ("h2d_ms", C.c_double), ("par_phase_ms", C.c_double),
@@ -112,6 +121,10 @@ def lib_gpu():
         L.grlgpu_level_park.argtypes = [vp, C.c_int, vp]
         L.grlgpu_copy_to_host.argtypes = [C.c_int, vp, vp, u64]
         L.grlgpu_invert.argtypes = [vp, vp, u64, C.c_int, u64, vp, u64, C.POINTER(Invert)]
+        L.grlgpu_fm_load.argtypes = [vp, vp, u64, C.POINTER(FmInfo)]
+        L.grlgpu_fm_count.argtypes = [vp, vp, vp, u64, C.c_int, vp, C.POINTER(FmQuery)]
+        L.grlgpu_fm_locate.argtypes = [vp, vp, vp, u64, C.c_int, vp, vp, vp, u64, C.POINTER(FmQuery)]
+        L.grlgpu_fm_drop.argtypes = [vp]
         L.grlgpu_selftest_scan.argtypes = [vp, u64, vp, vp]
         L.grlgpu_selftest_sort.argtypes = [vp, vp, u64, C.c_int]
         L.grlgpu_selftest_compact.argtypes = [vp, vp, u64, vp, vp]
@@ -326,6 +339,49 @@ class GrlGpu:
             raise err
         return out[: d["n_out"] * cell_bytes].view(CELL[cell_bytes]), d
 
+    def _fm_call(self, rc, info):
+        d = {k: getattr(info, k) for k, _ in type(info)._fields_}
+        if rc != 0:
+            err = GrlGpuError(rc, self._L.grlgpu_strerror(rc).decode() + " | " + self._L.grlgpu_last_error(self._h).decode())
+            err.info = d
+            raise err
+        return d
+
+    def fm_load(self, image):
+        """Loads a .rl_bwt image (what parse_rl_bwt takes: a path, bytes or a uint8 array) as this context's FM-index, replacing the
+        one loaded before; its text, levels and BWT are left as they are. -> dict of grlgpu_fm_t (n, n_strings, n_runs, sigma, sep)"""
+        raw = _image_bytes(image)
+        info = FmInfo()
+        return self._fm_call(self._L.grlgpu_fm_load(self._h, _ptr(raw), raw.size, C.byref(info)), info)
+
+    def fm_count(self, patterns):
+        """Backward search of every pattern (see _fm_patterns for the forms accepted) -> (sp, ep, info): uint64 arrays, the rows
+        [sp, ep) whose suffix starts with the pattern (sp = ep = 0 when it does not occur), and the dict of grlgpu_fm_query_t"""
+        cells, off = _fm_patterns(patterns)
+        n_pat = off.size - 1
+        sp_ep = np.zeros(2 * max(n_pat, 1), np.uint64)
+        info = FmQuery()
+        d = self._fm_call(self._L.grlgpu_fm_count(self._h, _ptr(cells), _ptr(off), n_pat, cells.dtype.itemsize, _ptr(sp_ep), C.byref(info)), info)
+        return sp_ep[0:2 * n_pat:2].copy(), sp_ep[1:2 * n_pat:2].copy(), d
+
+    def fm_locate(self, patterns):
+        """Every occurrence of every pattern -> (occ_off, str_id, str_pos, info): pattern q's occurrences are
+        [occ_off[q], occ_off[q + 1]) of str_id (string k) and str_pos (offset p), in row order. The output is sized by a count call."""
+        cells, off = _fm_patterns(patterns)
+        n_pat = off.size - 1
+        sp, ep, _ = self.fm_count((cells, off))
+        n_occ = int((ep - sp).sum())
+        occ_off = np.zeros(n_pat + 1, np.uint64)
+        str_id, str_pos = np.zeros(max(n_occ, 1), np.uint32), np.zeros(max(n_occ, 1), np.uint32)
+        info = FmQuery()
+        d = self._fm_call(self._L.grlgpu_fm_locate(self._h, _ptr(cells), _ptr(off), n_pat, cells.dtype.itemsize, _ptr(occ_off), _ptr(str_id), _ptr(str_pos),
+                                                   n_occ, C.byref(info)), info)
+        return occ_off, str_id[:n_occ], str_pos[:n_occ], d
+
+    def fm_drop(self):
+        """Frees this context's FM-index"""
+        self._check(self._L.grlgpu_fm_drop(self._h))
+
     def profile_enable(self, on: bool = True):
         self._check(self._L.grlgpu_profile_enable(self._h, int(on)))
 
@@ -432,6 +488,48 @@ def parse_rl_bwt(image) -> tuple:
     for i in range(fb):
         lens |= rec[:, sb + i].astype(np.uint64) << np.uint64(8 * i)
     return syms, lens, sb, fb
+
+
+def _image_bytes(image) -> np.ndarray:
+    """a .rl_bwt image as contiguous uint8: a path is read, bytes and arrays are viewed"""
+    if isinstance(image, (str, os.PathLike)):
+        return np.fromfile(image, np.uint8)
+    return np.ascontiguousarray(np.frombuffer(image, np.uint8))
+
+
+def _fm_patterns(patterns) -> tuple:
+    """checks of the patterns of fm_count / fm_locate, before the library is called -> (cells, uint64 offsets). Accepted: a list
+    of patterns (bytes, or 1-d arrays of one unsigned cell type), or a tuple (concatenated cells, offsets) with offsets[0] = 0.
+    Every pattern has at least one cell."""
+    if isinstance(patterns, tuple):
+        if len(patterns) != 2:
+            raise GrlGpuError(-1, "patterns: a pair (cells, offsets) is expected")
+        cells, off = np.asarray(patterns[0]), np.asarray(patterns[1])
+        if off.ndim != 1 or off.size == 0 or off.dtype.kind not in "iu":
+            raise GrlGpuError(-1, "patterns: offsets must be a non-empty 1-d integer array")
+        if off.dtype.kind == "i" and (off < 0).any():
+            raise GrlGpuError(-1, "patterns: offsets must not be negative")
+        off = off.astype(np.uint64)
+    elif isinstance(patterns, list):
+        parts = [np.frombuffer(p, np.uint8) if isinstance(p, (bytes, bytearray)) else np.asarray(p) for p in patterns]
+        if any(p.ndim != 1 for p in parts):
+            raise GrlGpuError(-1, "patterns: every pattern must be bytes or a 1-d array")
+        kinds = {p.dtype for p in parts}
+        if len(kinds) > 1:
+            raise GrlGpuError(-1, "patterns: every pattern must have the same cell type")
+        dt = kinds.pop() if kinds else np.dtype(np.uint8)
+        cells = np.concatenate(parts).astype(dt, copy=False) if parts else np.zeros(0, dt)
+        off = np.zeros(len(parts) + 1, np.uint64)
+        off[1:] = np.cumsum([p.size for p in parts], dtype=np.uint64)
+    else:
+        raise GrlGpuError(-1, "patterns: a list of patterns or a pair (cells, offsets) is expected")
+    if cells.ndim != 1 or cells.dtype not in [np.dtype(t) for t in CELL.values()]:
+        raise GrlGpuError(-1, "patterns: cells must be a 1-d array of uint8, uint16, uint32 or uint64")
+    if off[0] != 0 or int(off[-1]) > cells.size:
+        raise GrlGpuError(-1, "patterns: offsets must start at 0 and end inside the cells")
+    if (np.diff(off.astype(np.int64)) <= 0).any():
+        raise GrlGpuError(-1, "patterns: every pattern must have at least one cell (offsets strictly increasing)")
+    return np.ascontiguousarray(cells), np.ascontiguousarray(off)
 
 
 def _invert_args(image, cell_bytes, n_seqs, out):

@@ -1,0 +1,264 @@
+// Search of a BCR BWT ON THE DEVICE: a .rl_bwt image kept as a run-length FM-index, queried for count and locate.
+//   load     the LF table of invert.cuh (part a, shared), kept with its run arrays and the symbol-sorted run order; a symbol
+//            directory (per distinct symbol: its slice of that order and C[c]) from head flags over the sorted symbols; psi = LF^-1
+//   count    backward search, one thread per pattern, from its last symbol; LF_c(i) = C[c] + rank_c(BWT, i) for i in [0, n]:
+//            the run k holding i (upper bound on the run starts, k = r for i = n) gives F[k] + i - start[k] when its symbol is c,
+//            otherwise the last run q < k of c's slice (binary search) gives F[q] + len[q], or C[c] when there is none
+//   locate   one thread per occurrence (row j of some [sp, ep)), offsets of the occurrences = exclusive scan of ep - sp in u64:
+//            the offset p = LF steps from j to a row whose BWT symbol is the separator; the string k = the first row < N that
+//            psi steps reach from j (row k < N is $_k, the end of string k); both walks bounded by B (inv_walk_bound). A longer
+//            walk switches the call to a table of (k, p) for every row, built once per index by pointer jumping (invert.cuh,
+//            part c: p = d, k = the string whose chain from row k ends at succ) and kept for every later call.
+// Convention of reverse_bwt and grlgpu_invert: the separator is the smallest symbol of a non-empty record, N its count, strings in
+// input order. A pattern containing the separator or a symbol outside the directory has no occurrence; every empty interval is
+// reported as sp = ep = 0 (the host tool fm_query does the same). Positions and symbols are 32-bit, as for the inversion.
+// Included by grlgpu.cu inside its anonymous namespace, after invert.cuh.
+#pragma once
+
+constexpr u32 FM_OVER_POLL = 256;  // locate walk: steps between two reads of the "some walk is over the bound" flag
+
+struct FmView {  // device arrays of a loaded index, passed to the search kernels by value
+    const u32 *start, *sym, *len, *F, *order, *dir_sym, *dir_first, *dir_C;
+    u32 n, n_runs, n_dir, sep;
+};
+
+// position of symbol v in the directory, or n_dir when the index has no record of it (or v is the separator)
+__device__ __forceinline__ u32 fm_dir_find(const FmView& x, u64 v) {
+    if ((v >> 32) || (u32)v == x.sep) return x.n_dir;
+    const u32 d = ind_lower_bound(x.dir_sym, x.n_dir, (u32)v);
+    return (d < x.n_dir && x.dir_sym[d] == (u32)v) ? d : x.n_dir;
+}
+// LF_c(i) = C[c] + rank_c(BWT, i), i in [0, n], c = dir_sym[d]
+__device__ __forceinline__ u32 fm_lf_c(const FmView& x, u32 d, u32 i) {
+    const u32 c = x.dir_sym[d];
+    const u32 k = ind_upper_bound(x.start, x.n_runs + 1, i) - 1;  // start[n_runs] = n: k = n_runs for i = n
+    if (k < x.n_runs && x.sym[k] == c) return x.F[k] + (i - x.start[k]);
+    const u32 lo = x.dir_first[d], m = ind_lower_bound(x.order + lo, x.dir_first[d + 1] - lo, k);  // runs of c before run k
+    if (m == 0) return x.dir_C[d];
+    const u32 q = x.order[lo + m - 1];
+    return x.F[q] + x.len[q];
+}
+
+// one thread per pattern: sp_ep[2q], sp_ep[2q + 1]
+template <class CellT>
+__global__ void __launch_bounds__(INV_THREADS) fm_count_kernel(FmView x, const CellT* __restrict__ pat, const u64* __restrict__ pat_off, u64 n_pat, u64* __restrict__ sp_ep) {
+    const u64 q = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= n_pat) return;
+    u32 sp = 0, ep = x.n;
+    for (u64 a = pat_off[q + 1]; a > pat_off[q];) {  // the pattern's cells, last first
+        const u32 d = fm_dir_find(x, (u64)pat[--a]);
+        if (d == x.n_dir) { sp = ep = 0; break; }
+        sp = fm_lf_c(x, d, sp);
+        ep = fm_lf_c(x, d, ep);
+        if (sp >= ep) { sp = ep = 0; break; }
+    }
+    sp_ep[2 * q] = sp;
+    sp_ep[2 * q + 1] = ep;
+}
+static __global__ void __launch_bounds__(INV_THREADS) fm_occ_count_kernel(const u64* __restrict__ sp_ep, u64 n_pat, u64* __restrict__ cnt) {
+    const u64 q = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    if (q < n_pat) cnt[q] = sp_ep[2 * q + 1] - sp_ep[2 * q];
+}
+// row of occurrence o: the pattern q with occ_off[q] <= o < occ_off[q + 1], then sp + the rank inside [sp, ep)
+__device__ __forceinline__ u32 fm_occ_row(const u64* __restrict__ sp_ep, const u64* __restrict__ occ_off, u64 n_pat, u64 o) {
+    u64 lo = 0, hi = n_pat;  // last q with occ_off[q] <= o (occ_off[0] = 0 <= o)
+    while (hi - lo > 1) { const u64 mid = (lo + hi) >> 1; if (occ_off[mid] <= o) lo = mid; else hi = mid; }
+    return (u32)(sp_ep[2 * lo] + (o - occ_off[lo]));
+}
+// walk: at most `bound` LF steps for p and `bound` psi steps for k; a longer walk sets *over and leaves the occurrence unwritten.
+// Once *over is set the whole call goes to the table, so every thread stops: at its start, and every FM_OVER_POLL steps of a walk.
+static __global__ void __launch_bounds__(INV_THREADS) fm_locate_walk_kernel(const u64* __restrict__ E, const u32* __restrict__ psi, u32 N, u32 sep, const u64* __restrict__ sp_ep,
+                                                                            const u64* __restrict__ occ_off, u64 n_pat, u64 n_occ, u32 bound, u32* __restrict__ str_id,
+                                                                            u32* __restrict__ str_pos, u32* over) {
+    const u64 o = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    if (o >= n_occ) return;
+    const volatile u32* over_v = over;
+    if (*over_v) return;
+    const u32 j = fm_occ_row(sp_ep, occ_off, n_pat, o);
+    u32 r = j, p = 0;
+    for (; p < bound; p++) {  // bounded by `bound`
+        const u64 e = ld_gather8(E + r);
+        if (inv_sym(e) == sep) break;
+        r = inv_lf(e);
+        if ((p & (FM_OVER_POLL - 1)) == FM_OVER_POLL - 1 && *over_v) return;
+    }
+    u32 k = j, f = 0;
+    for (; f < bound; f++) {  // bounded by `bound`
+        k = ld_gather4(psi + k);
+        if (k < N) break;
+        if ((f & (FM_OVER_POLL - 1)) == FM_OVER_POLL - 1 && *over_v) return;
+    }
+    if (p == bound || f == bound) { atomicExch(over, 1u); return; }
+    str_id[o] = k;
+    str_pos[o] = p;
+}
+static __global__ void __launch_bounds__(INV_THREADS) fm_locate_table_kernel(const u64* __restrict__ doc, const u64* __restrict__ sp_ep, const u64* __restrict__ occ_off, u64 n_pat,
+                                                                             u64 n_occ, u32* __restrict__ str_id, u32* __restrict__ str_pos) {
+    const u64 o = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    if (o >= n_occ) return;
+    const u64 t = ld_gather8(doc + fm_occ_row(sp_ep, occ_off, n_pat, o));
+    str_id[o] = (u32)(t >> 32);
+    str_pos[o] = (u32)t;
+}
+
+// load: C[c] of every directory entry = F row of the first run of its slice
+static __global__ void __launch_bounds__(INV_THREADS) fm_dir_c_kernel(const u32* __restrict__ dir_first, const u32* __restrict__ order, const u32* __restrict__ F, u32 n_dir,
+                                                                      u32* __restrict__ dir_C) {
+    const u32 d = blockIdx.x * blockDim.x + threadIdx.x;
+    if (d < n_dir) dir_C[d] = F[order[dir_first[d]]];
+}
+static __global__ void __launch_bounds__(INV_THREADS) fm_psi_kernel(const u64* __restrict__ E, u32 n, u32* __restrict__ psi) {
+    const u32 j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j < n) psi[inv_lf(E[j])] = j;
+}
+// locate table from converged pointer jumping: doc[j] = {owner[succ] << 32 | d}; a chain that ends on a row that is not a
+// separator row, or on one no string i < N reaches, lies on a cycle without separator (*bad)
+static __global__ void __launch_bounds__(INV_THREADS) fm_doc_kernel(const u64* __restrict__ E, const u64* __restrict__ P, const u32* __restrict__ owner, u32 n, u32 N, u32 sep,
+                                                                    u64* __restrict__ doc, u32* bad) {
+    const u32 j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= n) return;
+    const u64 p = P[j];
+    const u32 s = (u32)p, k = ld_gather4(owner + s);
+    if (inv_sym(ld_gather8(E + s)) != sep || k >= N) { atomicExch(bad, 1u); return; }
+    doc[j] = ((u64)k << 32) | (p >> 32);
+}
+
+inline FmView fm_view(const FmIndex& x) {
+    return FmView{x.t.start.p, x.t.sym.p, x.t.len.p, x.t.F.p, x.t.order.p, x.dir_sym.p, x.dir_first.p, x.dir_C.p, (u32)x.t.n, (u32)x.t.n_runs, (u32)x.n_dir, x.t.sep};
+}
+
+// Load of a checked image (as lf_table_build) into the context's index; the index already loaded was dropped by the caller.
+inline void fm_load(grlgpu_ctx* c, const u8* image, u64 image_bytes, grlgpu_fm_t* info) {
+    cudaStream_t st = c->st;
+    Timer t_all(st);
+    t_all.start();
+    std::unique_ptr<FmIndex> x(new FmIndex());
+    LfTable& t = x->t;
+    DevBuf<u32> keys;
+    lf_table_build(image, image_bytes, t, &keys, st, "FM-index load on the device");
+    const u32 n = (u32)t.n, nr = (u32)t.n_runs;
+    if (n) {
+        {   // directory: one entry per distinct symbol of the sorted keys
+            DevBuf<u32> flags(nr, st), excl((u64)nr + 1, st);
+            GRL_LAUNCH("ind_head_flags", (u64)nr * 8, ind_head_flags_kernel, grid_for(nr, 256), 256, 0, st, keys.p, nr, flags.p);
+            x->n_dir = ind_scan_total(flags.p, excl.p, nr, st);
+            x->dir_sym.alloc(x->n_dir, st);
+            x->dir_first.alloc(x->n_dir + 1, st);
+            x->dir_C.alloc(x->n_dir, st);
+            GRL_LAUNCH("ind_compact_runs", (u64)nr * 16, ind_compact_runs_kernel, grid_for(nr, 256), 256, 0, st, keys.p, (const u32*)nullptr, flags.p, excl.p, nr, nr,
+                       (u32)x->n_dir, x->dir_sym.p, x->dir_first.p);
+            GRL_LAUNCH("fm_dir_c", x->n_dir * 12 + x->n_dir * 64, fm_dir_c_kernel, grid_for(x->n_dir, INV_THREADS), INV_THREADS, 0, st, x->dir_first.p, t.order.p, t.F.p,
+                       (u32)x->n_dir, x->dir_C.p);
+        }
+        keys.release();
+        x->psi.alloc(n, st);
+        GRL_LAUNCH("fm_psi", (u64)n * (8 + 32), fm_psi_kernel, grid_for(n, INV_THREADS), INV_THREADS, 0, st, t.E.p, n, x->psi.p);
+    }
+    t_all.stop();
+    info->n = t.n;
+    info->n_strings = t.N;
+    info->n_runs = t.n_runs;
+    info->sigma = x->n_dir;
+    info->sep = t.sep;
+    info->load_ms = t_all.ms();  // synchronises the stream
+    c->fm = std::move(x);
+}
+
+// the locate table of the loaded index (once): pointer jumping over LF, then one entry per row
+inline u32 fm_build_doc(FmIndex& x, u32* flag, cudaStream_t st) {
+    const u32 n = (u32)x.t.n, N = (u32)x.t.N;
+    DevBuf<u64> P(n, st);
+    DevBuf<u32> owner(n, st);
+    const u32 rounds = inv_jump_converge(x.t.E.p, n, x.t.sep, P, owner.p, flag, st, "locate");
+    {
+        DevBuf<u32> slen(N, st);
+        GRL_LAUNCH("inv_jump_owner", (u64)N * (8 + 4 + 32), inv_jump_owner_kernel, grid_for(N, INV_THREADS), INV_THREADS, 0, st, P.p, N, slen.p, owner.p);
+    }
+    x.doc.alloc(n, st);
+    GRL_CUDA(cudaMemsetAsync(flag, 0, 4, st));
+    GRL_LAUNCH("fm_doc", (u64)n * (8 + 32 + 32 + 8), fm_doc_kernel, grid_for(n, INV_THREADS), INV_THREADS, 0, st, x.t.E.p, P.p, owner.p, n, N, x.t.sep, x.doc.p, flag);
+    if (d2h_scalar(flag, st)) {
+        x.doc.release();
+        throw Error(GRLGPU_ERR_ILL_FORMED, "locate: a chain ends on a row that is not a string's separator row (an LF cycle without separator)");
+    }
+    x.doc_ready = true;
+    return rounds;
+}
+
+// count (str_id == nullptr) or locate of n_pat > 0 checked patterns on the loaded index
+inline void fm_query(grlgpu_ctx* c, const void* pat, const uint64_t* pat_off, u64 n_pat, int pat_bytes, uint64_t* sp_ep, uint64_t* occ_off, u32* str_id, u32* str_pos, u64 cap_occ,
+                     grlgpu_fm_query_t* info) {
+    cudaStream_t st = c->st;
+    FmIndex& x = *c->fm;
+    const u64 n_syms = pat_off[n_pat];
+    info->n_pat = n_pat;
+    info->n_pat_syms = n_syms;
+    const bool locate = str_id != nullptr || occ_off != nullptr;
+    Timer t_all(st), t_search(st), t_loc(st);
+    t_all.start();
+    t_search.start();
+    DevBuf<u64> d_se(2 * n_pat, st);
+    if (x.t.n == 0) d_se.zero();  // no rows: every interval is empty
+    else {
+        DevBuf<u8> d_pat(n_syms * pat_bytes, st);
+        DevBuf<u64> d_off(n_pat + 1, st);
+        GRL_CUDA(cudaMemcpyAsync(d_pat.p, pat, n_syms * pat_bytes, cudaMemcpyHostToDevice, st));
+        GRL_CUDA(cudaMemcpyAsync(d_off.p, pat_off, (n_pat + 1) * 8, cudaMemcpyHostToDevice, st));
+        const FmView v = fm_view(x);
+        // per pattern symbol two searches over the run starts and one over its slice: one 32 B sector per probe
+        const u64 model = n_pat * 24 + n_syms * (pat_bytes + 2 * 64 * 32);
+        switch (pat_bytes) {
+            case 1: GRL_LAUNCH("fm_count", model, (fm_count_kernel<u8>), grid_for(n_pat, INV_THREADS), INV_THREADS, 0, st, v, (const u8*)d_pat.p, d_off.p, n_pat, d_se.p); break;
+            case 2: GRL_LAUNCH("fm_count", model, (fm_count_kernel<u16>), grid_for(n_pat, INV_THREADS), INV_THREADS, 0, st, v, (const u16*)d_pat.p, d_off.p, n_pat, d_se.p); break;
+            case 4: GRL_LAUNCH("fm_count", model, (fm_count_kernel<u32>), grid_for(n_pat, INV_THREADS), INV_THREADS, 0, st, v, (const u32*)d_pat.p, d_off.p, n_pat, d_se.p); break;
+            default: GRL_LAUNCH("fm_count", model, (fm_count_kernel<u64>), grid_for(n_pat, INV_THREADS), INV_THREADS, 0, st, v, (const u64*)d_pat.p, d_off.p, n_pat, d_se.p); break;
+        }
+    }
+    t_search.stop();
+    if (!locate) {
+        GRL_CUDA(cudaMemcpyAsync(sp_ep, d_se.p, 2 * n_pat * 8, cudaMemcpyDeviceToHost, st));
+        t_all.stop();
+        info->search_ms = t_search.ms();
+        info->device_ms = t_all.ms();  // waits for the copy
+        return;
+    }
+    DevBuf<u64> d_occ(n_pat + 1, st);
+    {
+        DevBuf<u64> cnt(n_pat, st);
+        GRL_LAUNCH("fm_occ_count", n_pat * 24, fm_occ_count_kernel, grid_for(n_pat, INV_THREADS), INV_THREADS, 0, st, d_se.p, n_pat, cnt.p);
+        exclusive_scan<u64, u64>(cnt.p, d_occ.p, n_pat, d_occ.p + n_pat, st);
+    }
+    const u64 n_occ = d2h_scalar(d_occ.p + n_pat, st);
+    info->n_occ = n_occ;
+    if (n_occ > cap_occ) throw Error(GRLGPU_ERR_ARG, "locate: the occurrences need a capacity of " + std::to_string(n_occ));
+    t_loc.start();
+    DevBuf<u32> d_id(n_occ, st), d_pos(n_occ, st), flag(1, st);
+    const bool force_walk = (c->flags & GRLGPU_FLAG_FORCE_WALK) != 0, force_jump = (c->flags & GRLGPU_FLAG_FORCE_JUMP) != 0 && !force_walk;
+    bool walk = n_occ && !force_jump && (force_walk || !x.doc_ready);  // once built, the table answers every call
+    if (walk) {  // rows off a cycle reach a separator row within n LF steps and a row < N within n psi steps: the bound n never overflows
+        const u64 B = force_walk ? x.t.n : inv_walk_bound(x.t.n);
+        flag.zero();
+        GRL_LAUNCH("fm_locate_walk", n_occ * (8 + 8 + 8 * 2) + (u64)n_occ * 32 * 16, fm_locate_walk_kernel, grid_for(n_occ, INV_THREADS), INV_THREADS, 0, st, x.t.E.p, x.psi.p,
+                   (u32)x.t.N, x.t.sep, d_se.p, d_occ.p, n_pat, n_occ, (u32)B, d_id.p, d_pos.p, flag.p);
+        if (d2h_scalar(flag.p, st)) {
+            if (force_walk) throw Error(GRLGPU_ERR_ILL_FORMED, "locate: a walk of n steps met no separator (an LF cycle without separator)");
+            walk = false;
+        }
+    }
+    info->path = (walk || !n_occ) ? 0 : 1;
+    if (n_occ && !walk) {
+        if (!x.doc_ready) info->jump_rounds = fm_build_doc(x, flag.p, st);
+        GRL_LAUNCH("fm_locate_table", n_occ * (8 + 8 + 8 + 32), fm_locate_table_kernel, grid_for(n_occ, INV_THREADS), INV_THREADS, 0, st, x.doc.p, d_se.p, d_occ.p, n_pat, n_occ,
+                   d_id.p, d_pos.p);
+    }
+    t_loc.stop();
+    GRL_CUDA(cudaMemcpyAsync(occ_off, d_occ.p, (n_pat + 1) * 8, cudaMemcpyDeviceToHost, st));
+    if (n_occ) {
+        GRL_CUDA(cudaMemcpyAsync(str_id, d_id.p, n_occ * 4, cudaMemcpyDeviceToHost, st));
+        GRL_CUDA(cudaMemcpyAsync(str_pos, d_pos.p, n_occ * 4, cudaMemcpyDeviceToHost, st));
+    }
+    t_all.stop();
+    info->search_ms = t_search.ms();
+    info->locate_ms = t_loc.ms();
+    info->device_ms = t_all.ms();  // waits for the copies
+}

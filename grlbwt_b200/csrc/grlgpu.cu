@@ -37,6 +37,25 @@ struct IndLevel {  // a kept level (device): 32-bit symbols
     DevBuf<u64> pre_len;
 };
 
+// the LF table of a .rl_bwt image (invert.cuh, part a): runs, run starts, F rows, E[j] = {LF(j) << 32 | BWT[j]}
+struct LfTable {
+    u64 n = 0, n_runs = 0, N = 0;   // BWT length, records, separators
+    u32 sep = 0;                    // smallest symbol of a non-empty record
+    DevBuf<u32> sym, len, start, F; // start has n_runs + 1 entries
+    DevBuf<u32> order;              // run indices in (symbol, run index) order
+    DevBuf<u64> E;
+};
+
+// a loaded FM-index (fm.cuh): the LF table, a symbol directory, psi, and the locate table once some call needed it
+struct FmIndex {
+    LfTable t;
+    u64 n_dir = 0;
+    DevBuf<u32> dir_sym, dir_first, dir_C;  // per distinct symbol: the symbol, its slice [dir_first[d], dir_first[d + 1]) of t.order, C[c]
+    DevBuf<u32> psi;                        // psi[LF(j)] = j
+    DevBuf<u64> doc;                        // locate table: {string << 32 | offset} for every row
+    bool doc_ready = false;
+};
+
 struct grlgpu_ctx {
     int device = 0;
     int n_sm = 148;
@@ -101,6 +120,9 @@ struct grlgpu_ctx {
     DevBuf<u8> kd_D;
     DevBuf<u32> kd_off, kd_len, kd_order, kd_phr_of;
     DevBuf<u64> kd_freq, kd_meta;
+
+    // FM-index of a .rl_bwt image (grlgpu_fm_load), at most one
+    std::unique_ptr<FmIndex> fm;
 };
 
 namespace {
@@ -752,6 +774,7 @@ void run_round_t(grlgpu_ctx* c, grlgpu_round_t* out) {
 #include "mg2.cuh"
 #include "induce.cuh"
 #include "invert.cuh"
+#include "fm.cuh"
 
 void run_round(grlgpu_ctx* c, grlgpu_round_t* out) {
     if (c->first) {
@@ -1658,17 +1681,67 @@ int grlgpu_fetch_bwt_packed(grlgpu_ctx* ctx, int sb, int fb, void* out, uint64_t
     });
 }
 
+// a .rl_bwt image the device accepts: [sb u64][fb u64] in 1..8, then a whole, non-zero number of records
+static bool image_ok(const void* image, uint64_t image_bytes) {
+    if (image_bytes < 16) return false;
+    u64 hdr[2];
+    memcpy(hdr, image, 16);
+    if (hdr[0] < 1 || hdr[0] > 8 || hdr[1] < 1 || hdr[1] > 8) return false;
+    const u64 body = image_bytes - 16;
+    return body != 0 && body % (hdr[0] + hdr[1]) == 0;
+}
+
 int grlgpu_invert(grlgpu_ctx* ctx, const void* image, uint64_t image_bytes, int cell_bytes, uint64_t n_seqs, void* out, uint64_t cap_bytes, grlgpu_invert_t* info) {
     if (!ctx || !image || !info || !(cell_bytes == 1 || cell_bytes == 2 || cell_bytes == 4 || cell_bytes == 8)) return GRLGPU_ERR_ARG;
     memset(info, 0, sizeof(*info));
-    if (image_bytes < 16) return GRLGPU_ERR_ARG;
-    u64 hdr[2];
-    memcpy(hdr, image, 16);
-    if (hdr[0] < 1 || hdr[0] > 8 || hdr[1] < 1 || hdr[1] > 8) return GRLGPU_ERR_ARG;
-    const u64 body = image_bytes - 16;
-    if (body == 0 || body % (hdr[0] + hdr[1])) return GRLGPU_ERR_ARG;
+    if (!image_ok(image, image_bytes)) return GRLGPU_ERR_ARG;
     if (!out && cap_bytes) return GRLGPU_ERR_ARG;
     return guarded(ctx, [&] { invert_image(ctx, (const u8*)image, image_bytes, cell_bytes, n_seqs, out, cap_bytes, info); });
+}
+
+int grlgpu_fm_load(grlgpu_ctx* ctx, const void* image, uint64_t image_bytes, grlgpu_fm_t* info) {
+    if (!ctx) return GRLGPU_ERR_ARG;
+    ctx->fm.reset();  // the index already loaded goes first: a failed load leaves none
+    if (!image || !info) return GRLGPU_ERR_ARG;
+    memset(info, 0, sizeof(*info));
+    if (!image_ok(image, image_bytes)) return GRLGPU_ERR_ARG;
+    return guarded(ctx, [&] { fm_load(ctx, (const u8*)image, image_bytes, info); });
+}
+
+// patterns: cell width in {1,2,4,8}, n_pat + 1 offsets from 0, each pattern at least one cell
+static int fm_patterns_ok(const void* pat, const uint64_t* pat_off, uint64_t n_pat, int pat_bytes) {
+    if (!(pat_bytes == 1 || pat_bytes == 2 || pat_bytes == 4 || pat_bytes == 8)) return GRLGPU_ERR_ARG;
+    if (n_pat == 0) return GRLGPU_OK;
+    if (!pat || !pat_off || pat_off[0] != 0) return GRLGPU_ERR_ARG;
+    for (u64 q = 0; q < n_pat; q++)
+        if (pat_off[q + 1] <= pat_off[q]) return GRLGPU_ERR_ARG;
+    return GRLGPU_OK;
+}
+
+int grlgpu_fm_count(grlgpu_ctx* ctx, const void* pat, const uint64_t* pat_off, uint64_t n_pat, int pat_bytes, uint64_t* sp_ep, grlgpu_fm_query_t* info) {
+    if (!ctx || !info) return GRLGPU_ERR_ARG;
+    memset(info, 0, sizeof(*info));
+    if (const int rc = fm_patterns_ok(pat, pat_off, n_pat, pat_bytes)) return rc;
+    if (n_pat && !sp_ep) return GRLGPU_ERR_ARG;
+    if (!ctx->fm) return GRLGPU_ERR_STATE;
+    if (n_pat == 0) return GRLGPU_OK;
+    return guarded(ctx, [&] { fm_query(ctx, pat, pat_off, n_pat, pat_bytes, sp_ep, nullptr, nullptr, nullptr, 0, info); });
+}
+
+int grlgpu_fm_locate(grlgpu_ctx* ctx, const void* pat, const uint64_t* pat_off, uint64_t n_pat, int pat_bytes, uint64_t* occ_off, uint32_t* str_id, uint32_t* str_pos,
+                     uint64_t cap_occ, grlgpu_fm_query_t* info) {
+    if (!ctx || !info) return GRLGPU_ERR_ARG;
+    memset(info, 0, sizeof(*info));
+    if (const int rc = fm_patterns_ok(pat, pat_off, n_pat, pat_bytes)) return rc;
+    if ((n_pat && !occ_off) || (cap_occ && (!str_id || !str_pos))) return GRLGPU_ERR_ARG;
+    if (!ctx->fm) return GRLGPU_ERR_STATE;
+    if (n_pat == 0) return GRLGPU_OK;
+    return guarded(ctx, [&] { fm_query(ctx, pat, pat_off, n_pat, pat_bytes, nullptr, occ_off, str_id, str_pos, cap_occ, info); });
+}
+
+int grlgpu_fm_drop(grlgpu_ctx* ctx) {
+    if (!ctx) return GRLGPU_ERR_ARG;
+    return guarded(ctx, [&] { ctx->fm.reset(); });
 }
 
 int grlgpu_profile_enable(grlgpu_ctx* ctx, int on) {

@@ -11,6 +11,7 @@
 // backwards. LF built from any run list is a permutation that maps the separator rows onto [0, N), so that chain ends within
 // n steps for every input; a run list that is not a BWT can still leave rows on cycles without a separator, which both paths
 // detect. Positions and lengths are 32-bit (n < 0xfffffff0, symbols < 2^32): larger inputs are left to the host tool.
+// Part a (lf_table_build), the walk bound and pointer jumping (inv_jump_converge) are shared with the FM-index of fm.cuh.
 // Included by grlgpu.cu inside its anonymous namespace.
 #pragma once
 
@@ -221,17 +222,40 @@ void inv_jump_scatter(const u64* E, const u64* P, const u32* owner, const u32* o
                sep, (CellT*)out, bad);
 }
 
-// The whole inversion of a checked image ([sb][fb] in 1..8, a whole number of records, at least one): fills *info, and `out`
-// when n_out * w <= cap_bytes (GRLGPU_ERR_ARG otherwise, with info->n_out set). Every buffer comes from the context's pool.
-inline void invert_image(grlgpu_ctx* c, const u8* image, u64 image_bytes, int w, u64 n_seqs, void* out, u64 cap_bytes, grlgpu_invert_t* info) {
-    cudaStream_t st = c->st;
-    Timer t_all(st), t_lf(st), t_inv(st);
-    t_all.start();
-    t_lf.start();
+// pointer jumping to convergence (part c, shared with the locate table of fm.cuh): P[j] = {steps from j to its separator row << 32 |
+// that row}; owner[] as inv_jump_init leaves it. Returns the rounds; GRLGPU_ERR_ILL_FORMED when it does not converge (the message
+// starts with `who`, the caller's name for itself).
+inline u32 inv_jump_converge(const u64* E, u32 n, u32 sep, DevBuf<u64>& P, u32* owner, u32* flag, cudaStream_t st, const char* who) {
+    GRL_LAUNCH("inv_jump_init", (u64)n * 20, inv_jump_init_kernel, grid_for(n, INV_THREADS), INV_THREADS, 0, st, E, n, sep, P.p, owner);
+    DevBuf<u64> Q(n, st);
+    // after k rounds succ = LF^(2^k) stopped at the separator row, so ceil(log2 n) rounds converge any BWT and one more
+    // moves nothing; an entry still moving after that lies on a cycle without separator
+    const u32 cap = (u32)bit_width64(n - 1) + 1;
+    bool moved = true;
+    u32 rounds = 0;
+    while (moved && rounds < cap) {  // at most cap rounds
+        GRL_CUDA(cudaMemsetAsync(flag, 0, 4, st));
+        GRL_LAUNCH("inv_jump_round", (u64)n * (8 + 32 + 8), inv_jump_round_kernel, grid_for(n, INV_THREADS), INV_THREADS, 0, st, P.p, n, Q.p, flag);
+        std::swap(P, Q);
+        rounds++;
+        moved = d2h_scalar(flag, st) != 0;
+    }
+    if (moved) throw Error(GRLGPU_ERR_ILL_FORMED, std::string(who) + ": pointer jumping did not converge (an LF cycle without separator)");
+    return rounds;
+}
+
+// the walk's step bound B = max(INV_B_MIN, n / INV_B_DIV), at most n: the inversion's count pass and fm.cuh's locate walk
+inline u64 inv_walk_bound(u64 n) { return std::min<u64>(n, std::max<u64>(INV_B_MIN, n / INV_B_DIV)); }
+
+// Part a on a checked image ([sb][fb] in 1..8, a whole number of records, at least one): decode, run starts, F rows, LF table,
+// into `t`. The inversion needs only E and frees the rest; the FM-index (fm.cuh) keeps it all. With `sorted_keys` the symbol-sorted
+// run order stays in t.order and the sorted symbols are handed over for the index's symbol directory (only when n > 0). Error
+// messages start with `who`, the caller's name for itself.
+inline void lf_table_build(const u8* image, u64 image_bytes, LfTable& t, DevBuf<u32>* sorted_keys, cudaStream_t st, const char* who) {
     const u64 sb = ((const u64*)image)[0], fb = ((const u64*)image)[1], rec = sb + fb, nr = (image_bytes - 16) / rec;
-    info->n_runs = nr;
-    // ---- a: decode, run starts, F positions, LF table ----
-    DevBuf<u32> sym(nr, st), len(nr, st);
+    t.n_runs = nr;
+    t.sym.alloc(nr, st);
+    t.len.alloc(nr, st);
     u32 h[3];  // does not fit 32 bits, largest symbol, separator
     {
         DevBuf<u8> raw(nr * rec, st);
@@ -239,47 +263,71 @@ inline void invert_image(grlgpu_ctx* c, const u8* image, u64 image_bytes, int w,
         const u32 init[3] = {0u, 0u, 0xffffffffu};
         GRL_CUDA(cudaMemcpyAsync(raw.p, image + 16, nr * rec, cudaMemcpyHostToDevice, st));
         GRL_CUDA(cudaMemcpyAsync(stv.p, init, sizeof(init), cudaMemcpyHostToDevice, st));
-        GRL_LAUNCH("inv_decode", nr * (rec + 8), inv_decode_kernel, grid_for(nr, INV_THREADS), INV_THREADS, 0, st, raw.p, nr, (int)sb, (int)fb, sym.p, len.p, stv.p);
+        GRL_LAUNCH("inv_decode", nr * (rec + 8), inv_decode_kernel, grid_for(nr, INV_THREADS), INV_THREADS, 0, st, raw.p, nr, (int)sb, (int)fb, t.sym.p, t.len.p, stv.p);
         d2h_small(h, stv.p, sizeof(h), st);  // synchronises the stream: `init` is no longer read
     }
-    if (h[0]) throw Error(GRLGPU_ERR_LIMIT, "inversion on the device: a symbol or a run length of the image does not fit 32 bits");
+    if (h[0]) throw Error(GRLGPU_ERR_LIMIT, std::string(who) + ": a symbol or a run length of the image does not fit 32 bits");
     u64 n = 0;
     {
         DevBuf<u64> start64(nr, st), tot(1, st);
-        exclusive_scan<u32, u64>(len.p, start64.p, nr, tot.p, st);
+        exclusive_scan<u32, u64>(t.len.p, start64.p, nr, tot.p, st);
         n = d2h_scalar(tot.p, st);
     }
-    if (n >= 0xfffffff0ull) throw Error(GRLGPU_ERR_LIMIT, "inversion on the device: the BWT has 2^32 symbols or more");
-    info->n = n;
-    const u32 sep = h[2];
-    DevBuf<u64> E(n, st);
-    u64 N = 0;
-    if (n) {
-        {
-            DevBuf<u64> cnt(1, st);
-            cnt.zero();
-            GRL_LAUNCH("inv_sep_count", nr * 8, inv_sep_count_kernel, grid_for(nr, INV_THREADS), INV_THREADS, 0, st, sym.p, len.p, nr, sep, cnt.p);
-            N = d2h_scalar(cnt.p, st);
-        }
-        DevBuf<u32> start(nr + 1, st), F(nr, st);
-        exclusive_scan<u32, u32>(len.p, start.p, nr, start.p + nr, st);
-        {   // stable sort of the run indices by symbol, lengths scanned in that order, scattered back to the runs
-            DevBuf<u32> keys(nr, st), keys_alt(nr, st), vals(nr, st), vals_alt(nr, st);
-            GRL_CUDA(cudaMemcpyAsync(keys.p, sym.p, nr * 4, cudaMemcpyDeviceToDevice, st));
-            GRL_LAUNCH("inv_iota", nr * 4, inv_iota_kernel, grid_for(nr, INV_THREADS), INV_THREADS, 0, st, vals.p, nr);
-            u32 *kp = keys.p, *vp = vals.p, *ka = keys_alt.p, *va = vals_alt.p;
-            radix_sort_pairs_u32(&kp, &vp, &ka, &va, nr, std::max(1, bit_width64(h[1])), st);
-            u32* fpos = ka;  // the alternate key buffer is free after the sort
-            GRL_LAUNCH("inv_sorted_len", nr * 12, inv_sorted_len_kernel, grid_for(nr, INV_THREADS), INV_THREADS, 0, st, vp, len.p, nr, fpos);
-            exclusive_scan<u32, u32>(fpos, fpos, nr, (u32*)nullptr, st);
-            GRL_LAUNCH("inv_scatter_f", nr * 12, inv_scatter_f_kernel, grid_for(nr, INV_THREADS), INV_THREADS, 0, st, vp, fpos, nr, F.p);
-            GRL_CUDA(cudaStreamSynchronize(st));
-        }
-        GRL_LAUNCH("inv_fill", n * 8 + nr * 12, inv_fill_kernel, (unsigned)div_up(n, INV_FILL_TILE), INV_THREADS, 0, st, start.p, F.p, sym.p, (u32)nr, (u32)n, E.p);
-        GRL_CUDA(cudaStreamSynchronize(st));
+    if (n >= 0xfffffff0ull) throw Error(GRLGPU_ERR_LIMIT, std::string(who) + ": the BWT has 2^32 symbols or more");
+    t.n = n;
+    t.sep = h[2];
+    t.E.alloc(n, st);
+    t.N = 0;
+    if (!n) return;
+    {
+        DevBuf<u64> cnt(1, st);
+        cnt.zero();
+        GRL_LAUNCH("inv_sep_count", nr * 8, inv_sep_count_kernel, grid_for(nr, INV_THREADS), INV_THREADS, 0, st, t.sym.p, t.len.p, nr, t.sep, cnt.p);
+        t.N = d2h_scalar(cnt.p, st);
     }
-    sym.release();
-    len.release();
+    t.start.alloc(nr + 1, st);
+    t.F.alloc(nr, st);
+    exclusive_scan<u32, u32>(t.len.p, t.start.p, nr, t.start.p + nr, st);
+    {   // stable sort of the run indices by symbol, lengths scanned in that order, scattered back to the runs
+        DevBuf<u32> keys(nr, st), keys_alt(nr, st), vals(nr, st), vals_alt(nr, st);
+        GRL_CUDA(cudaMemcpyAsync(keys.p, t.sym.p, nr * 4, cudaMemcpyDeviceToDevice, st));
+        GRL_LAUNCH("inv_iota", nr * 4, inv_iota_kernel, grid_for(nr, INV_THREADS), INV_THREADS, 0, st, vals.p, nr);
+        u32 *kp = keys.p, *vp = vals.p, *ka = keys_alt.p, *va = vals_alt.p;
+        radix_sort_pairs_u32(&kp, &vp, &ka, &va, nr, std::max(1, bit_width64(h[1])), st);
+        u32* fpos = ka;  // the alternate key buffer is free after the sort
+        GRL_LAUNCH("inv_sorted_len", nr * 12, inv_sorted_len_kernel, grid_for(nr, INV_THREADS), INV_THREADS, 0, st, vp, t.len.p, nr, fpos);
+        exclusive_scan<u32, u32>(fpos, fpos, nr, (u32*)nullptr, st);
+        GRL_LAUNCH("inv_scatter_f", nr * 12, inv_scatter_f_kernel, grid_for(nr, INV_THREADS), INV_THREADS, 0, st, vp, fpos, nr, t.F.p);
+        GRL_CUDA(cudaStreamSynchronize(st));
+        if (sorted_keys) {  // the buffers that hold the sorted symbols and the order after the sort
+            *sorted_keys = std::move(kp == keys.p ? keys : keys_alt);
+            t.order = std::move(vp == vals.p ? vals : vals_alt);
+        }
+    }
+    GRL_LAUNCH("inv_fill", n * 8 + nr * 12, inv_fill_kernel, (unsigned)div_up(n, INV_FILL_TILE), INV_THREADS, 0, st, t.start.p, t.F.p, t.sym.p, (u32)nr, (u32)n, t.E.p);
+    GRL_CUDA(cudaStreamSynchronize(st));
+}
+
+// The whole inversion of a checked image (as lf_table_build): fills *info, and `out` when n_out * w <= cap_bytes
+// (GRLGPU_ERR_ARG otherwise, with info->n_out set). Every buffer comes from the context's pool.
+inline void invert_image(grlgpu_ctx* c, const u8* image, u64 image_bytes, int w, u64 n_seqs, void* out, u64 cap_bytes, grlgpu_invert_t* info) {
+    cudaStream_t st = c->st;
+    Timer t_all(st), t_lf(st), t_inv(st);
+    t_all.start();
+    t_lf.start();
+    const u64 sb = ((const u64*)image)[0], fb = ((const u64*)image)[1];
+    info->n_runs = (image_bytes - 16) / (sb + fb);
+    // ---- a: decode, run starts, F positions, LF table ----
+    LfTable t;
+    lf_table_build(image, image_bytes, t, nullptr, st, "inversion on the device");
+    info->n = t.n;
+    t.start.release();
+    t.F.release();
+    t.sym.release();
+    t.len.release();
+    const u64 n = t.n, N = t.N;
+    const u32 sep = t.sep;
+    DevBuf<u64>& E = t.E;
     t_lf.stop();
     info->n_strings = N;
     const u32 n_req = (u32)std::min<u64>(n_seqs, N);
@@ -289,7 +337,7 @@ inline void invert_image(grlgpu_ctx* c, const u8* image, u64 image_bytes, int w,
     const bool force_walk = (c->flags & GRLGPU_FLAG_FORCE_WALK) != 0, force_jump = (c->flags & GRLGPU_FLAG_FORCE_JUMP) != 0 && !force_walk;
     bool walk = !force_jump;
     if (walk) {  // count pass: chains of rows < N end within n steps, so the bound n never overflows
-        const u64 B = force_walk ? n : std::min<u64>(n, std::max<u64>(INV_B_MIN, n / INV_B_DIV));
+        const u64 B = force_walk ? n : inv_walk_bound(n);
         flag.zero();
         GRL_LAUNCH("inv_walk_count", (u64)n_req * 4 + (n - N) * 32, inv_walk_count_kernel, grid_for(n_req, INV_THREADS), INV_THREADS, 0, st, E.p, n_req, sep, (u32)B, slen.p, flag.p);
         walk = d2h_scalar(flag.p, st) == 0;
@@ -316,24 +364,7 @@ inline void invert_image(grlgpu_ctx* c, const u8* image, u64 image_bytes, int w,
         info->path = 1;
         DevBuf<u64> P(n, st);
         DevBuf<u32> owner(n, st);
-        GRL_LAUNCH("inv_jump_init", n * 20, inv_jump_init_kernel, grid_for(n, INV_THREADS), INV_THREADS, 0, st, E.p, (u32)n, sep, P.p, owner.p);
-        {
-            DevBuf<u64> Q(n, st);
-            // after k rounds succ = LF^(2^k) stopped at the separator row, so ceil(log2 n) rounds converge any BWT and one more
-            // moves nothing; an entry still moving after that lies on a cycle without separator
-            const u32 cap = (u32)bit_width64(n - 1) + 1;
-            bool moved = true;
-            u32 rounds = 0;
-            while (moved && rounds < cap) {  // at most cap rounds
-                flag.zero();
-                GRL_LAUNCH("inv_jump_round", n * (8 + 32 + 8), inv_jump_round_kernel, grid_for(n, INV_THREADS), INV_THREADS, 0, st, P.p, (u32)n, Q.p, flag.p);
-                std::swap(P, Q);
-                rounds++;
-                moved = d2h_scalar(flag.p, st) != 0;
-            }
-            info->jump_rounds = rounds;
-            if (moved) throw Error(GRLGPU_ERR_ILL_FORMED, "inversion: pointer jumping did not converge (an LF cycle without separator)");
-        }
+        info->jump_rounds = inv_jump_converge(E.p, (u32)n, sep, P, owner.p, flag.p, st, "inversion");
         GRL_LAUNCH("inv_jump_owner", (u64)n_req * (8 + 4 + 32), inv_jump_owner_kernel, grid_for(n_req, INV_THREADS), INV_THREADS, 0, st, P.p, n_req, slen.p, owner.p);
         exclusive_scan<u32, u32>(slen.p, off.p, n_req, off.p + n_req, st);
         const u64 n_out = (u64)d2h_scalar(off.p + n_req, st) + n_req;

@@ -7,6 +7,7 @@
 #include <exception>
 #include <iostream>
 #include <map>
+#include <stdexcept>
 #include <string>
 #include <vector>
 
@@ -58,6 +59,80 @@ struct RlBwt {
         const size_t k = (size_t)(std::upper_bound(start.begin(), start.end(), i) - start.begin()) - 1;
         const uint64_t c = runs.sym[k];
         return {c, C.at(c) + before[k] + (i - start[k])};
+    }
+
+    // ---- search (fm_query): per-symbol run lists, built by index_runs() ----
+    std::vector<uint64_t> by_sym;                                  // run indices in (symbol, run index) order
+    std::map<uint64_t, std::pair<uint64_t, uint64_t>> slice;       // symbol -> its range [lo, hi) of by_sym
+    std::vector<uint64_t> c_val, c_sym;                            // C[c] and c, in symbol order
+    void index_runs() {
+        const size_t r = runs.size();
+        by_sym.resize(r);
+        uint64_t max_sym = 0;
+        for (size_t i = 0; i < r; i++) max_sym = std::max(max_sym, runs.sym[i]);
+        if (max_sym < (1ull << 26)) {  // counting sort by symbol
+            std::vector<uint64_t> first(max_sym + 2, 0);
+            for (size_t i = 0; i < r; i++) first[runs.sym[i] + 1]++;
+            for (uint64_t c = 0; c <= max_sym; c++) first[c + 1] += first[c];
+            std::vector<uint64_t> at(first.begin(), first.end() - 1);
+            for (size_t i = 0; i < r; i++) by_sym[at[runs.sym[i]]++] = i;
+        } else {
+            for (size_t i = 0; i < r; i++) by_sym[i] = i;
+            std::stable_sort(by_sym.begin(), by_sym.end(), [&](uint64_t a, uint64_t b) { return runs.sym[a] < runs.sym[b]; });
+        }
+        for (size_t q = 0; q < r;) {
+            size_t e = q;
+            while (e < r && runs.sym[by_sym[e]] == runs.sym[by_sym[q]]) e++;
+            slice[runs.sym[by_sym[q]]] = {q, e};
+            q = e;
+        }
+        for (auto& kv : C) { c_sym.push_back(kv.first); c_val.push_back(kv.second); }
+    }
+    // rank_c(BWT, i) for i in [0, n]: from the run holding i, or the last run of c before it
+    uint64_t rank(uint64_t c, uint64_t i) const {
+        const size_t k = (size_t)(std::upper_bound(start.begin(), start.end(), i) - start.begin()) - 1;  // i = n: k = r
+        if (k < runs.size() && runs.sym[k] == c) return before[k] + (i - start[k]);
+        const auto sl = slice.find(c);
+        if (sl == slice.end()) return 0;
+        const auto lo = by_sym.begin() + (long)sl->second.first;
+        const size_t m = (size_t)(std::lower_bound(lo, by_sym.begin() + (long)sl->second.second, (uint64_t)k) - lo);
+        if (m == 0) return 0;
+        const uint64_t q = *(lo + (long)(m - 1));
+        return before[q] + runs.len[q];
+    }
+    // rows [sp, ep) whose suffix starts with P; a pattern without occurrence (the separator or an absent symbol in it, or an empty
+    // interval) gives sp = ep = 0, as the device search does
+    std::pair<uint64_t, uint64_t> count(const uint64_t* P, size_t m) const {
+        uint64_t sp = 0, ep = n;
+        for (size_t a = m; a-- > 0;) {
+            const auto it = C.find(P[a]);
+            if (P[a] == sep || it == C.end()) return {0, 0};
+            sp = it->second + rank(P[a], sp);
+            ep = it->second + rank(P[a], ep);
+            if (sp >= ep) return {0, 0};
+        }
+        return {sp, ep};
+    }
+    // psi(j) = LF^-1(j): the c of F row j, then the run of c that holds its (j - C[c])-th occurrence
+    uint64_t psi(uint64_t j) const {
+        const size_t d = (size_t)(std::upper_bound(c_val.begin(), c_val.end(), j) - c_val.begin()) - 1;
+        const uint64_t x = j - c_val[d];
+        const auto sl = slice.at(c_sym[d]);
+        const auto lo = by_sym.begin() + (long)sl.first, hi = by_sym.begin() + (long)sl.second;
+        const uint64_t q = *(std::upper_bound(lo, hi, x, [&](uint64_t v, uint64_t run) { return v < before[run]; }) - 1);
+        return start[q] + (x - before[q]);
+    }
+    // occurrence at row j: string k (row k < n_strings is $_k, reached by psi) and offset p (LF steps to a separator)
+    std::pair<uint64_t, uint64_t> locate(uint64_t j) const {
+        uint64_t p = 0, r = j;
+        for (auto e = lf(r); e.first != sep; e = lf(r = e.second))
+            if (++p > n) throw std::runtime_error("the file is ill formed (an LF cycle without separator)");
+        uint64_t k = j, f = 0;
+        do {
+            if (++f > n) throw std::runtime_error("the file is ill formed (an LF cycle without separator)");
+            k = psi(k);
+        } while (k >= n_strings);
+        return {k, p};
     }
 };
 

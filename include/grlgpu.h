@@ -35,8 +35,8 @@ enum grlgpu_status {
 #define GRLGPU_FLAG_SMALL_PILOT 16ull /* tests: one pilot tile, so small inputs exercise pilot + remainder */
 #define GRLGPU_FLAG_FORCE_DOUBLING 32ull /* tests: refine suffix groups by prefix doubling even when key extension would do */
 #define GRLGPU_FLAG_KEEP_DICT 4ull /* tests: keep the last round's dictionary for grlgpu_fetch_dictionary */
-#define GRLGPU_FLAG_FORCE_WALK 64ull /* tests: grlgpu_invert walks every string, whatever the chain lengths */
-#define GRLGPU_FLAG_FORCE_JUMP 128ull /* tests: grlgpu_invert runs pointer jumping, whatever the chain lengths */
+#define GRLGPU_FLAG_FORCE_WALK 64ull /* tests: grlgpu_invert walks every string and grlgpu_fm_locate walks every occurrence, whatever the chain lengths */
+#define GRLGPU_FLAG_FORCE_JUMP 128ull /* tests: grlgpu_invert runs pointer jumping and grlgpu_fm_locate answers from its table, whatever the chain lengths */
 
 /* = str_collection (external/cdt/include/utils.h:20-28) as filled by collection_stats (utils.cpp:100-189) */
 typedef struct {
@@ -182,6 +182,45 @@ typedef struct {
 } grlgpu_invert_t;
 int grlgpu_invert(grlgpu_ctx* ctx, const void* image, uint64_t image_bytes, int cell_bytes,
                   uint64_t n_seqs /* UINT64_MAX: all */, void* out, uint64_t cap_bytes, grlgpu_invert_t* info);
+
+/* search of a BCR BWT: the .rl_bwt image loaded as a run-length FM-index on the device (grlbwt_b200/csrc/fm.cuh). The reference has
+ * no such interface (its scripts/fm_index.h only serves reverse_bwt); the host tool fm_query is the general path and the same answers.
+ * Conventions of grlgpu_invert: the separator is the smallest symbol of a non-empty record, N = its count, S_0 .. S_{N-1} the strings
+ * in the order reverse_bwt writes them (input order). An occurrence of a pattern P (m >= 1 cells) is a pair (k, p) with
+ * S_k[p .. p + m) = P; overlapping occurrences all count; a pattern containing the separator or a symbol absent from the BWT has none.
+ *   grlgpu_fm_load    builds the index from an image (checks and GRLGPU_ERR_LIMIT exactly as grlgpu_invert) and keeps it in the
+ *                     context: at most one index, so a load first drops the index already loaded (a failed load leaves none). Its
+ *                     memory comes from the context's pool; the context's text, levels and BWT are left untouched.
+ *   grlgpu_fm_count   backward search of n_pat patterns: pattern q is cells [pat_off[q], pat_off[q + 1]) of pat, cells of pat_bytes
+ *                     little-endian bytes. sp_ep[2q], sp_ep[2q + 1] = the rows [sp, ep) whose suffix starts with the pattern, its
+ *                     count ep - sp; a pattern without occurrence gets sp = ep = 0.
+ *   grlgpu_fm_locate  every occurrence: occ_off[q] .. occ_off[q + 1] (n_pat + 1 entries) are pattern q's, listed in row order
+ *                     sp, sp + 1, ..: str_id = k, str_pos = p. Each occurrence walks LF and psi from its row, at most
+ *                     B = max(4096, n / 2048) steps; a longer walk makes the call, and every later call on the index, answer from
+ *                     a table of (k, p) for every row, built once by pointer jumping (GRLGPU_FLAG_FORCE_WALK / _JUMP force one path).
+ *   grlgpu_fm_drop    frees the index (grlgpu_destroy does too).
+ * GRLGPU_ERR_ARG: pat_bytes not in {1,2,4,8}, pat_off[0] != 0, an empty pattern (offsets not increasing), cap_occ < n_occ (info->n_occ
+ * is then set to the number needed). GRLGPU_ERR_STATE: count or locate without a loaded index. GRLGPU_ERR_ILL_FORMED: the run list is
+ * not a BWT (its LF has a cycle without separator) and a locate met it. n_pat = 0 is accepted and writes nothing. */
+typedef struct {
+    uint64_t n, n_strings, n_runs;  /* BWT length, separators, records of the image */
+    uint64_t sigma;                 /* distinct symbols of the records */
+    uint64_t sep;                   /* the separator */
+    float load_ms;                  /* CUDA events on the context's stream: image upload and every table of the index */
+} grlgpu_fm_t;
+typedef struct {
+    uint64_t n_pat, n_pat_syms;     /* patterns and their cells */
+    uint64_t n_occ;                 /* locate: occurrences (written, or needed when cap_occ is too small) */
+    uint32_t path;                  /* locate: 0 walk per occurrence, 1 the table */
+    uint32_t jump_rounds;           /* locate: pointer-jumping rounds when this call built the table, else 0 */
+    float device_ms, search_ms, locate_ms; /* CUDA events on the context's stream: whole call (copies included) / backward search / locate */
+} grlgpu_fm_query_t;
+int grlgpu_fm_load(grlgpu_ctx* ctx, const void* image, uint64_t image_bytes, grlgpu_fm_t* info);
+int grlgpu_fm_count(grlgpu_ctx* ctx, const void* pat, const uint64_t* pat_off /* n_pat + 1 cell offsets */, uint64_t n_pat, int pat_bytes,
+                    uint64_t* sp_ep /* 2 * n_pat */, grlgpu_fm_query_t* info);
+int grlgpu_fm_locate(grlgpu_ctx* ctx, const void* pat, const uint64_t* pat_off, uint64_t n_pat, int pat_bytes, uint64_t* occ_off /* n_pat + 1 */,
+                     uint32_t* str_id, uint32_t* str_pos, uint64_t cap_occ, grlgpu_fm_query_t* info);
+int grlgpu_fm_drop(grlgpu_ctx* ctx);
 
 /* digest of the last round's level artefacts, computed on the device before they are fetched: four sums mod 2^64
  * {rules weighted by rank, hocc marks weighted by rank, sum of the preliminary-BWT run lengths, runs weighted by symbol}.
