@@ -161,6 +161,22 @@ def _ptr(a):
     return None if a is None else a.ctypes.data_as(C.c_void_p)
 
 
+def _carve(sizes, arena, offset):
+    """[(count, dtype)] -> (arrays, end): fresh zeroed arrays (end None) without an arena, else views of `arena` placed from byte
+    `offset` on at 16-byte boundaries, and the 16-byte aligned end of the last one"""
+    if arena is None:
+        return [np.zeros(n, dt) for n, dt in sizes], None
+    arrs, off = [], int(offset)
+    for n, dt in sizes:
+        nb = n * np.dtype(dt).itemsize
+        off = (off + 15) & ~15
+        if off + nb > arena.size:
+            raise GrlGpuError(-1, "fetch arena too small")
+        arrs.append(arena[off:off + nb].view(dt))
+        off += nb
+    return arrs, (off + 15) & ~15
+
+
 class GrlGpu:
     """One device context = the GPU parse strategy (mirrors the duck-typed strategy concept used by
     par_round, exact_par_phase.cpp:374-497: get_phrases / map / parse_text, fused into round())."""
@@ -223,25 +239,14 @@ class GrlGpu:
         st = np.uint32 if r.sym_bytes == 4 else np.uint64
         narrow = bool(narrow_len) and r.n_in + r.parse_len < (1 << 32)
         sizes = [(r.tot_phrases, st), (r.tot_phrases, st), (r.tot_phrases, np.uint8), (r.n_pre_runs, st), (r.n_pre_runs, np.uint32 if narrow else np.uint64)]
-        if arena is None:
-            arrs = [np.zeros(n, dt) for n, dt in sizes]
-        else:
-            arrs, off = [], int(offset)
-            for n, dt in sizes:
-                nb = n * np.dtype(dt).itemsize
-                off = (off + 15) & ~15
-                if off + nb > arena.size:
-                    raise GrlGpuError(-1, "fetch arena too small")
-                arrs.append(arena[off:off + nb].view(dt))
-                off += nb
-        rl, rr, hh, ps, pl = arrs
+        (rl, rr, hh, ps, pl), end = _carve(sizes, arena, offset)
         if narrow:
             self._check(self._L.grlgpu_fetch_level32(self._h, _ptr(rl), _ptr(rr), _ptr(hh), _ptr(ps), _ptr(pl), int(async_)))
         else:
             fn = self._L.grlgpu_fetch_level_async if async_ else self._L.grlgpu_fetch_level
             self._check(fn(self._h, _ptr(rl), _ptr(rr), _ptr(hh), _ptr(ps), _ptr(pl)))
         if arena is not None:
-            self.arena_end = (off + 15) & ~15
+            self.arena_end = end
         if widen and arena is None:
             rl, rr, ps = rl.astype(np.uint64), rr.astype(np.uint64), ps.astype(np.uint64)
         return {"rule_l": rl, "rule_r": rr, "has_hocc": hh, "pre_sym": ps, "pre_len": pl}
@@ -304,19 +309,9 @@ class GrlGpu:
         sl = self.mg_slice_info()
         st = np.uint32 if sl.sym_bytes == 4 else np.uint64
         sizes = [(sl.tot_local, st), (sl.tot_local, st), (sl.tot_local, np.uint8), (sl.n_pre_local, st), (sl.n_pre_local, np.uint32 if narrow_len else np.uint64)]
-        if arena is None:
-            arrs = [np.zeros(n, dt) for n, dt in sizes]
-        else:
-            arrs, off = [], int(offset)
-            for n, dt in sizes:
-                nb = n * np.dtype(dt).itemsize
-                off = (off + 15) & ~15
-                if off + nb > arena.size:
-                    raise GrlGpuError(-1, "fetch arena too small")
-                arrs.append(arena[off:off + nb].view(dt))
-                off += nb
-            self.arena_end = (off + 15) & ~15
-        rl, rr, hh, ps, pl = arrs
+        (rl, rr, hh, ps, pl), end = _carve(sizes, arena, offset)
+        if arena is not None:
+            self.arena_end = end
         self._check(self._L.grlgpu_mg_fetch_slice(self._h, _ptr(rl), _ptr(rr), _ptr(hh), _ptr(ps), _ptr(pl), 4 if narrow_len else 8, int(async_)))
         return {"rule_l": rl, "rule_r": rr, "has_hocc": hh, "pre_sym": ps, "pre_len": pl, "rank_base": sl.rank_base, "pre_first": sl.pre_first}
 

@@ -15,14 +15,37 @@
 using namespace grl;
 
 
-// level slices of the last multi-GPU round (owned by the context until the next round / fetch)
-struct Mg2Slices {
+// the artefacts of one level on the device: tot rules (rule_l / rule_r of sym_bytes each, has_hocc) and n_pre preliminary-BWT runs
+struct DevLevel {
     int sym_bytes = 4;
-    u64 rank_base = 0, tot_local = 0, tot = 0;
-    u64 pre_drop = 0, n_pre_local = 0, pre_first = 0, n_pre_global = 0;  // runs [pre_drop, pre_drop + n_pre_local) of pre_* are this rank's
+    u64 tot = 0, n_pre = 0;
     DevBuf<u8> rule_l, rule_r, has_hocc, pre_sym;
     DevBuf<u64> pre_len;
+    bool present() const { return rule_l.p != nullptr; }
+};
+
+// the level one call acts on (not owning): the last round's level, this rank's slice of a multi-GPU level, or a kept level
+struct LevelView {
+    int sym_bytes;
+    u64 tot, n_pre, rank_base;  // rank_base: global rank of the first rule (checksum weights)
+    const void *rule_l, *rule_r;
+    const u8* has_hocc;
+    const void* pre_sym;
+    const u64* pre_len;
+};
+// pre_drop: leading runs of the arrays that belong to another rank
+inline LevelView view_of(const DevLevel& L, u64 rank_base = 0, u64 pre_drop = 0) {
+    return {L.sym_bytes, L.tot, L.n_pre - pre_drop, rank_base, L.rule_l.p, L.rule_r.p, L.has_hocc.p, L.pre_sym.p + pre_drop * (u64)L.sym_bytes, L.pre_len.p + pre_drop};
+}
+
+// level slice of the last multi-GPU round (owned by the context until the next round / fetch): lvl.tot rules from global rank
+// rank_base on; runs [pre_drop, lvl.n_pre) of lvl.pre_* are this rank's and go to global run pre_first on
+struct Mg2Slices {
+    DevLevel lvl;
+    u64 rank_base = 0, tot_global = 0;
+    u64 pre_drop = 0, pre_first = 0, n_pre_global = 0;
     bool valid = false;
+    LevelView view() const { return view_of(lvl, rank_base, pre_drop); }
 };
 
 // device-side induction (induce.cuh): a level's BWT as maximal runs, and a level kept on the device for it
@@ -32,9 +55,14 @@ struct IndBwt {
 };
 
 struct IndLevel {  // a kept level (device): 32-bit symbols
-    u64 alphabet = 0, tot = 0, n_pre = 0;
-    DevBuf<u8> rule_l, rule_r, has_hocc, pre_sym;
-    DevBuf<u64> pre_len;
+    u64 alphabet = 0;
+    DevLevel lvl;
+};
+
+// a level handed over until grlgpu_fetch_wait: its arrays, and the 32-bit run lengths when the host takes those
+struct ParkedLevel {
+    DevLevel lvl;
+    DevBuf<u32> len32;
 };
 
 // the LF table of a .rl_bwt image (invert.cuh, part a): runs, run starts, F rows, E[j] = {LF(j) << 32 | BWT[j]}
@@ -84,19 +112,15 @@ struct grlgpu_ctx {
     u64 hist[256] = {0};  // byte alphabets: histogram of the (local) text
 
     // artefacts of the last round (device)
-    int lvl_sym_bytes = 4;
+    DevLevel lvl;
     u64 lvl_alphabet = 0;
-    u64 lvl_tot = 0, lvl_npre = 0, lvl_n_in = ~0ull;  // upper bound of the sum of the level's run lengths (all ones: unknown)
-    DevBuf<u8> rule_l, rule_r, has_hocc, pre_sym;
-    DevBuf<u64> pre_len;
+    u64 lvl_n_in = ~0ull;  // upper bound of the sum of the level's run lengths (all ones: unknown)
 
     // asynchronous level fetches: a second stream copies while the next round computes; the level's device buffers
     // are parked here (not returned to the pool) until grlgpu_fetch_wait
     cudaStream_t copy_st = nullptr;
     cudaEvent_t copy_ev = nullptr;
-    std::vector<DevBuf<u8>> parked_u8;
-    std::vector<DevBuf<u64>> parked_u64;
-    std::vector<DevBuf<u32>> parked_u32;
+    std::vector<ParkedLevel> parked;
 
     // streaming ingest (grlgpu_text_begin / _stage / _commit / _end): two pinned staging buffers, H2D on the copy stream
     u8* stage_buf[2] = {nullptr, nullptr};
@@ -619,7 +643,8 @@ void stage_dict(Round& R) {
     R.tot = tot;
 
     // -- preliminary BWT: maximal runs over the valid groups --
-    c->lvl_sym_bytes = sizeof(SymT);
+    DevLevel& L = c->lvl;
+    L.sym_bytes = sizeof(SymT);
     {
         DevBuf<u64> csym(nV, st), clen(nV, st);
         GRL_LAUNCH("prebwt_compact", 0, prebwt_compact_kernel, grid_for(G, 256), 256, 0, st, vflag.p, vidx.p, psym.p, gacc.p, G, csym.p, clen.p);
@@ -627,10 +652,10 @@ void stage_dict(Round& R) {
         GRL_LAUNCH("key_head_flags", 0, key_head_flags_kernel, grid_for(nV, 256), 256, 0, st, csym.p, nV, hflag.p);
         exclusive_scan<u32, u32>(hflag.p, hexcl.p, nV, nrun.p, st);
         R.n_pre = d2h_scalar(nrun.p, st);
-        c->pre_sym.alloc(R.n_pre * sizeof(SymT), st);
-        c->pre_len.alloc(R.n_pre, st);
-        c->pre_len.zero();
-        GRL_LAUNCH("prebwt_runs", 0, (prebwt_runs_kernel<SymT>), grid_for(nV, 256), 256, 0, st, csym.p, clen.p, hflag.p, hexcl.p, nV, (SymT*)c->pre_sym.p, c->pre_len.p);
+        L.pre_sym.alloc(R.n_pre * sizeof(SymT), st);
+        L.pre_len.alloc(R.n_pre, st);
+        L.pre_len.zero();
+        GRL_LAUNCH("prebwt_runs", 0, (prebwt_runs_kernel<SymT>), grid_for(nV, 256), 256, 0, st, csym.p, clen.p, hflag.p, hexcl.p, nV, (SymT*)L.pre_sym.p, L.pre_len.p);
     }
 
     // -- metasymbols, next is_suffix, hocc marks, rules --
@@ -649,15 +674,15 @@ void stage_dict(Round& R) {
         GRL_LAUNCH("pack_ginfo", G * 20, pack_ginfo_kernel, grid_for(G, 256), 256, 0, st, gcnt.p, rflag.p, rrank.p, ghead.p, G, ginfo.p);
         GRL_LAUNCH("entry_finalize", nE * 12, entry_finalize_kernel, grid_for(nE, 256), 256, 0, st, R.rank.p, nE, ginfo.p, erank.p);
     }
-    c->rule_l.alloc(tot * sizeof(SymT), st);
-    c->rule_r.alloc(tot * sizeof(SymT), st);
-    c->has_hocc.alloc(tot, st);
+    L.rule_l.alloc(tot * sizeof(SymT), st);
+    L.rule_r.alloc(tot * sizeof(SymT), st);
+    L.has_hocc.alloc(tot, st);
     const u64 alph3 = A + 3, metasym_dummy = alph3 + tot + 1;  // exact_par_phase.cpp:19-20
     // model: 16 B of sequential group records + three random 32-byte sectors per ranked group (rem, hocc mark, symbols of the representative)
     // + the rule written (2 symbols + 1 byte)
-    GRL_LAUNCH("rules", G * 16 + tot * (96 + 2 * sizeof(SymT) + 1), (rules_kernel<SymT>), grid_for(G, 256), 256, 0, st, gcnt.p, rflag.p, rrank.p, grep.p, G, D, R.rem.p, erank.p, isuf, alph3, metasym_dummy, (SymT*)c->rule_l.p, (SymT*)c->rule_r.p, c->has_hocc.p);
-    c->lvl_tot = tot;
-    c->lvl_npre = R.n_pre;
+    GRL_LAUNCH("rules", G * 16 + tot * (96 + 2 * sizeof(SymT) + 1), (rules_kernel<SymT>), grid_for(G, 256), 256, 0, st, gcnt.p, rflag.p, rrank.p, grep.p, G, D, R.rem.p, erank.p, isuf, alph3, metasym_dummy, (SymT*)L.rule_l.p, (SymT*)L.rule_r.p, L.has_hocc.p);
+    L.tot = tot;
+    L.n_pre = R.n_pre;
     // every valid dictionary entry contributes its phrase's frequency to exactly one run: the lengths of a level sum to at most
     // n + p (phrases overlap by one cell)
     c->lvl_n_in = R.n + R.p;
@@ -708,7 +733,7 @@ void finish_round(grlgpu_ctx* c, Round& R, u64 tot, u64 n_pre, u64 dict_d, u64 d
     out->n_pre_runs = n_pre;
     out->cell_bytes_in = (u32)c->w;
     out->cell_bytes_out = (u32)w_out;
-    out->sym_bytes = (u32)c->lvl_sym_bytes;
+    out->sym_bytes = (u32)c->lvl.sym_bytes;
     out->done = R.p == c->n_strings;
     out->algorithmic_bytes = R.n * (u64)c->w + R.p * (u64)w_out + dict_nE * (u64)c->w + 8 * dict_d;
     out->device_ms = t_all ? t_all->ms() : tm.all;
@@ -863,12 +888,15 @@ static __global__ void __launch_bounds__(256) level_checksum_kernel(const SymT* 
     a0 = warp_sum(a0); a1 = warp_sum(a1); a2 = warp_sum(a2); a3 = warp_sum(a3);
     if (lane_id() == 0) { atomicAdd(&acc[0], a0); atomicAdd(&acc[1], a1); atomicAdd(&acc[2], a2); atomicAdd(&acc[3], a3); }
 }
-inline void level_checksum(cudaStream_t st, int sym_bytes, const void* rl, const void* rr, const u8* hh, u64 tot, u64 rank_base, const void* ps, const u64* pl, u64 n_pre,
-                           u64* host_out4) {
+inline void level_checksum(cudaStream_t st, const LevelView& v, u64* host_out4) {
     DevBuf<u64> acc(4, st);
     acc.zero();
-    if (sym_bytes == 8) GRL_LAUNCH("level_checksum", 0, (level_checksum_kernel<u64>), 296, 256, 0, st, (const u64*)rl, (const u64*)rr, hh, tot, rank_base, (const u64*)ps, pl, n_pre, acc.p);
-    else GRL_LAUNCH("level_checksum", 0, (level_checksum_kernel<u32>), 296, 256, 0, st, (const u32*)rl, (const u32*)rr, hh, tot, rank_base, (const u32*)ps, pl, n_pre, acc.p);
+    if (v.sym_bytes == 8)
+        GRL_LAUNCH("level_checksum", 0, (level_checksum_kernel<u64>), 296, 256, 0, st, (const u64*)v.rule_l, (const u64*)v.rule_r, v.has_hocc, v.tot, v.rank_base, (const u64*)v.pre_sym,
+                   v.pre_len, v.n_pre, acc.p);
+    else
+        GRL_LAUNCH("level_checksum", 0, (level_checksum_kernel<u32>), 296, 256, 0, st, (const u32*)v.rule_l, (const u32*)v.rule_r, v.has_hocc, v.tot, v.rank_base, (const u32*)v.pre_sym,
+                   v.pre_len, v.n_pre, acc.p);
     d2h_small(host_out4, acc.p, 32, st);
 }
 
@@ -1000,102 +1028,90 @@ int grlgpu_round(grlgpu_ctx* ctx, grlgpu_round_t* out) {
     return guarded(ctx, [&] { run_round(ctx, out); });
 }
 
-int grlgpu_fetch_level(grlgpu_ctx* ctx, void* rule_l, void* rule_r, uint8_t* has_hocc, void* pre_sym, uint64_t* pre_len) {
-    if (!ctx) return GRLGPU_ERR_ARG;
-    if (ctx->round == 0 || !ctx->rule_l.p) return GRLGPU_ERR_STATE;
-    return guarded(ctx, [&] {
-        const u64 sb = (u64)ctx->lvl_sym_bytes;
-        if (rule_l) GRL_CUDA(cudaMemcpyAsync(rule_l, ctx->rule_l.p, ctx->lvl_tot * sb, cudaMemcpyDeviceToHost, ctx->st));
-        if (rule_r) GRL_CUDA(cudaMemcpyAsync(rule_r, ctx->rule_r.p, ctx->lvl_tot * sb, cudaMemcpyDeviceToHost, ctx->st));
-        if (has_hocc) GRL_CUDA(cudaMemcpyAsync(has_hocc, ctx->has_hocc.p, ctx->lvl_tot, cudaMemcpyDeviceToHost, ctx->st));
-        if (pre_sym) GRL_CUDA(cudaMemcpyAsync(pre_sym, ctx->pre_sym.p, ctx->lvl_npre * sb, cudaMemcpyDeviceToHost, ctx->st));
-        if (pre_len) GRL_CUDA(cudaMemcpyAsync(pre_len, ctx->pre_len.p, ctx->lvl_npre * 8, cudaMemcpyDeviceToHost, ctx->st));
-        GRL_CUDA(cudaStreamSynchronize(ctx->st));
-    });
-}
-
+// ---- level hand-over: every way a level leaves the context (copied to the host, parked for the fetch threads) goes through
+// copy_level and park ----
 static __global__ void __launch_bounds__(256) narrow_u64_kernel(const u64* __restrict__ in, u64 n, u32* __restrict__ out) {
     const u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) out[i] = (u32)in[i];
 }
-// Same as grlgpu_fetch_level / _async with 32-bit run lengths (the run lengths of a level sum to at most n_in + parse_len,
-// so this applies whenever that is < 2^32): 4 bytes less per preliminary-BWT run over PCIe.
-int grlgpu_fetch_level32(grlgpu_ctx* ctx, void* rule_l, void* rule_r, uint8_t* has_hocc, void* pre_sym, uint32_t* pre_len32, int async) {
-    if (!ctx) return GRLGPU_ERR_ARG;
-    if (ctx->round == 0 || !ctx->rule_l.p) return GRLGPU_ERR_STATE;
-    if (ctx->lvl_n_in >= (1ull << 32)) return GRLGPU_ERR_LIMIT;
-    return guarded(ctx, [&] {
-        cudaStream_t cs = ctx->st;
-        DevBuf<u32> len32(pre_len32 ? ctx->lvl_npre : 0, ctx->st);
-        if (pre_len32 && ctx->lvl_npre)
-            GRL_LAUNCH("narrow_u64", ctx->lvl_npre * 12, narrow_u64_kernel, grid_for(ctx->lvl_npre, 256), 256, 0, ctx->st, ctx->pre_len.p, ctx->lvl_npre, len32.p);
-        if (async) {
-            if (!ctx->copy_st) {
-                GRL_CUDA(cudaStreamCreateWithFlags(&ctx->copy_st, cudaStreamNonBlocking));
-                GRL_CUDA(cudaEventCreateWithFlags(&ctx->copy_ev, cudaEventDisableTiming));
-            }
-            GRL_CUDA(cudaEventRecord(ctx->copy_ev, ctx->st));
-            GRL_CUDA(cudaStreamWaitEvent(ctx->copy_st, ctx->copy_ev, 0));
-            cs = ctx->copy_st;
-        }
-        const u64 sb = (u64)ctx->lvl_sym_bytes;
-        if (pre_sym) GRL_CUDA(cudaMemcpyAsync(pre_sym, ctx->pre_sym.p, ctx->lvl_npre * sb, cudaMemcpyDeviceToHost, cs));
-        if (pre_len32) GRL_CUDA(cudaMemcpyAsync(pre_len32, len32.p, ctx->lvl_npre * 4, cudaMemcpyDeviceToHost, cs));
-        if (rule_l) GRL_CUDA(cudaMemcpyAsync(rule_l, ctx->rule_l.p, ctx->lvl_tot * sb, cudaMemcpyDeviceToHost, cs));
-        if (rule_r) GRL_CUDA(cudaMemcpyAsync(rule_r, ctx->rule_r.p, ctx->lvl_tot * sb, cudaMemcpyDeviceToHost, cs));
-        if (has_hocc) GRL_CUDA(cudaMemcpyAsync(has_hocc, ctx->has_hocc.p, ctx->lvl_tot, cudaMemcpyDeviceToHost, cs));
-        if (async) {
-            ctx->parked_u8.push_back(std::move(ctx->rule_l));
-            ctx->parked_u8.push_back(std::move(ctx->rule_r));
-            ctx->parked_u8.push_back(std::move(ctx->has_hocc));
-            ctx->parked_u8.push_back(std::move(ctx->pre_sym));
-            ctx->parked_u32.push_back(std::move(len32));
-            ctx->pre_len.release();
-        } else GRL_CUDA(cudaStreamSynchronize(ctx->st));
-    });
-}
-
-int grlgpu_fetch_level_async(grlgpu_ctx* ctx, void* rule_l, void* rule_r, uint8_t* has_hocc, void* pre_sym, uint64_t* pre_len) {
-    if (!ctx) return GRLGPU_ERR_ARG;
-    if (ctx->round == 0 || !ctx->rule_l.p) return GRLGPU_ERR_STATE;
-    return guarded(ctx, [&] {
-        if (!ctx->copy_st) {
-            GRL_CUDA(cudaStreamCreateWithFlags(&ctx->copy_st, cudaStreamNonBlocking));
-            GRL_CUDA(cudaEventCreateWithFlags(&ctx->copy_ev, cudaEventDisableTiming));
-        }
-        // the round that produced the level has been synchronised already; order the copy stream after it anyway
-        GRL_CUDA(cudaEventRecord(ctx->copy_ev, ctx->st));
-        GRL_CUDA(cudaStreamWaitEvent(ctx->copy_st, ctx->copy_ev, 0));
-        const u64 sb = (u64)ctx->lvl_sym_bytes;
-        if (rule_l) GRL_CUDA(cudaMemcpyAsync(rule_l, ctx->rule_l.p, ctx->lvl_tot * sb, cudaMemcpyDeviceToHost, ctx->copy_st));
-        if (rule_r) GRL_CUDA(cudaMemcpyAsync(rule_r, ctx->rule_r.p, ctx->lvl_tot * sb, cudaMemcpyDeviceToHost, ctx->copy_st));
-        if (has_hocc) GRL_CUDA(cudaMemcpyAsync(has_hocc, ctx->has_hocc.p, ctx->lvl_tot, cudaMemcpyDeviceToHost, ctx->copy_st));
-        if (pre_sym) GRL_CUDA(cudaMemcpyAsync(pre_sym, ctx->pre_sym.p, ctx->lvl_npre * sb, cudaMemcpyDeviceToHost, ctx->copy_st));
-        if (pre_len) GRL_CUDA(cudaMemcpyAsync(pre_len, ctx->pre_len.p, ctx->lvl_npre * 8, cudaMemcpyDeviceToHost, ctx->copy_st));
-        ctx->parked_u8.push_back(std::move(ctx->rule_l));
-        ctx->parked_u8.push_back(std::move(ctx->rule_r));
-        ctx->parked_u8.push_back(std::move(ctx->has_hocc));
-        ctx->parked_u8.push_back(std::move(ctx->pre_sym));
-        ctx->parked_u64.push_back(std::move(ctx->pre_len));
-    });
-}
-
-int grlgpu_level_checksum(grlgpu_ctx* ctx, uint64_t* out4) {
-    if (!ctx || !out4) return GRLGPU_ERR_ARG;
-    if (ctx->round == 0 || !ctx->rule_l.p) return GRLGPU_ERR_STATE;
-    return guarded(ctx, [&] {
-        level_checksum(ctx->st, ctx->lvl_sym_bytes, ctx->rule_l.p, ctx->rule_r.p, ctx->has_hocc.p, ctx->lvl_tot, 0, ctx->pre_sym.p, ctx->pre_len.p, ctx->lvl_npre, (u64*)out4);
-    });
-}
-
-// ---- streaming ingest: the caller fills pinned staging buffers (e.g. read() straight from the input file), the copies to the
-// device run on the copy stream while the caller fills the other buffer ----
+// the second stream of asynchronous level fetches and of the streaming ingest
 static void ensure_copy_stream(grlgpu_ctx* ctx) {
     if (!ctx->copy_st) {
         GRL_CUDA(cudaStreamCreateWithFlags(&ctx->copy_st, cudaStreamNonBlocking));
         GRL_CUDA(cudaEventCreateWithFlags(&ctx->copy_ev, cudaEventDisableTiming));
     }
 }
+// the run lengths of `v` as 32-bit values, written on the compute stream (the caller has checked that they fit)
+static DevBuf<u32> narrow_lengths(grlgpu_ctx* ctx, const LevelView& v) {
+    DevBuf<u32> len32(v.n_pre, ctx->st);
+    if (v.n_pre) GRL_LAUNCH("narrow_u64", v.n_pre * 12, narrow_u64_kernel, grid_for(v.n_pre, 256), 256, 0, ctx->st, v.pre_len, v.n_pre, len32.p);
+    return len32;
+}
+// Copies the arrays of `v` whose host destination is not null, run lengths as len_bytes (4 or 8) each. Synchronous on the
+// compute stream, or (async) queued on the copy stream behind the work queued on the compute stream so far: the copies then
+// still read the level's arrays and the returned 32-bit lengths, and the caller parks both.
+static DevBuf<u32> copy_level(grlgpu_ctx* ctx, const LevelView& v, void* rule_l, void* rule_r, u8* has_hocc, void* pre_sym, void* pre_len, int len_bytes, bool async) {
+    DevBuf<u32> len32;
+    if (pre_len && len_bytes == 4) len32 = narrow_lengths(ctx, v);
+    cudaStream_t cs = ctx->st;
+    if (async) {
+        ensure_copy_stream(ctx);
+        GRL_CUDA(cudaEventRecord(ctx->copy_ev, ctx->st));
+        GRL_CUDA(cudaStreamWaitEvent(ctx->copy_st, ctx->copy_ev, 0));
+        cs = ctx->copy_st;
+    }
+    const u64 sb = (u64)v.sym_bytes;
+    const void* lens = len32.p ? (const void*)len32.p : (const void*)v.pre_len;
+    struct Copy { void* dst; const void* src; u64 bytes; };
+    for (const Copy& c : {Copy{rule_l, v.rule_l, v.tot * sb}, Copy{rule_r, v.rule_r, v.tot * sb}, Copy{has_hocc, v.has_hocc, v.tot}, Copy{pre_sym, v.pre_sym, v.n_pre * sb},
+                          Copy{pre_len, lens, v.n_pre * (u64)len_bytes}})
+        if (c.dst) GRL_CUDA(cudaMemcpyAsync(c.dst, c.src, c.bytes, cudaMemcpyDeviceToHost, cs));
+    if (!async) GRL_CUDA(cudaStreamSynchronize(ctx->st));
+    return len32;
+}
+// Keeps a level's arrays out of the pool until grlgpu_fetch_wait. len32: the 32-bit run lengths the host takes instead of the
+// 64-bit ones; those then go back to the pool at once, since their only reader, narrow_u64, runs on the compute stream before
+// the pool can hand the memory out again.
+static void park(grlgpu_ctx* ctx, DevLevel&& L, DevBuf<u32>&& len32) {
+    if (len32.p) L.pre_len.release();
+    ctx->parked.push_back({std::move(L), std::move(len32)});
+}
+
+int grlgpu_fetch_level(grlgpu_ctx* ctx, void* rule_l, void* rule_r, uint8_t* has_hocc, void* pre_sym, uint64_t* pre_len) {
+    if (!ctx) return GRLGPU_ERR_ARG;
+    if (ctx->round == 0 || !ctx->lvl.present()) return GRLGPU_ERR_STATE;
+    return guarded(ctx, [&] { copy_level(ctx, view_of(ctx->lvl), rule_l, rule_r, has_hocc, pre_sym, pre_len, 8, false); });
+}
+
+// Same as grlgpu_fetch_level / _async with 32-bit run lengths (the run lengths of a level sum to at most n_in + parse_len,
+// so this applies whenever that is < 2^32): 4 bytes less per preliminary-BWT run over PCIe.
+int grlgpu_fetch_level32(grlgpu_ctx* ctx, void* rule_l, void* rule_r, uint8_t* has_hocc, void* pre_sym, uint32_t* pre_len32, int async) {
+    if (!ctx) return GRLGPU_ERR_ARG;
+    if (ctx->round == 0 || !ctx->lvl.present()) return GRLGPU_ERR_STATE;
+    if (ctx->lvl_n_in >= (1ull << 32)) return GRLGPU_ERR_LIMIT;
+    return guarded(ctx, [&] {
+        DevBuf<u32> len32 = copy_level(ctx, view_of(ctx->lvl), rule_l, rule_r, has_hocc, pre_sym, pre_len32, 4, async != 0);
+        if (async) park(ctx, std::move(ctx->lvl), std::move(len32));
+    });
+}
+
+int grlgpu_fetch_level_async(grlgpu_ctx* ctx, void* rule_l, void* rule_r, uint8_t* has_hocc, void* pre_sym, uint64_t* pre_len) {
+    if (!ctx) return GRLGPU_ERR_ARG;
+    if (ctx->round == 0 || !ctx->lvl.present()) return GRLGPU_ERR_STATE;
+    return guarded(ctx, [&] {
+        DevBuf<u32> len32 = copy_level(ctx, view_of(ctx->lvl), rule_l, rule_r, has_hocc, pre_sym, pre_len, 8, true);
+        park(ctx, std::move(ctx->lvl), std::move(len32));
+    });
+}
+
+int grlgpu_level_checksum(grlgpu_ctx* ctx, uint64_t* out4) {
+    if (!ctx || !out4) return GRLGPU_ERR_ARG;
+    if (ctx->round == 0 || !ctx->lvl.present()) return GRLGPU_ERR_STATE;
+    return guarded(ctx, [&] { level_checksum(ctx->st, view_of(ctx->lvl), (u64*)out4); });
+}
+
+// ---- streaming ingest: the caller fills pinned staging buffers (e.g. read() straight from the input file), the copies to the
+// device run on the copy stream while the caller fills the other buffer ----
 int grlgpu_text_begin(grlgpu_ctx* ctx, uint64_t n_syms, int sym_bytes, uint64_t stage_bytes) {
     if (!ctx || n_syms == 0 || !(sym_bytes == 1 || sym_bytes == 2 || sym_bytes == 4 || sym_bytes == 8)) return GRLGPU_ERR_ARG;
     return guarded(ctx, [&] {
@@ -1156,46 +1172,20 @@ int grlgpu_text_end(grlgpu_ctx* ctx) {
 int grlgpu_level_park(grlgpu_ctx* ctx, int len_bytes, grlgpu_level_ptrs_t* out) {
     if (!ctx || !out || !(len_bytes == 4 || len_bytes == 8)) return GRLGPU_ERR_ARG;
     const bool mg = ctx->mg_sl.valid;
-    if (!mg && (ctx->round == 0 || !ctx->rule_l.p)) return GRLGPU_ERR_STATE;
+    if (!mg && (ctx->round == 0 || !ctx->lvl.present())) return GRLGPU_ERR_STATE;
     if (!mg && len_bytes == 4 && ctx->lvl_n_in >= (1ull << 32)) return GRLGPU_ERR_LIMIT;
     return guarded(ctx, [&] {
         memset(out, 0, sizeof(*out));
-        out->device = ctx->device;
-        out->len_bytes = (uint32_t)len_bytes;
-        const u64* len64;
-        u64 n_pre;
-        if (mg) {
-            Mg2Slices& S = ctx->mg_sl;
-            out->sym_bytes = (uint32_t)S.sym_bytes; out->tot = S.tot_local; out->n_pre = S.n_pre_local;
-            out->rule_l = S.rule_l.p; out->rule_r = S.rule_r.p; out->has_hocc = S.has_hocc.p;
-            out->pre_sym = S.pre_sym.p + S.pre_drop * (u64)S.sym_bytes;
-            len64 = S.pre_len.p + S.pre_drop;
-            n_pre = S.n_pre_local;
-        } else {
-            out->sym_bytes = (uint32_t)ctx->lvl_sym_bytes; out->tot = ctx->lvl_tot; out->n_pre = ctx->lvl_npre;
-            out->rule_l = ctx->rule_l.p; out->rule_r = ctx->rule_r.p; out->has_hocc = ctx->has_hocc.p; out->pre_sym = ctx->pre_sym.p;
-            len64 = ctx->pre_len.p;
-            n_pre = ctx->lvl_npre;
-        }
-        out->pre_len = len64;
-        if (len_bytes == 4) {
-            DevBuf<u32> len32(n_pre, ctx->st);
-            if (n_pre) GRL_LAUNCH("narrow_u64", n_pre * 12, narrow_u64_kernel, grid_for(n_pre, 256), 256, 0, ctx->st, len64, n_pre, len32.p);
-            out->pre_len = len32.p;
-            ctx->parked_u32.push_back(std::move(len32));
-        }
+        const LevelView v = mg ? ctx->mg_sl.view() : view_of(ctx->lvl);
+        DevBuf<u32> len32;
+        if (len_bytes == 4) len32 = narrow_lengths(ctx, v);
         GRL_CUDA(cudaStreamSynchronize(ctx->st));
-        if (mg) {
-            Mg2Slices& S = ctx->mg_sl;
-            ctx->parked_u8.push_back(std::move(S.rule_l)); ctx->parked_u8.push_back(std::move(S.rule_r));
-            ctx->parked_u8.push_back(std::move(S.has_hocc)); ctx->parked_u8.push_back(std::move(S.pre_sym));
-            ctx->parked_u64.push_back(std::move(S.pre_len));
-            S.valid = false;
-        } else {
-            ctx->parked_u8.push_back(std::move(ctx->rule_l)); ctx->parked_u8.push_back(std::move(ctx->rule_r));
-            ctx->parked_u8.push_back(std::move(ctx->has_hocc)); ctx->parked_u8.push_back(std::move(ctx->pre_sym));
-            ctx->parked_u64.push_back(std::move(ctx->pre_len));
-        }
+        out->device = ctx->device;
+        out->sym_bytes = (uint32_t)v.sym_bytes; out->len_bytes = (uint32_t)len_bytes; out->tot = v.tot; out->n_pre = v.n_pre;
+        out->rule_l = v.rule_l; out->rule_r = v.rule_r; out->has_hocc = v.has_hocc; out->pre_sym = v.pre_sym;
+        out->pre_len = len32.p ? (const void*)len32.p : (const void*)v.pre_len;
+        park(ctx, std::move(mg ? ctx->mg_sl.lvl : ctx->lvl), std::move(len32));
+        ctx->mg_sl.valid = false;
     });
 }
 // blocking device -> host copy on a stream private to the calling thread; thread-safe, needs no context
@@ -1214,9 +1204,7 @@ int grlgpu_fetch_wait(grlgpu_ctx* ctx) {
     if (!ctx) return GRLGPU_ERR_ARG;
     return guarded(ctx, [&] {
         if (ctx->copy_st) GRL_CUDA(cudaStreamSynchronize(ctx->copy_st));
-        ctx->parked_u8.clear();
-        ctx->parked_u64.clear();
-        ctx->parked_u32.clear();
+        ctx->parked.clear();
     });
 }
 
@@ -1254,7 +1242,7 @@ int grlgpu_fetch_dictionary(grlgpu_ctx* ctx, uint64_t* syms, uint64_t* lens, uin
         const u64 d = ctx->kd_d, nE = ctx->kd_nE, nS = ctx->kd_nS;
         std::vector<u32> order(nS), phr_of(nE), off(d + 1), len(d);
         std::vector<u64> freq(d), meta(d);
-        std::vector<u8> Draw(nE * (u64)ctx->lvl_sym_bytes);
+        std::vector<u8> Draw(nE * (u64)ctx->lvl.sym_bytes);
         GRL_CUDA(cudaMemcpy(order.data(), ctx->kd_order.p, nS * 4, cudaMemcpyDeviceToHost));
         GRL_CUDA(cudaMemcpy(phr_of.data(), ctx->kd_phr_of.p, nE * 4, cudaMemcpyDeviceToHost));
         GRL_CUDA(cudaMemcpy(off.data(), ctx->kd_off.p, (d + 1) * 4, cudaMemcpyDeviceToHost));
@@ -1271,7 +1259,7 @@ int grlgpu_fetch_dictionary(grlgpu_ctx* ctx, uint64_t* syms, uint64_t* lens, uin
             if (metas) metas[k] = meta[ph];
             if (syms)
                 for (u32 t = 0; t < len[ph]; t++)
-                    syms[so + t] = ctx->lvl_sym_bytes == 4 ? ((const u32*)Draw.data())[e + t] : ((const u64*)Draw.data())[e + t];
+                    syms[so + t] = ctx->lvl.sym_bytes == 4 ? ((const u32*)Draw.data())[e + t] : ((const u64*)Draw.data())[e + t];
             so += len[ph];
             k++;
         }
@@ -1463,8 +1451,8 @@ int grlgpu_mg_slice_info(grlgpu_ctx* ctx, grlgpu_slice_t* out) {
     if (!ctx || !out) return GRLGPU_ERR_ARG;
     if (!ctx->mg_n_strings || ctx->round == 0) return GRLGPU_ERR_STATE;
     const Mg2Slices& S = ctx->mg_sl;
-    out->rank_base = S.rank_base; out->tot_local = S.tot_local; out->pre_first = S.pre_first; out->n_pre_local = S.n_pre_local;
-    out->exchange_bytes = ctx->mg_exchange_bytes; out->sym_bytes = (uint32_t)S.sym_bytes; out->reserved = 0;
+    out->rank_base = S.rank_base; out->tot_local = S.lvl.tot; out->pre_first = S.pre_first; out->n_pre_local = S.lvl.n_pre - S.pre_drop;
+    out->exchange_bytes = ctx->mg_exchange_bytes; out->sym_bytes = (uint32_t)S.lvl.sym_bytes; out->reserved = 0;
     out->n_in_local = ctx->mg_n_in_local; out->parse_len_local = ctx->mg_parse_len_local;
     return GRLGPU_OK;
 }
@@ -1474,73 +1462,38 @@ int grlgpu_mg_fetch_slice(grlgpu_ctx* ctx, void* rule_l, void* rule_r, uint8_t* 
     if (!ctx->mg_sl.valid) return GRLGPU_ERR_STATE;
     return guarded(ctx, [&] {
         Mg2Slices& S = ctx->mg_sl;
-        cudaStream_t cs = ctx->st;
-        const u64 sb = (u64)S.sym_bytes;
-        const u64* len64 = S.pre_len.p + S.pre_drop;
-        DevBuf<u32> len32((pre_len && len_bytes == 4) ? S.n_pre_local : 0, ctx->st);
-        if (pre_len && len_bytes == 4 && S.n_pre_local)
-            GRL_LAUNCH("narrow_u64", S.n_pre_local * 12, narrow_u64_kernel, grid_for(S.n_pre_local, 256), 256, 0, ctx->st, len64, S.n_pre_local, len32.p);
-        if (async) {
-            if (!ctx->copy_st) {
-                GRL_CUDA(cudaStreamCreateWithFlags(&ctx->copy_st, cudaStreamNonBlocking));
-                GRL_CUDA(cudaEventCreateWithFlags(&ctx->copy_ev, cudaEventDisableTiming));
-            }
-            GRL_CUDA(cudaEventRecord(ctx->copy_ev, ctx->st));
-            GRL_CUDA(cudaStreamWaitEvent(ctx->copy_st, ctx->copy_ev, 0));
-            cs = ctx->copy_st;
-        }
-        if (pre_sym) GRL_CUDA(cudaMemcpyAsync(pre_sym, S.pre_sym.p + S.pre_drop * sb, S.n_pre_local * sb, cudaMemcpyDeviceToHost, cs));
-        if (pre_len && len_bytes == 4) GRL_CUDA(cudaMemcpyAsync(pre_len, len32.p, S.n_pre_local * 4, cudaMemcpyDeviceToHost, cs));
-        if (pre_len && len_bytes == 8) GRL_CUDA(cudaMemcpyAsync(pre_len, len64, S.n_pre_local * 8, cudaMemcpyDeviceToHost, cs));
-        if (rule_l) GRL_CUDA(cudaMemcpyAsync(rule_l, S.rule_l.p, S.tot_local * sb, cudaMemcpyDeviceToHost, cs));
-        if (rule_r) GRL_CUDA(cudaMemcpyAsync(rule_r, S.rule_r.p, S.tot_local * sb, cudaMemcpyDeviceToHost, cs));
-        if (has_hocc) GRL_CUDA(cudaMemcpyAsync(has_hocc, S.has_hocc.p, S.tot_local, cudaMemcpyDeviceToHost, cs));
-        if (async) {  // parked until grlgpu_fetch_wait; the slices cannot be fetched again
-            ctx->parked_u8.push_back(std::move(S.rule_l));
-            ctx->parked_u8.push_back(std::move(S.rule_r));
-            ctx->parked_u8.push_back(std::move(S.has_hocc));
-            ctx->parked_u8.push_back(std::move(S.pre_sym));
-            ctx->parked_u64.push_back(std::move(S.pre_len));
-            ctx->parked_u32.push_back(std::move(len32));
+        DevBuf<u32> len32 = copy_level(ctx, S.view(), rule_l, rule_r, has_hocc, pre_sym, pre_len, len_bytes, async != 0);
+        if (async) {  // the slice cannot be fetched again
+            park(ctx, std::move(S.lvl), std::move(len32));
             S.valid = false;
-        } else GRL_CUDA(cudaStreamSynchronize(ctx->st));
+        }
     });
 }
 
 int grlgpu_mg_slice_checksum(grlgpu_ctx* ctx, uint64_t* out4) {
     if (!ctx || !out4) return GRLGPU_ERR_ARG;
     if (!ctx->mg_sl.valid) return GRLGPU_ERR_STATE;
-    return guarded(ctx, [&] {
-        const Mg2Slices& S = ctx->mg_sl;
-        level_checksum(ctx->st, S.sym_bytes, S.rule_l.p, S.rule_r.p, S.has_hocc.p, S.tot_local, S.rank_base, S.pre_sym.p + S.pre_drop * (u64)S.sym_bytes, S.pre_len.p + S.pre_drop,
-                       S.n_pre_local, (u64*)out4);
-    });
+    return guarded(ctx, [&] { level_checksum(ctx->st, ctx->mg_sl.view(), (u64*)out4); });
 }
 
 // ---- induction phase on the device (induce.cuh) ----
 int grlgpu_keep_level(grlgpu_ctx* ctx) {
     if (!ctx) return GRLGPU_ERR_ARG;
-    if (ctx->round == 0 || !ctx->rule_l.p) return GRLGPU_ERR_STATE;
-    if (ctx->lvl_sym_bytes != 4) return GRLGPU_ERR_LIMIT;
-    return guarded(ctx, [&] {
-        IndLevel L;
-        L.alphabet = ctx->lvl_alphabet; L.tot = ctx->lvl_tot; L.n_pre = ctx->lvl_npre;
-        L.rule_l = std::move(ctx->rule_l); L.rule_r = std::move(ctx->rule_r); L.has_hocc = std::move(ctx->has_hocc);
-        L.pre_sym = std::move(ctx->pre_sym); L.pre_len = std::move(ctx->pre_len);
-        ctx->kept.push_back(std::move(L));
-    });
+    if (ctx->round == 0 || !ctx->lvl.present()) return GRLGPU_ERR_STATE;
+    if (ctx->lvl.sym_bytes != 4) return GRLGPU_ERR_LIMIT;
+    return guarded(ctx, [&] { ctx->kept.push_back({ctx->lvl_alphabet, std::move(ctx->lvl)}); });
 }
 int grlgpu_level_adopt(grlgpu_ctx* ctx, uint64_t alphabet, uint64_t tot, uint64_t n_pre, grlgpu_level_ptrs_t* out) {
     if (!ctx || !out) return GRLGPU_ERR_ARG;
     return guarded(ctx, [&] {
-        IndLevel L;
-        L.alphabet = alphabet; L.tot = tot; L.n_pre = n_pre;
+        DevLevel L;
+        L.tot = tot; L.n_pre = n_pre;
         L.rule_l.alloc(tot * 4, ctx->st); L.rule_r.alloc(tot * 4, ctx->st); L.has_hocc.alloc(tot, ctx->st);
         L.pre_sym.alloc(n_pre * 4, ctx->st); L.pre_len.alloc(n_pre, ctx->st);
         memset(out, 0, sizeof(*out));
         out->rule_l = L.rule_l.p; out->rule_r = L.rule_r.p; out->has_hocc = L.has_hocc.p; out->pre_sym = L.pre_sym.p; out->pre_len = L.pre_len.p;
         out->tot = tot; out->n_pre = n_pre; out->sym_bytes = 4; out->len_bytes = 8; out->device = ctx->device;
-        ctx->kept.push_back(std::move(L));
+        ctx->kept.push_back({alphabet, std::move(L)});
         GRL_CUDA(cudaStreamSynchronize(ctx->st));
     });
 }
@@ -1563,16 +1516,11 @@ int grlgpu_fetch_kept_level(grlgpu_ctx* ctx, int level, uint64_t* alphabet, uint
                             uint64_t* pre_len) {
     if (!ctx || level < 0 || (size_t)level >= ctx->kept.size()) return GRLGPU_ERR_ARG;
     return guarded(ctx, [&] {
-        const IndLevel& L = ctx->kept[(size_t)level];
-        if (alphabet) *alphabet = L.alphabet;
-        if (tot) *tot = L.tot;
-        if (n_pre) *n_pre = L.n_pre;
-        if (rule_l) GRL_CUDA(cudaMemcpyAsync(rule_l, L.rule_l.p, L.tot * 4, cudaMemcpyDeviceToHost, ctx->st));
-        if (rule_r) GRL_CUDA(cudaMemcpyAsync(rule_r, L.rule_r.p, L.tot * 4, cudaMemcpyDeviceToHost, ctx->st));
-        if (has_hocc) GRL_CUDA(cudaMemcpyAsync(has_hocc, L.has_hocc.p, L.tot, cudaMemcpyDeviceToHost, ctx->st));
-        if (pre_sym) GRL_CUDA(cudaMemcpyAsync(pre_sym, L.pre_sym.p, L.n_pre * 4, cudaMemcpyDeviceToHost, ctx->st));
-        if (pre_len) GRL_CUDA(cudaMemcpyAsync(pre_len, L.pre_len.p, L.n_pre * 8, cudaMemcpyDeviceToHost, ctx->st));
-        GRL_CUDA(cudaStreamSynchronize(ctx->st));
+        const IndLevel& K = ctx->kept[(size_t)level];
+        if (alphabet) *alphabet = K.alphabet;
+        if (tot) *tot = K.lvl.tot;
+        if (n_pre) *n_pre = K.lvl.n_pre;
+        copy_level(ctx, view_of(K.lvl), rule_l, rule_r, has_hocc, pre_sym, pre_len, 8, false);
     });
 }
 int grlgpu_drop_kept(grlgpu_ctx* ctx) {
@@ -1650,10 +1598,7 @@ int grlgpu_fetch_bwt_packed(grlgpu_ctx* ctx, int sb, int fb, void* out, uint64_t
         const u64 hdr[2] = {(u64)sb, (u64)fb};
         memcpy(out, hdr, 16);
         if (n == 0) return;
-        if (!ctx->copy_st) {
-            GRL_CUDA(cudaStreamCreateWithFlags(&ctx->copy_st, cudaStreamNonBlocking));
-            GRL_CUDA(cudaEventCreateWithFlags(&ctx->copy_ev, cudaEventDisableTiming));
-        }
+        ensure_copy_stream(ctx);
         const u64 piece = std::min<u64>(n, (u64)IND_PACK_RUNS * 32768);  // 32 M runs
         DevBuf<u8> buf0(piece * rec, st), buf1(piece * rec, st);
         DevBuf<u32> err(1, st);

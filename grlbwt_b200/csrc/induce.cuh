@@ -217,8 +217,9 @@ inline void ind_maximal_runs(const u32* sym, const u32* off, u32 n, u32 total, I
 }
 
 // one level step BWT_{i+1} -> BWT_i; throws GRLGPU_ERR_STATE when the level's artefacts disagree
-inline void ind_level_step(IndBwt& bwt, const IndLevel& L, cudaStream_t st, bool trace) {
-    const u32 A = (u32)L.alphabet, alph3 = A + 3, bwt_dummy = A + 1, hocc_dummy = A + 2;
+inline void ind_level_step(IndBwt& bwt, const IndLevel& K, cudaStream_t st, bool trace) {
+    const DevLevel& L = K.lvl;
+    const u32 A = (u32)K.alphabet, alph3 = A + 3, bwt_dummy = A + 1, hocc_dummy = A + 2;
     const u32 m = bwt.n_runs, n_pre = (u32)L.n_pre;
     const u32* rule_l = (const u32*)L.rule_l.p;
     const u32* rule_r = (const u32*)L.rule_r.p;

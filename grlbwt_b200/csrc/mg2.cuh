@@ -600,7 +600,7 @@ void mg2_rank(grlgpu_ctx* c, Comm& cm, Mg2Part& P, Mg2Slices& S) {
     const u64 tot_local = hc[0], nV = hc[1];
     if (tot_local >= (1ull << 30)) throw Error(GRLGPU_ERR_LIMIT, "more than 2^30 ranks in one rank's key range");
     u64 n_pre_raw = 0;
-    S.sym_bytes = sizeof(SymT);
+    S.lvl.sym_bytes = sizeof(SymT);
     {
         DevBuf<u64> csym(nV, st), clen(nV, st);
         GRL_LAUNCH("prebwt_compact", 0, prebwt_compact_kernel, grid_for(Gn, 256), 256, 0, st, vflag.p, vidx.p, psym.p, gacc.p, Gn, csym.p, clen.p);
@@ -608,10 +608,10 @@ void mg2_rank(grlgpu_ctx* c, Comm& cm, Mg2Part& P, Mg2Slices& S) {
         GRL_LAUNCH("key_head_flags", 0, key_head_flags_kernel, grid_for(nV, 256), 256, 0, st, csym.p, nV, hflag.p);
         exclusive_scan<u32, u32>(hflag.p, hexcl.p, nV, nrun.p, st);
         n_pre_raw = nV ? d2h_scalar(nrun.p, st) : 0;
-        S.pre_sym.alloc(n_pre_raw * sizeof(SymT), st);
-        S.pre_len.alloc(n_pre_raw, st);
-        S.pre_len.zero();
-        GRL_LAUNCH("prebwt_runs", 0, (prebwt_runs_kernel<SymT>), grid_for(nV, 256), 256, 0, st, csym.p, clen.p, hflag.p, hexcl.p, nV, (SymT*)S.pre_sym.p, S.pre_len.p);
+        S.lvl.pre_sym.alloc(n_pre_raw * sizeof(SymT), st);
+        S.lvl.pre_len.alloc(n_pre_raw, st);
+        S.lvl.pre_len.zero();
+        GRL_LAUNCH("prebwt_runs", 0, (prebwt_runs_kernel<SymT>), grid_for(nV, 256), 256, 0, st, csym.p, clen.p, hflag.p, hexcl.p, nV, (SymT*)S.lvl.pre_sym.p, S.lvl.pre_len.p);
         GRL_CUDA(cudaStreamSynchronize(st));
     }
     // rank offsets and the seams of the preliminary BWT: equal symbols can only meet where two ranges meet
@@ -622,9 +622,9 @@ void mg2_rank(grlgpu_ctx* c, Comm& cm, Mg2Part& P, Mg2Slices& S) {
         mine[1] = n_pre_raw;
         if (n_pre_raw) {
             SymT fs, ls;
-            d2h_small(&fs, (const SymT*)S.pre_sym.p, sizeof(SymT), st);
-            d2h_small(&ls, (const SymT*)S.pre_sym.p + (n_pre_raw - 1), sizeof(SymT), st);
-            d2h_small(&mine[3], S.pre_len.p, 8, st);
+            d2h_small(&fs, (const SymT*)S.lvl.pre_sym.p, sizeof(SymT), st);
+            d2h_small(&ls, (const SymT*)S.lvl.pre_sym.p + (n_pre_raw - 1), sizeof(SymT), st);
+            d2h_small(&mine[3], S.lvl.pre_len.p, 8, st);
             mine[2] = (u64)fs;
             mine[4] = (u64)ls;
         }
@@ -652,19 +652,19 @@ void mg2_rank(grlgpu_ctx* c, Comm& cm, Mg2Part& P, Mg2Slices& S) {
             S.n_pre_global += keep;
         }
         S.pre_drop = drop[(size_t)me];
-        S.n_pre_local = n_pre_raw - S.pre_drop;
-        if (add[(size_t)me]) GRL_LAUNCH("mg_add_u64", 0, mg2_add_u64_kernel, 1, 32, 0, st, S.pre_len.p + (n_pre_raw - 1), add[(size_t)me]);
+        S.lvl.n_pre = n_pre_raw;
+        if (add[(size_t)me]) GRL_LAUNCH("mg_add_u64", 0, mg2_add_u64_kernel, 1, 32, 0, st, S.lvl.pre_len.p + (n_pre_raw - 1), add[(size_t)me]);
     }
     S.rank_base = bases[(size_t)me];
-    S.tot_local = tot_local;
-    S.tot = bases[(size_t)G];
+    S.lvl.tot = tot_local;
+    S.tot_global = bases[(size_t)G];
     clk.lap("G groups + pre-BWT");
     // ---- E3: one code per entry back to its owner ----
     DevBuf<u64> ecode(nE, st);
     {
         DevBuf<u32> ginfo(Gn, st);
         GRL_LAUNCH("pack_ginfo_dense", Gn * 16, pack_ginfo_dense_kernel, grid_for(Gn, 256), 256, 0, st, gcnt.p, rflag.p, rrank.p, Gn, ginfo.p);
-        const bool narrow_code = S.tot < (1ull << 29);  // ((rank << 2) | flags) + 1 fits 32 bits
+        const bool narrow_code = S.tot_global < (1ull << 29);  // ((rank << 2) | flags) + 1 fits 32 bits
         const u64 cb = narrow_code ? 4 : 8;
         DevBuf<u8> codes(nL * cb, st), back(nS * cb, st);
         codes.zero();
@@ -695,10 +695,10 @@ void mg2_rank(grlgpu_ctx* c, Comm& cm, Mg2Part& P, Mg2Slices& S) {
         exclusive_scan<u32, u32>(rfl.p, rex.p, nE, rc.p, st);
         nR = d2h_scalar(rc.p, st);
     }
-    const u64 alph3 = A + 3, metasym_dummy = alph3 + S.tot + 1;  // exact_par_phase.cpp:19-20
+    const u64 alph3 = A + 3, metasym_dummy = alph3 + S.tot_global + 1;  // exact_par_phase.cpp:19-20
     std::vector<u64> rs_cnt, rr_cnt;
     {
-        const bool narrow_u = S.tot < (1ull << 32);
+        const bool narrow_u = S.tot_global < (1ull << 32);
         const u64 ub = narrow_u ? 4 : 8;
         const bool zip = narrow_u && sizeof(SymT) == 4;  // 32-bit symbols and ranks: the rules travel through the sort as 16-byte records
         DevBuf<u64> ru(zip ? 0 : nR, st);
@@ -719,7 +719,7 @@ void mg2_rank(grlgpu_ctx* c, Comm& cm, Mg2Part& P, Mg2Slices& S) {
             DevBuf<u32> sv(nR, st), sv_alt(nR, st);
             if (nR) GRL_LAUNCH("mg_iota", nR * 4, mg2_iota_kernel, grid_for(nR, 256), 256, 0, st, sv.p, nR);
             u32 *vp = sv.p, *va = sv_alt.p;
-            const int rank_bits = std::max(1, bit_width64(S.tot));
+            const int rank_bits = std::max(1, bit_width64(S.tot_global));
             if (zip) {
                 DevBuf<u32> k32_alt(nR, st);
                 u32 *kp = k32.p, *ka = k32_alt.p;
@@ -758,16 +758,16 @@ void mg2_rank(grlgpu_ctx* c, Comm& cm, Mg2Part& P, Mg2Slices& S) {
         if (mR != tot_local) throw Error(GRLGPU_ERR_STATE, "multi-GPU round: " + std::to_string(mR) + " rules arrived for " + std::to_string(tot_local) + " ranks of this range");
         DevBuf<u8> qu(mR * ub, st), ql(mR * sizeof(SymT), st), qr(mR * sizeof(SymT), st), qh(mR, st);
         mg2_a2a_soa(cm, {{su.p, qu.p, ub}, {sl.p, ql.p, sizeof(SymT)}, {sr.p, qr.p, sizeof(SymT)}, {sh.p, qh.p, 1}}, rs_cnt, rr_cnt, st);
-        S.rule_l.alloc(tot_local * sizeof(SymT), st);
-        S.rule_r.alloc(tot_local * sizeof(SymT), st);
-        S.has_hocc.alloc(tot_local, st);
+        S.lvl.rule_l.alloc(tot_local * sizeof(SymT), st);
+        S.lvl.rule_r.alloc(tot_local * sizeof(SymT), st);
+        S.lvl.has_hocc.alloc(tot_local, st);
         if (mR) {
             if (narrow_u)
                 GRL_LAUNCH("mg_rule_scatter", mR * 2 * (9 + 2 * sizeof(SymT)), (mg2_rule_scatter_kernel<SymT, u32>), grid_for(mR, 256), 256, 0, st, (const u32*)qu.p, (const SymT*)ql.p,
-                           (const SymT*)qr.p, qh.p, mR, S.rank_base, tot_local, (SymT*)S.rule_l.p, (SymT*)S.rule_r.p, S.has_hocc.p, err.p);
+                           (const SymT*)qr.p, qh.p, mR, S.rank_base, tot_local, (SymT*)S.lvl.rule_l.p, (SymT*)S.lvl.rule_r.p, S.lvl.has_hocc.p, err.p);
             else
                 GRL_LAUNCH("mg_rule_scatter", mR * 2 * (9 + 2 * sizeof(SymT)), (mg2_rule_scatter_kernel<SymT, u64>), grid_for(mR, 256), 256, 0, st, (const u64*)qu.p, (const SymT*)ql.p,
-                           (const SymT*)qr.p, qh.p, mR, S.rank_base, tot_local, (SymT*)S.rule_l.p, (SymT*)S.rule_r.p, S.has_hocc.p, err.p);
+                           (const SymT*)qr.p, qh.p, mR, S.rank_base, tot_local, (SymT*)S.lvl.rule_l.p, (SymT*)S.lvl.rule_r.p, S.lvl.has_hocc.p, err.p);
         }
         if (d2h_scalar(err.p, st)) throw Error(GRLGPU_ERR_STATE, "multi-GPU round: a phrase came back unranked or a rule left its rank range");
     }
@@ -937,8 +937,9 @@ void mg2_round_t(grlgpu_ctx* c, Comm& cm, grlgpu_round_t* out) {
     RoundTimes tm;
     tm.text = t_text.ms();
     tm.dict = t_dict.ms();
-    c->lvl_sym_bytes = S.sym_bytes;
-    finish_round(c, R, S.tot, S.n_pre_global, d_g, nE_g, maxf_g, tm, &t_all, out);
+    c->lvl = DevLevel();  // the level lives in the slices
+    c->lvl.sym_bytes = S.lvl.sym_bytes;
+    finish_round(c, R, S.tot_global, S.n_pre_global, d_g, nE_g, maxf_g, tm, &t_all, out);
     clk.lap("rewrite");
     out->done = done_global ? 1u : 0u;  // the phase ends when EVERY rank's strings are single cells
     c->done = done_global;
@@ -949,8 +950,7 @@ void mg2_round_t(grlgpu_ctx* c, Comm& cm, grlgpu_round_t* out) {
     out->parse_len = parse_total;
     // this rank's share of B_r (SURVEY.md 8d): its text in, its parse out, its partition of the dictionary
     out->algorithmic_bytes = R.n * (u64)out->cell_bytes_in + R.p * (u64)out->cell_bytes_out + nE_part * (u64)out->cell_bytes_in + 8 * d_part;
-    c->rule_l.release(); c->rule_r.release(); c->has_hocc.release(); c->pre_sym.release(); c->pre_len.release();  // the level lives in the slices
-    c->lvl_tot = 0; c->lvl_npre = 0; c->lvl_n_in = ~0ull;
+    c->lvl_n_in = ~0ull;
     c->is_suffix.release();
     c->mg_exchange_bytes = cm.bytes_sent - sent0;
 }

@@ -165,34 +165,29 @@ inline double load_text(const CtxHandle& ctx, const TextSource& src, int sym_byt
         return ms_since(t0);
     }
     ctx.check("grlgpu_text_begin", grlgpu_text_begin(ctx.p, src.bytes / (uint64_t)sym_bytes, sym_bytes, 0));
-    int fd = -1;
-    if (!src.mem) {
-        fd = open(src.file.c_str(), O_RDONLY);
-        if (fd < 0) throw std::runtime_error("cannot open " + src.file);
-        posix_fadvise(fd, (off_t)src.offset, (off_t)src.bytes, POSIX_FADV_SEQUENTIAL);
-    }
+    const int fd = open(src.file.c_str(), O_RDONLY);
+    if (fd < 0) throw std::runtime_error("cannot open " + src.file);
+    posix_fadvise(fd, (off_t)src.offset, (off_t)src.bytes, POSIX_FADV_SEQUENTIAL);
     try {
         for (uint64_t done = 0; done < src.bytes;) {
             void* buf = nullptr;
             uint64_t cap = 0;
             ctx.check("grlgpu_text_stage", grlgpu_text_stage(ctx.p, &buf, &cap));
             uint64_t got = 0;
-            if (src.mem) { memcpy(buf, src.mem + src.offset + done, cap); got = cap; }
-            else
-                while (got < cap) {
-                    const ssize_t r = pread(fd, (char*)buf + got, cap - got, (off_t)(src.offset + done + got));
-                    if (r <= 0) throw std::runtime_error("cannot read " + src.file);
-                    got += (uint64_t)r;
-                }
+            while (got < cap) {
+                const ssize_t r = pread(fd, (char*)buf + got, cap - got, (off_t)(src.offset + done + got));
+                if (r <= 0) throw std::runtime_error("cannot read " + src.file);
+                got += (uint64_t)r;
+            }
             ctx.check("grlgpu_text_commit", grlgpu_text_commit(ctx.p, got));
             done += got;
         }
         ctx.check("grlgpu_text_end", grlgpu_text_end(ctx.p));
     } catch (...) {
-        if (fd >= 0) close(fd);
+        close(fd);
         throw;
     }
-    if (fd >= 0) close(fd);
+    close(fd);
     return ms_since(t0);
 }
 
@@ -349,6 +344,52 @@ inline void widen_levels(ParseResult& res) {
     res.wide = true;
 }
 
+// the collected levels in round order into res.levels32, or into res.levels from the first wide level on (every level then
+// moves to 64-bit symbols)
+inline void collect_levels(std::vector<std::unique_ptr<LevelSink>>& sinks, ParseResult& res) {
+    res.wide = false;
+    for (auto& s : sinks) {
+        if (!s->wide) res.levels32.push_back(std::move(s->l32));
+        else {
+            if (!res.wide) widen_levels(res);
+            res.levels.push_back(std::move(s->l64));
+        }
+    }
+}
+
+// every level kept on the device, copied to the host (the device induction is not going to consume them); drops them there
+inline std::vector<Level32> fetch_kept_levels(const CtxHandle& ctx) {
+    std::vector<Level32> out;
+    for (int lv = 0; lv < grlgpu_kept_levels(ctx.p); lv++) {
+        Level32 L;
+        uint64_t A = 0, tot = 0, n_pre = 0;
+        ctx.check("grlgpu_fetch_kept_level", grlgpu_fetch_kept_level(ctx.p, lv, &A, &tot, &n_pre, nullptr, nullptr, nullptr, nullptr, nullptr));
+        L.alphabet = A; L.tot_phrases = tot;
+        L.rule_l.resize(tot); L.rule_r.resize(tot); L.has_hocc.resize(tot); L.pre_sym.resize(n_pre); L.pre_len.resize(n_pre);
+        ctx.check("grlgpu_fetch_kept_level", grlgpu_fetch_kept_level(ctx.p, lv, nullptr, nullptr, nullptr, L.rule_l.data(), L.rule_r.data(), L.has_hocc.data(), L.pre_sym.data(),
+                                                                    (uint64_t*)L.pre_len.data()));
+        out.push_back(std::move(L));
+    }
+    grlgpu_drop_kept(ctx.p);
+    return out;
+}
+
+// n cells of `width` bytes each -> 64-bit values
+inline void decode_cells(const unsigned char* raw, uint64_t n, uint32_t width, uint64_t* dst) {
+    for (uint64_t i = 0; i < n; i++) {
+        uint64_t v = 0;
+        memcpy(&v, raw + i * width, width);
+        dst[i] = v;
+    }
+}
+
+// the sizes of a round's digest (the checksums are added by the caller)
+inline RoundDigest digest_of(const grlgpu_round_t& r) {
+    RoundDigest dg;
+    dg.tot = r.tot_phrases; dg.n_pre = r.n_pre_runs; dg.parse_len = r.parse_len; dg.n_phrases = r.n_phrases; dg.dict_syms = r.dict_syms;
+    return dg;
+}
+
 // header widths of the level-0 BWT (exact_ind_phase.cpp:274-276 with the level-0 dictionary: alphabet = max_sym+1+3,
 // prev_alphabet = 0, max_sym_freq from collection_stats; SURVEY.md App. C)
 inline void header_widths(const grlgpu_stats_t& stats, uint64_t& sb, uint64_t& fb) {
@@ -400,17 +441,7 @@ inline bool induce_on_device(const CtxHandle& ctx, ParseResult& res, const void*
     if (verbose) { printf("  (the device cannot hold the induction of this collection: %s; inducing on the host)\n", grlgpu_last_error(ctx.p)); fflush(stdout); }
     const int n_kept = grlgpu_kept_levels(ctx.p);  // the levels the failed attempt had not consumed yet are still there: all of them, it fails before consuming
     if (n_kept != (int)res.rounds.size()) throw GpuError(rc, std::string("grlgpu_induce: ") + grlgpu_strerror(rc) + " (" + grlgpu_last_error(ctx.p) + ")");
-    for (int lv = 0; lv < n_kept; lv++) {
-        Level32 L;
-        uint64_t A = 0, tot = 0, n_pre = 0;
-        ctx.check("grlgpu_fetch_kept_level", grlgpu_fetch_kept_level(ctx.p, lv, &A, &tot, &n_pre, nullptr, nullptr, nullptr, nullptr, nullptr));
-        L.alphabet = A; L.tot_phrases = tot;
-        L.rule_l.resize(tot); L.rule_r.resize(tot); L.has_hocc.resize(tot); L.pre_sym.resize(n_pre); L.pre_len.resize(n_pre);
-        ctx.check("grlgpu_fetch_kept_level", grlgpu_fetch_kept_level(ctx.p, lv, nullptr, nullptr, nullptr, L.rule_l.data(), L.rule_r.data(), L.has_hocc.data(), L.pre_sym.data(),
-                                                                    (uint64_t*)L.pre_len.data()));
-        res.levels32.push_back(std::move(L));
-    }
-    grlgpu_drop_kept(ctx.p);
+    res.levels32 = fetch_kept_levels(ctx);
     return false;
 }
 
@@ -431,8 +462,7 @@ inline ParseResult gpu_par_phase(const TextSource& src, int sym_bytes, int devic
     for (;;) {
         grlgpu_round_t r;
         ctx.check("grlgpu_round", grlgpu_round(ctx.p, &r));
-        RoundDigest dg;
-        dg.tot = r.tot_phrases; dg.n_pre = r.n_pre_runs; dg.parse_len = r.parse_len; dg.n_phrases = r.n_phrases; dg.dict_syms = r.dict_syms;
+        RoundDigest dg = digest_of(r);
         ctx.check("grlgpu_level_checksum", grlgpu_level_checksum(ctx.p, dg.cs));
         res.digests.push_back(dg);
         if (dev_induction && r.sym_bytes == 4) {
@@ -440,17 +470,10 @@ inline ParseResult gpu_par_phase(const TextSource& src, int sym_bytes, int devic
         } else {
             if (dev_induction) {  // a wide level: the whole induction goes to the host; move what was kept so far
                 dev_induction = false;
-                for (int lv = 0; lv < grlgpu_kept_levels(ctx.p); lv++) {
-                    uint64_t A = 0, tot = 0, n_pre = 0;
-                    ctx.check("grlgpu_fetch_kept_level", grlgpu_fetch_kept_level(ctx.p, lv, &A, &tot, &n_pre, nullptr, nullptr, nullptr, nullptr, nullptr));
+                for (Level32& L : fetch_kept_levels(ctx)) {
                     sinks.emplace_back(new LevelSink());
-                    Level32& L = sinks.back()->l32;
-                    L.alphabet = A; L.tot_phrases = tot;
-                    L.rule_l.resize(tot); L.rule_r.resize(tot); L.has_hocc.resize(tot); L.pre_sym.resize(n_pre); L.pre_len.resize(n_pre);
-                    ctx.check("grlgpu_fetch_kept_level", grlgpu_fetch_kept_level(ctx.p, lv, nullptr, nullptr, nullptr, L.rule_l.data(), L.rule_r.data(), L.has_hocc.data(),
-                                                                                L.pre_sym.data(), (uint64_t*)L.pre_len.data()));
+                    sinks.back()->l32 = std::move(L);
                 }
-                grlgpu_drop_kept(ctx.p);
             }
             // the copies of the previous level ran while this round computed; release its device arrays, then hand this level over
             pool.wait_all();
@@ -471,11 +494,7 @@ inline ParseResult gpu_par_phase(const TextSource& src, int sym_bytes, int devic
             std::vector<unsigned char> raw(r.parse_len * (uint64_t)r.cell_bytes_out);
             ctx.check("grlgpu_fetch_parse", grlgpu_fetch_parse(ctx.p, raw.data()));
             res.final_parse.resize(r.parse_len);
-            for (uint64_t i = 0; i < r.parse_len; i++) {
-                uint64_t v = 0;
-                memcpy(&v, raw.data() + i * r.cell_bytes_out, r.cell_bytes_out);
-                res.final_parse[i] = v;
-            }
+            decode_cells(raw.data(), r.parse_len, r.cell_bytes_out, res.final_parse.data());
             break;
         }
     }
@@ -486,18 +505,7 @@ inline ParseResult gpu_par_phase(const TextSource& src, int sym_bytes, int devic
     pool.wait_all();
     ctx.check("grlgpu_fetch_wait", grlgpu_fetch_wait(ctx.p));
     for (auto& f : after) f();
-    // levels in round order; a wide level anywhere moves every level to 64-bit symbols
-    bool any_wide = false;
-    for (auto& s : sinks) any_wide = any_wide || s->wide;
-    res.wide = false;
-    for (auto& s : sinks) {
-        if (!s->wide) res.levels32.push_back(std::move(s->l32));
-        else {
-            if (!res.wide) widen_levels(res);
-            res.levels.push_back(std::move(s->l64));
-        }
-    }
-    (void)any_wide;
+    collect_levels(sinks, res);
     res.par_ms = ms_since(t0);
     return res;
 }
@@ -615,8 +623,7 @@ inline ParseResult gpu_par_phase_mg(const TextSource& src, int sym_bytes, const 
                 ctx.check("grlgpu_fetch_wait", grlgpu_fetch_wait(ctx.p));
                 bar.wait();
                 if (me == 0) {    // the level's host arrays, sized from the global counts every rank was told
-                    RoundDigest dg;
-                    dg.tot = r.tot_phrases; dg.n_pre = r.n_pre_runs; dg.parse_len = r.parse_len; dg.n_phrases = r.n_phrases; dg.dict_syms = r.dict_syms;
+                    RoundDigest dg = digest_of(r);
                     for (int p = 0; p < G; p++)
                         for (int k = 0; k < 4; k++) dg.cs[k] += cs_part[(size_t)p][(size_t)k];
                     res.digests.push_back(dg);
@@ -632,17 +639,10 @@ inline ParseResult gpu_par_phase_mg(const TextSource& src, int sym_bytes, const 
                         dev_ind = false;
                         std::unique_ptr<LevelSink> cur = std::move(sinks.back());
                         sinks.pop_back();
-                        for (int lv = 0; lv < grlgpu_kept_levels(ctx.p); lv++) {
-                            uint64_t A = 0, tot = 0, n_pre = 0;
-                            ctx.check("grlgpu_fetch_kept_level", grlgpu_fetch_kept_level(ctx.p, lv, &A, &tot, &n_pre, nullptr, nullptr, nullptr, nullptr, nullptr));
+                        for (Level32& L : fetch_kept_levels(ctx)) {
                             sinks.emplace_back(new LevelSink());
-                            Level32& L = sinks.back()->l32;
-                            L.alphabet = A; L.tot_phrases = tot;
-                            L.rule_l.resize(tot); L.rule_r.resize(tot); L.has_hocc.resize(tot); L.pre_sym.resize(n_pre); L.pre_len.resize(n_pre);
-                            ctx.check("grlgpu_fetch_kept_level", grlgpu_fetch_kept_level(ctx.p, lv, nullptr, nullptr, nullptr, L.rule_l.data(), L.rule_r.data(),
-                                                                                        L.has_hocc.data(), L.pre_sym.data(), (uint64_t*)L.pre_len.data()));
+                            sinks.back()->l32 = std::move(L);
                         }
-                        grlgpu_drop_kept(ctx.p);
                         sinks.push_back(std::move(cur));
                     }
                 }
@@ -650,12 +650,12 @@ inline ParseResult gpu_par_phase_mg(const TextSource& src, int sym_bytes, const 
                 if (dev_ind) {
                     grlgpu_level_ptrs_t lp;
                     ctx.check("grlgpu_level_park", grlgpu_level_park(ctx.p, 8, &lp));
-                    const int d0 = adopt.device;
-                    int rc = grlgpu_copy_dev(d0, (char*)adopt.rule_l + sl.rank_base * 4, lp.device, lp.rule_l, lp.tot * 4);
-                    if (rc == GRLGPU_OK) rc = grlgpu_copy_dev(d0, (char*)adopt.rule_r + sl.rank_base * 4, lp.device, lp.rule_r, lp.tot * 4);
-                    if (rc == GRLGPU_OK) rc = grlgpu_copy_dev(d0, (char*)adopt.has_hocc + sl.rank_base, lp.device, lp.has_hocc, lp.tot);
-                    if (rc == GRLGPU_OK) rc = grlgpu_copy_dev(d0, (char*)adopt.pre_sym + sl.pre_first * 4, lp.device, lp.pre_sym, lp.n_pre * 4);
-                    if (rc == GRLGPU_OK) rc = grlgpu_copy_dev(d0, (char*)adopt.pre_len + sl.pre_first * 8, lp.device, lp.pre_len, lp.n_pre * 8);
+                    struct C { char* dst; const void* src; uint64_t bytes; };
+                    int rc = GRLGPU_OK;
+                    for (const C& c : {C{(char*)adopt.rule_l + sl.rank_base * 4, lp.rule_l, lp.tot * 4}, C{(char*)adopt.rule_r + sl.rank_base * 4, lp.rule_r, lp.tot * 4},
+                                       C{(char*)adopt.has_hocc + sl.rank_base, lp.has_hocc, lp.tot}, C{(char*)adopt.pre_sym + sl.pre_first * 4, lp.pre_sym, lp.n_pre * 4},
+                                       C{(char*)adopt.pre_len + sl.pre_first * 8, lp.pre_len, lp.n_pre * 8}})
+                        if (rc == GRLGPU_OK) rc = grlgpu_copy_dev(adopt.device, c.dst, lp.device, c.src, c.bytes);
                     if (rc != GRLGPU_OK) throw GpuError(rc, "copying a level slice to rank 0's device failed");
                     ctx.check("grlgpu_fetch_wait", grlgpu_fetch_wait(ctx.p));
                     bar.wait();  // the adopted level is complete before rank 0 adopts the next one
@@ -665,11 +665,7 @@ inline ParseResult gpu_par_phase_mg(const TextSource& src, int sym_bytes, const 
                     std::vector<unsigned char> raw(sl.parse_len_local * (uint64_t)r.cell_bytes_out + 8);
                     ctx.check("grlgpu_fetch_parse", grlgpu_fetch_parse(ctx.p, raw.data()));
                     if (sl.parse_len_local != local_strings[(size_t)me]) throw std::runtime_error("the final parse of a rank is not one cell per string");
-                    for (uint64_t i = 0; i < sl.parse_len_local; i++) {
-                        uint64_t v = 0;
-                        memcpy(&v, raw.data() + i * r.cell_bytes_out, r.cell_bytes_out);
-                        res.final_parse[str_off[(size_t)me] + i] = v;
-                    }
+                    decode_cells(raw.data(), sl.parse_len_local, r.cell_bytes_out, res.final_parse.data() + str_off[(size_t)me]);
                     break;
                 }
             }
@@ -708,15 +704,7 @@ inline ParseResult gpu_par_phase_mg(const TextSource& src, int sym_bytes, const 
                                                          errors[(size_t)r].find("another rank failed") == std::string::npos)))
             first_bad = r;
     if (first_bad >= 0) throw GpuError(err_status[(size_t)first_bad], "rank " + std::to_string(first_bad) + ": " + errors[(size_t)first_bad]);
-    res.wide = false;
-    if (!res.induced_on_device && res.levels32.empty())
-        for (auto& s : sinks) {
-            if (!s->wide) res.levels32.push_back(std::move(s->l32));
-            else {
-                if (!res.wide) widen_levels(res);
-                res.levels.push_back(std::move(s->l64));
-            }
-        }
+    if (!res.induced_on_device && res.levels32.empty()) collect_levels(sinks, res);
     for (int r = 0; r < G; r++) { res.exchange_bytes += xbytes[(size_t)r]; res.h2d_ms = std::max(res.h2d_ms, h2d[(size_t)r]); }
     res.par_ms = par_done_ms - res.h2d_ms;
     return res;
