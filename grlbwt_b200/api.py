@@ -54,6 +54,11 @@ class FmQuery(C.Structure):
                [(k, C.c_float) for k in ("device_ms", "search_ms", "locate_ms")]
 
 
+class FmExtract(C.Structure):
+    _fields_ = [(k, C.c_uint64) for k in ("n_req", "n_cells")] + [(k, C.c_uint32) for k in ("path", "jump_rounds")] + \
+               [(k, C.c_float) for k in ("device_ms", "extract_ms")]
+
+
 class BwtResult(C.Structure):
     _fields_ = [("n_runs", C.c_uint64), ("sb", C.c_uint64), ("fb", C.c_uint64), ("syms", C.POINTER(C.c_uint64)),
                 ("lens", C.POINTER(C.c_uint64)), ("n_rounds", C.c_uint64), ("h2d_ms", C.c_double), ("par_phase_ms", C.c_double),
@@ -124,6 +129,7 @@ def lib_gpu():
         L.grlgpu_fm_load.argtypes = [vp, vp, u64, C.POINTER(FmInfo)]
         L.grlgpu_fm_count.argtypes = [vp, vp, vp, u64, C.c_int, vp, C.POINTER(FmQuery)]
         L.grlgpu_fm_locate.argtypes = [vp, vp, vp, u64, C.c_int, vp, vp, vp, u64, C.POINTER(FmQuery)]
+        L.grlgpu_fm_extract.argtypes = [vp, vp, vp, vp, u64, C.c_int, vp, vp, u64, C.POINTER(FmExtract)]
         L.grlgpu_fm_drop.argtypes = [vp]
         L.grlgpu_selftest_scan.argtypes = [vp, u64, vp, vp]
         L.grlgpu_selftest_sort.argtypes = [vp, vp, u64, C.c_int]
@@ -373,6 +379,34 @@ class GrlGpu:
                                                    n_occ, C.byref(info)), info)
         return occ_off, str_id[:n_occ], str_pos[:n_occ], d
 
+    def fm_extract(self, str_id, start=0, length=None, cell_bytes: int = 1):
+        """Substrings of the indexed strings (see _fm_requests for the forms accepted) -> (out_off, cells, info): request q is
+        S_k[start .. min(start + length, |S_k|)) with k = str_id[q] (to the end of the string when length is None), the cells
+        [out_off[q], out_off[q + 1]) of `cells`, whose dtype has cell_bytes bytes (each cell the symbol's low bytes), and the dict
+        of grlgpu_fm_extract_t. The output is sized from the lengths when they are given and small, else by a first call without
+        capacity; info then covers both calls: device_ms and extract_ms are their sums, jump_rounds those of the call that built
+        the locate table."""
+        ids, frm, ln = _fm_requests(str_id, start, length, cell_bytes)
+        n_req = ids.size
+        out_off = np.zeros(n_req + 1, np.uint64)
+        info = FmExtract()
+        cap = int(ln.sum(dtype=np.uint64)) if length is not None else None
+        sizing = None
+        if cap is None or cap > _FM_EXTRACT_DIRECT_CAP:
+            rc = self._L.grlgpu_fm_extract(self._h, _ptr(ids), _ptr(frm), _ptr(ln), n_req, cell_bytes, _ptr(out_off), None, 0, C.byref(info))
+            if rc != -1 or info.n_cells == 0:   # done (no cells), or an error other than the capacity
+                return out_off, np.zeros(0, CELL[cell_bytes]), self._fm_call(rc, info)
+            sizing = {k: getattr(info, k) for k, _ in FmExtract._fields_}
+            cap = int(info.n_cells)
+        cells = np.zeros(max(cap, 1), CELL[cell_bytes])
+        d = self._fm_call(self._L.grlgpu_fm_extract(self._h, _ptr(ids), _ptr(frm), _ptr(ln), n_req, cell_bytes, _ptr(out_off), _ptr(cells), cap, C.byref(info)), info)
+        if sizing:
+            d["device_ms"] += sizing["device_ms"]
+            d["extract_ms"] += sizing["extract_ms"]
+            d["jump_rounds"] = max(d["jump_rounds"], sizing["jump_rounds"])
+        n = d["n_cells"]
+        return out_off, (cells[:n].copy() if n < cap // 2 else cells[:n]), d   # lengths past the strings: do not keep the whole allocation
+
     def fm_drop(self):
         """Frees this context's FM-index"""
         self._check(self._L.grlgpu_fm_drop(self._h))
@@ -525,6 +559,41 @@ def _fm_patterns(patterns) -> tuple:
     if (np.diff(off.astype(np.int64)) <= 0).any():
         raise GrlGpuError(-1, "patterns: every pattern must have at least one cell (offsets strictly increasing)")
     return np.ascontiguousarray(cells), np.ascontiguousarray(off)
+
+
+_FM_EXTRACT_DIRECT_CAP = 1 << 26   # fm_extract: cells allocated up front from the given lengths; beyond, the library sizes the output
+_U32_MAX = (1 << 32) - 1
+
+
+def _fm_requests(str_id, start=0, length=None, cell_bytes=1) -> tuple:
+    """checks of fm_extract's arguments, before the library is called -> three contiguous uint32 arrays (str_id, start, length).
+    str_id is an integer or a 1-d integer array; start and length are integers or 1-d integer arrays of its size; length None means
+    to the end of the string. Offsets are 32-bit on the device: a length beyond 32 bits is taken as 2^32 - 1 (still to the end), a
+    start at or beyond 2^32 gives an empty substring."""
+    if cell_bytes not in CELL:
+        raise GrlGpuError(-1, "extract: cell_bytes must be 1, 2, 4 or 8")
+    n_req = np.asarray(str_id).size if np.ndim(str_id) else 1
+    cols = []
+    for v, what in ((str_id, "str_id"), (start, "start"), (length, "length")):
+        a = np.asarray(_U32_MAX if v is None else v)
+        if a.size == 0:
+            a = a.astype(np.uint64)
+        if a.ndim > 1 or a.dtype.kind not in "iu":
+            raise GrlGpuError(-1, f"extract: {what} must be an integer or a 1-d integer array")
+        if a.dtype.kind == "i" and (a < 0).any():
+            raise GrlGpuError(-1, f"extract: {what} must not be negative")
+        a = a.astype(np.uint64)
+        if a.ndim == 0:
+            a = np.full(n_req, a, np.uint64)
+        elif a.size != n_req:
+            raise GrlGpuError(-1, f"extract: {what} has {a.size} entries for {n_req} requests")
+        cols.append(a)
+    ids, frm, ln = cols
+    if (ids > _U32_MAX).any():
+        raise GrlGpuError(-1, "extract: str_id must be below 2^32")
+    far = frm > _U32_MAX
+    return (np.ascontiguousarray(ids.astype(np.uint32)), np.ascontiguousarray(np.where(far, _U32_MAX, frm).astype(np.uint32)),
+            np.ascontiguousarray(np.where(far, 0, np.minimum(ln, _U32_MAX)).astype(np.uint32)))
 
 
 def _invert_args(image, cell_bytes, n_seqs, out):

@@ -9,6 +9,11 @@
 //            psi steps reach from j (row k < N is $_k, the end of string k); both walks bounded by B (inv_walk_bound). A longer
 //            walk switches the call to a table of (k, p) for every row, built once per index by pointer jumping (invert.cuh,
 //            part c: p = d, k = the string whose chain from row k ends at succ) and kept for every later call.
+//   extract  one thread per request (k, from, len), S_k[from .. e) with e = min(from + len, L_k): the walk counts L_k by LF steps
+//            from row k (the count pass of invert.cuh with the request's k, bound B), then walks again from row k at position
+//            L_k, writing the cells below e backwards through InvStage. A string longer than B switches the call to samples: the
+//            row at every FM_EXTRACT_SAMPLE-th position of every string, taken from the locate table (built here when no locate
+//            built it) and kept for every later call; the walk then starts at the first sample at or after e.
 // Convention of reverse_bwt and grlgpu_invert: the separator is the smallest symbol of a non-empty record, N its count, strings in
 // input order. A pattern containing the separator or a symbol outside the directory has no occurrence; every empty interval is
 // reported as sp = ep = 0 (the host tool fm_query does the same). Positions and symbols are 32-bit, as for the inversion.
@@ -16,6 +21,9 @@
 #pragma once
 
 constexpr u32 FM_OVER_POLL = 256;  // locate walk: steps between two reads of the "some walk is over the bound" flag
+// extract: one sampled row per FM_EXTRACT_SAMPLE positions of a string (n / 16 bytes, plus 4 bytes per string), so a request walks at
+// most FM_EXTRACT_SAMPLE - 1 steps more than it writes (DESIGN.md §12, "Extract")
+constexpr u32 FM_EXTRACT_SAMPLE = 64;
 
 struct FmView {  // device arrays of a loaded index, passed to the search kernels by value
     const u32 *start, *sym, *len, *F, *order, *dir_sym, *dir_first, *dir_C;
@@ -123,6 +131,57 @@ static __global__ void __launch_bounds__(INV_THREADS) fm_doc_kernel(const u64* _
     doc[j] = ((u64)k << 32) | (p >> 32);
 }
 
+// extract samples from the locate table: string k (row k < N has offset L_k) has L_k / S + 1 samples, at offsets 0, S, ..
+static __global__ void __launch_bounds__(INV_THREADS) fm_samp_len_kernel(const u64* __restrict__ doc, u32 N, u32* __restrict__ cnt) {
+    const u32 k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k < N) cnt[k] = (u32)doc[k] / FM_EXTRACT_SAMPLE + 1;
+}
+static __global__ void __launch_bounds__(INV_THREADS) fm_samp_fill_kernel(const u64* __restrict__ doc, u32 n, const u32* __restrict__ samp_off, u32* __restrict__ samp) {
+    const u32 j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= n) return;
+    const u64 t = doc[j];
+    const u32 p = (u32)t;
+    if (p % FM_EXTRACT_SAMPLE == 0) samp[ld_gather4(samp_off + (u32)(t >> 32)) + p / FM_EXTRACT_SAMPLE] = j;
+}
+// request q: L_k of its string (read from the locate table into Lq when doc is given, else left there by the count pass) and its
+// cell count e - from, e = min(from + len, L_k) in 64 bits (0 when from >= e)
+static __global__ void __launch_bounds__(INV_THREADS) fm_extract_size_kernel(const u32* __restrict__ str_id, const u32* __restrict__ from, const u32* __restrict__ len, u32 n_req,
+                                                                             const u64* __restrict__ doc, u32* __restrict__ Lq, u64* __restrict__ cnt) {
+    const u32 q = blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= n_req) return;
+    u32 L;
+    if (doc) Lq[q] = L = (u32)ld_gather8(doc + str_id[q]);
+    else L = Lq[q];
+    const u64 e = min((u64)from[q] + len[q], (u64)L);
+    cnt[q] = from[q] < e ? e - from[q] : 0;
+}
+// request q: walk LF back from a row at a known position of string k down to position from, writing the cells of the positions
+// below e: from row k at L_k (the end of the string), or, with samples, from the first sampled position at or after e that lies
+// inside the string. The row at position p has BWT = S_k[p - 1], so a step from p emits S_k[p - 1].
+template <class CellT>
+__global__ void __launch_bounds__(INV_THREADS) fm_extract_write_kernel(const u64* __restrict__ E, const u32* __restrict__ str_id, const u32* __restrict__ from,
+                                                                       const u32* __restrict__ len, const u32* __restrict__ Lq, const u64* __restrict__ out_off, u32 n_req,
+                                                                       const u32* __restrict__ samp, const u32* __restrict__ samp_off, u8* __restrict__ out) {
+    const u32 q = blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= n_req) return;
+    const u32 k = str_id[q], L = Lq[q], f = from[q];
+    const u32 e = (u32)min((u64)f + len[q], (u64)L);
+    if (f >= e) return;
+    u32 r = k, p = L;
+    if (samp) {
+        const u32 s = (u32)(((u64)e + FM_EXTRACT_SAMPLE - 1) / FM_EXTRACT_SAMPLE);
+        if ((u64)s * FM_EXTRACT_SAMPLE < L) { r = ld_gather4(samp + ld_gather4(samp_off + k) + s); p = s * FM_EXTRACT_SAMPLE; }
+    }
+    const u64 o = out_off[q];  // position x of the string is cell o + x - f
+    InvStage<CellT> sg{out, o * sizeof(CellT), (o + e - f) * sizeof(CellT)};
+    for (; p > f; p--) {  // p - f steps: L_k - f on the walk, fewer than e - f + FM_EXTRACT_SAMPLE from a sample
+        const u64 x = ld_gather8(E + r);
+        if (p <= e) sg.put(o + (p - 1 - f), inv_sym(x));
+        r = inv_lf(x);
+    }
+    sg.flush();
+}
+
 inline FmView fm_view(const FmIndex& x) {
     return FmView{x.t.start.p, x.t.sym.p, x.t.len.p, x.t.F.p, x.t.order.p, x.dir_sym.p, x.dir_first.p, x.dir_C.p, (u32)x.t.n, (u32)x.t.n_runs, (u32)x.n_dir, x.t.sep};
 }
@@ -164,12 +223,12 @@ inline void fm_load(grlgpu_ctx* c, const u8* image, u64 image_bytes, grlgpu_fm_t
     c->fm = std::move(x);
 }
 
-// the locate table of the loaded index (once): pointer jumping over LF, then one entry per row
-inline u32 fm_build_doc(FmIndex& x, u32* flag, cudaStream_t st) {
+// the locate table of the loaded index (once): pointer jumping over LF, then one entry per row; error messages start with `who`
+inline u32 fm_build_doc(FmIndex& x, u32* flag, cudaStream_t st, const char* who) {
     const u32 n = (u32)x.t.n, N = (u32)x.t.N;
     DevBuf<u64> P(n, st);
     DevBuf<u32> owner(n, st);
-    const u32 rounds = inv_jump_converge(x.t.E.p, n, x.t.sep, P, owner.p, flag, st, "locate");
+    const u32 rounds = inv_jump_converge(x.t.E.p, n, x.t.sep, P, owner.p, flag, st, who);
     {
         DevBuf<u32> slen(N, st);
         GRL_LAUNCH("inv_jump_owner", (u64)N * (8 + 4 + 32), inv_jump_owner_kernel, grid_for(N, INV_THREADS), INV_THREADS, 0, st, P.p, N, slen.p, owner.p);
@@ -179,7 +238,7 @@ inline u32 fm_build_doc(FmIndex& x, u32* flag, cudaStream_t st) {
     GRL_LAUNCH("fm_doc", (u64)n * (8 + 32 + 32 + 8), fm_doc_kernel, grid_for(n, INV_THREADS), INV_THREADS, 0, st, x.t.E.p, P.p, owner.p, n, N, x.t.sep, x.doc.p, flag);
     if (d2h_scalar(flag, st)) {
         x.doc.release();
-        throw Error(GRLGPU_ERR_ILL_FORMED, "locate: a chain ends on a row that is not a string's separator row (an LF cycle without separator)");
+        throw Error(GRLGPU_ERR_ILL_FORMED, std::string(who) + ": a chain ends on a row that is not a string's separator row (an LF cycle without separator)");
     }
     x.doc_ready = true;
     return rounds;
@@ -247,7 +306,7 @@ inline void fm_query(grlgpu_ctx* c, const void* pat, const uint64_t* pat_off, u6
     }
     info->path = (walk || !n_occ) ? 0 : 1;
     if (n_occ && !walk) {
-        if (!x.doc_ready) info->jump_rounds = fm_build_doc(x, flag.p, st);
+        if (!x.doc_ready) info->jump_rounds = fm_build_doc(x, flag.p, st, "locate");
         GRL_LAUNCH("fm_locate_table", n_occ * (8 + 8 + 8 + 32), fm_locate_table_kernel, grid_for(n_occ, INV_THREADS), INV_THREADS, 0, st, x.doc.p, d_se.p, d_occ.p, n_pat, n_occ,
                    d_id.p, d_pos.p);
     }
@@ -260,5 +319,87 @@ inline void fm_query(grlgpu_ctx* c, const void* pat, const uint64_t* pat_off, u6
     t_all.stop();
     info->search_ms = t_search.ms();
     info->locate_ms = t_loc.ms();
+    info->device_ms = t_all.ms();  // waits for the copies
+}
+
+// the extract samples of the loaded index (once), from its locate table
+inline void fm_build_samples(FmIndex& x, cudaStream_t st) {
+    const u32 n = (u32)x.t.n, N = (u32)x.t.N;
+    x.samp_off.alloc((u64)N + 1, st);
+    GRL_LAUNCH("fm_samp_len", (u64)N * (8 + 4), fm_samp_len_kernel, grid_for(N, INV_THREADS), INV_THREADS, 0, st, x.doc.p, N, x.samp_off.p);
+    exclusive_scan<u32, u32>(x.samp_off.p, x.samp_off.p, N, x.samp_off.p + N, st);
+    const u32 n_samp = d2h_scalar(x.samp_off.p + N, st);  // at most n / S + N
+    x.samp.alloc(n_samp, st);
+    GRL_LAUNCH("fm_samp_fill", (u64)n * 8 + (u64)n_samp * (32 + 32), fm_samp_fill_kernel, grid_for(n, INV_THREADS), INV_THREADS, 0, st, x.doc.p, n, x.samp_off.p, x.samp.p);
+    x.samp_ready = true;
+}
+
+template <class CellT>
+void fm_extract_write(const FmIndex& x, const u32* id, const u32* from, const u32* len, const u32* Lq, const u64* off, u32 n_req, bool samples, u8* out, u64 steps,
+                      u64 n_cells, cudaStream_t st) {
+    GRL_LAUNCH("fm_extract_write", (u64)n_req * (4 * 4 + 8) + steps * 32 + n_cells * sizeof(CellT), (fm_extract_write_kernel<CellT>), grid_for(n_req, INV_THREADS), INV_THREADS, 0, st,
+               x.t.E.p, id, from, len, Lq, off, n_req, samples ? x.samp.p : nullptr, samples ? x.samp_off.p : nullptr, out);
+}
+
+// extract of 0 < n_req < 2^32 checked requests (every str_id < N) on the loaded index
+inline void fm_extract(grlgpu_ctx* c, const u32* str_id, const u32* from, const u32* len, u32 n_req, int w, uint64_t* out_off, void* out, u64 cap_cells,
+                       grlgpu_fm_extract_t* info) {
+    cudaStream_t st = c->st;
+    FmIndex& x = *c->fm;
+    const u64 n = x.t.n, N = x.t.N, mean_len = (n - N) / N;  // N >= 1: some request names a string
+    info->n_req = n_req;
+    Timer t_all(st), t_ext(st);
+    t_all.start();
+    DevBuf<u32> d_req(3 * (u64)n_req, st);
+    u32 *d_id = d_req.p, *d_from = d_id + n_req, *d_len = d_from + n_req;
+    GRL_CUDA(cudaMemcpyAsync(d_id, str_id, (u64)n_req * 4, cudaMemcpyHostToDevice, st));
+    GRL_CUDA(cudaMemcpyAsync(d_from, from, (u64)n_req * 4, cudaMemcpyHostToDevice, st));
+    GRL_CUDA(cudaMemcpyAsync(d_len, len, (u64)n_req * 4, cudaMemcpyHostToDevice, st));
+    t_ext.start();
+    DevBuf<u32> Lq(n_req, st), flag(1, st);
+    const bool force_walk = (c->flags & GRLGPU_FLAG_FORCE_WALK) != 0, force_jump = (c->flags & GRLGPU_FLAG_FORCE_JUMP) != 0 && !force_walk;
+    bool walk = !force_jump && (force_walk || !(x.doc_ready || x.samp_ready));  // once the samples or the locate table exist, they answer
+    if (walk) {  // a walk from row k ends within n steps (the LF cycle of k holds the separator row LF^-1(k)): the bound n never overflows
+        const u64 B = force_walk ? n : inv_walk_bound(n);
+        flag.zero();
+        GRL_LAUNCH("inv_walk_count", (u64)n_req * (8 + mean_len * 32), inv_walk_count_kernel, grid_for(n_req, INV_THREADS), INV_THREADS, 0, st, x.t.E.p, (const u32*)d_id, n_req,
+                   x.t.sep, (u32)B, Lq.p, flag.p);
+        walk = d2h_scalar(flag.p, st) == 0;
+    }
+    info->path = walk ? 0 : 1;
+    if (!walk) {
+        if (!x.doc_ready) info->jump_rounds = fm_build_doc(x, flag.p, st, "extract");
+        if (!x.samp_ready) fm_build_samples(x, st);
+    }
+    DevBuf<u64> d_off((u64)n_req + 1, st);
+    {
+        DevBuf<u64> cnt(n_req, st);
+        GRL_LAUNCH("fm_extract_size", (u64)n_req * (4 * 4 + 8) + (walk ? 0 : (u64)n_req * 32), fm_extract_size_kernel, grid_for(n_req, INV_THREADS), INV_THREADS, 0, st, d_id, d_from,
+                   d_len, n_req, walk ? (const u64*)nullptr : x.doc.p, Lq.p, cnt.p);
+        exclusive_scan<u64, u64>(cnt.p, d_off.p, n_req, d_off.p + n_req, st);
+    }
+    const u64 n_cells = d2h_scalar(d_off.p + n_req, st);
+    info->n_cells = n_cells;
+    if (n_cells > cap_cells) {  // the times of the work done so far (a sizing call may have built the locate table and the samples)
+        t_ext.stop();
+        t_all.stop();
+        info->extract_ms = t_ext.ms();
+        info->device_ms = t_all.ms();
+        throw Error(GRLGPU_ERR_ARG, "extract: the cells need a capacity of " + std::to_string(n_cells));
+    }
+    DevBuf<u8> dout(n_cells * w + 16, st);
+    // steps of the model: the walk goes from each string's end (mean length), a sample at most S - 1 positions past e (S / 2 on average)
+    const u64 steps = walk ? (u64)n_req * mean_len : n_cells + (u64)n_req * FM_EXTRACT_SAMPLE / 2;
+    switch (w) {
+        case 1: fm_extract_write<u8>(x, d_id, d_from, d_len, Lq.p, d_off.p, n_req, !walk, dout.p, steps, n_cells, st); break;
+        case 2: fm_extract_write<u16>(x, d_id, d_from, d_len, Lq.p, d_off.p, n_req, !walk, dout.p, steps, n_cells, st); break;
+        case 4: fm_extract_write<u32>(x, d_id, d_from, d_len, Lq.p, d_off.p, n_req, !walk, dout.p, steps, n_cells, st); break;
+        default: fm_extract_write<u64>(x, d_id, d_from, d_len, Lq.p, d_off.p, n_req, !walk, dout.p, steps, n_cells, st); break;
+    }
+    t_ext.stop();
+    GRL_CUDA(cudaMemcpyAsync(out_off, d_off.p, ((u64)n_req + 1) * 8, cudaMemcpyDeviceToHost, st));
+    if (n_cells) GRL_CUDA(cudaMemcpyAsync(out, dout.p, n_cells * w, cudaMemcpyDeviceToHost, st));
+    t_all.stop();
+    info->extract_ms = t_ext.ms();
     info->device_ms = t_all.ms();  // waits for the copies
 }

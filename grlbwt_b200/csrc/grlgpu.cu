@@ -74,7 +74,7 @@ struct LfTable {
     DevBuf<u64> E;
 };
 
-// a loaded FM-index (fm.cuh): the LF table, a symbol directory, psi, and the locate table once some call needed it
+// a loaded FM-index (fm.cuh): the LF table, a symbol directory, psi, and the locate table and extract samples once some call needed them
 struct FmIndex {
     LfTable t;
     u64 n_dir = 0;
@@ -82,6 +82,8 @@ struct FmIndex {
     DevBuf<u32> psi;                        // psi[LF(j)] = j
     DevBuf<u64> doc;                        // locate table: {string << 32 | offset} for every row
     bool doc_ready = false;
+    DevBuf<u32> samp, samp_off;             // extract samples: the row at offset s * FM_EXTRACT_SAMPLE of string k is samp[samp_off[k] + s]
+    bool samp_ready = false;
 };
 
 struct grlgpu_ctx {
@@ -1682,6 +1684,23 @@ int grlgpu_fm_locate(grlgpu_ctx* ctx, const void* pat, const uint64_t* pat_off, 
     if (!ctx->fm) return GRLGPU_ERR_STATE;
     if (n_pat == 0) return GRLGPU_OK;
     return guarded(ctx, [&] { fm_query(ctx, pat, pat_off, n_pat, pat_bytes, nullptr, occ_off, str_id, str_pos, cap_occ, info); });
+}
+
+int grlgpu_fm_extract(grlgpu_ctx* ctx, const uint32_t* str_id, const uint32_t* from, const uint32_t* len, uint64_t n_req, int cell_bytes, uint64_t* out_off, void* out,
+                      uint64_t cap_cells, grlgpu_fm_extract_t* info) {
+    if (!ctx || !info) return GRLGPU_ERR_ARG;
+    memset(info, 0, sizeof(*info));
+    if (!(cell_bytes == 1 || cell_bytes == 2 || cell_bytes == 4 || cell_bytes == 8)) return GRLGPU_ERR_ARG;
+    if ((n_req && (!str_id || !from || !len || !out_off)) || (cap_cells && !out)) return GRLGPU_ERR_ARG;
+    if (!ctx->fm) return GRLGPU_ERR_STATE;
+    if (n_req >> 32) return GRLGPU_ERR_LIMIT;
+    for (u64 q = 0; q < n_req; q++)
+        if (str_id[q] >= ctx->fm->t.N) return GRLGPU_ERR_ARG;
+    if (n_req == 0) {
+        if (out_off) out_off[0] = 0;
+        return GRLGPU_OK;
+    }
+    return guarded(ctx, [&] { fm_extract(ctx, str_id, from, len, (u32)n_req, cell_bytes, out_off, out, cap_cells, info); });
 }
 
 int grlgpu_fm_drop(grlgpu_ctx* ctx) {

@@ -11,7 +11,7 @@
 // backwards. LF built from any run list is a permutation that maps the separator rows onto [0, N), so that chain ends within
 // n steps for every input; a run list that is not a BWT can still leave rows on cycles without a separator, which both paths
 // detect. Positions and lengths are 32-bit (n < 0xfffffff0, symbols < 2^32): larger inputs are left to the host tool.
-// Part a (lf_table_build), the walk bound and pointer jumping (inv_jump_converge) are shared with the FM-index of fm.cuh.
+// Part a (lf_table_build), the walk bound, the count pass and pointer jumping (inv_jump_converge) are shared with the FM-index of fm.cuh.
 // Included by grlgpu.cu inside its anonymous namespace.
 #pragma once
 
@@ -104,11 +104,13 @@ static __global__ void __launch_bounds__(INV_THREADS) inv_fill_kernel(const u32*
 
 // ---- b: walk per string ----
 // count pass: steps from row i to its separator row, at most `bound` (chains from rows < N end within n steps: bound >= n
-// never overflows); more than `bound` raises *over and the caller switches to pointer jumping
-static __global__ void __launch_bounds__(INV_THREADS) inv_walk_count_kernel(const u64* __restrict__ E, u32 n_req, u32 sep, u32 bound, u32* __restrict__ len, u32* over) {
+// never overflows); more than `bound` raises *over and the caller switches to pointer jumping. Thread i walks string ids[i]
+// (fm.cuh's extract), or string i when ids is null.
+static __global__ void __launch_bounds__(INV_THREADS) inv_walk_count_kernel(const u64* __restrict__ E, const u32* __restrict__ ids, u32 n_req, u32 sep, u32 bound, u32* __restrict__ len,
+                                                                            u32* over) {
     const u32 i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n_req) return;
-    u32 j = i;
+    u32 j = ids ? ids[i] : i;
     for (u32 t = 0; t < bound; t++) {  // bounded by `bound`
         const u64 e = ld_gather8(E + j);
         if (inv_sym(e) == sep) { len[i] = t; return; }
@@ -339,7 +341,7 @@ inline void invert_image(grlgpu_ctx* c, const u8* image, u64 image_bytes, int w,
     if (walk) {  // count pass: chains of rows < N end within n steps, so the bound n never overflows
         const u64 B = force_walk ? n : inv_walk_bound(n);
         flag.zero();
-        GRL_LAUNCH("inv_walk_count", (u64)n_req * 4 + (n - N) * 32, inv_walk_count_kernel, grid_for(n_req, INV_THREADS), INV_THREADS, 0, st, E.p, n_req, sep, (u32)B, slen.p, flag.p);
+        GRL_LAUNCH("inv_walk_count", (u64)n_req * 4 + (n - N) * 32, inv_walk_count_kernel, grid_for(n_req, INV_THREADS), INV_THREADS, 0, st, E.p, (const u32*)nullptr, n_req, sep, (u32)B, slen.p, flag.p);
         walk = d2h_scalar(flag.p, st) == 0;
     }
     const auto sized = [&](u64 n_out) {  // output size known: check the caller's capacity

@@ -134,6 +134,21 @@ struct RlBwt {
         } while (k >= n_strings);
         return {k, p};
     }
+
+    // ---- extract (fm_extract) ----
+    // S_k for k < n_strings: walked backwards by LF from row k, as reverse_bwt does. The walk ends within n steps for any run list:
+    // the LF cycle of row k holds the separator row LF^-1(k).
+    std::vector<uint64_t> string_of(uint64_t k) const {
+        std::vector<uint64_t> s;
+        for (auto e = lf(k); e.first != sep; e = lf(e.second)) s.push_back(e.first);
+        std::reverse(s.begin(), s.end());
+        return s;
+    }
+    // the cells [from, e) of S_k[from .. e) in a string of length L: e = min(from + len, L) without overflow, empty when from >= L
+    static std::pair<uint64_t, uint64_t> clamp(uint64_t L, uint64_t from, uint64_t len) {
+        if (from >= L) return {0, 0};
+        return {from, len > L - from ? L : from + len};
+    }
 };
 
 inline void put_cell(std::vector<unsigned char>& out, uint64_t v, int width) {

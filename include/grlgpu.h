@@ -35,8 +35,8 @@ enum grlgpu_status {
 #define GRLGPU_FLAG_SMALL_PILOT 16ull /* tests: one pilot tile, so small inputs exercise pilot + remainder */
 #define GRLGPU_FLAG_FORCE_DOUBLING 32ull /* tests: refine suffix groups by prefix doubling even when key extension would do */
 #define GRLGPU_FLAG_KEEP_DICT 4ull /* tests: keep the last round's dictionary for grlgpu_fetch_dictionary */
-#define GRLGPU_FLAG_FORCE_WALK 64ull /* tests: grlgpu_invert walks every string and grlgpu_fm_locate walks every occurrence, whatever the chain lengths */
-#define GRLGPU_FLAG_FORCE_JUMP 128ull /* tests: grlgpu_invert runs pointer jumping and grlgpu_fm_locate answers from its table, whatever the chain lengths */
+#define GRLGPU_FLAG_FORCE_WALK 64ull /* tests: grlgpu_invert walks every string, grlgpu_fm_locate walks every occurrence and grlgpu_fm_extract walks every request from its string's end, whatever the chain lengths */
+#define GRLGPU_FLAG_FORCE_JUMP 128ull /* tests: grlgpu_invert runs pointer jumping, grlgpu_fm_locate answers from its table and grlgpu_fm_extract starts from the samples, whatever the chain lengths */
 
 /* = str_collection (external/cdt/include/utils.h:20-28) as filled by collection_stats (utils.cpp:100-189) */
 typedef struct {
@@ -221,6 +221,30 @@ int grlgpu_fm_count(grlgpu_ctx* ctx, const void* pat, const uint64_t* pat_off /*
 int grlgpu_fm_locate(grlgpu_ctx* ctx, const void* pat, const uint64_t* pat_off, uint64_t n_pat, int pat_bytes, uint64_t* occ_off /* n_pat + 1 */,
                      uint32_t* str_id, uint32_t* str_pos, uint64_t cap_occ, grlgpu_fm_query_t* info);
 int grlgpu_fm_drop(grlgpu_ctx* ctx);
+
+/* extract from the loaded index (the host tool fm_extract is the general path and writes the same cells):
+ *   grlgpu_fm_extract  substrings of the indexed strings: request q = (str_id[q], from[q], len[q]) yields S_k[from .. e) with
+ *                      k = str_id[q], e = min(from + len, L_k) (computed in 64 bits, so len = UINT32_MAX means "to the end");
+ *                      from >= e yields nothing. Cells of cell_bytes little-endian bytes, each the symbol's low bytes (as
+ *                      reverse_bwt's put_cell), no separators. out_off (n_req + 1 entries) receives the cell offsets:
+ *                      request q is cells [out_off[q], out_off[q + 1]) of out.
+ *                      Each request walks LF back from row k, the end of string k: a count pass of at most B = max(4096, n / 2048)
+ *                      steps gives L_k, a write pass walks again. A string longer than B makes the call, and every later call on the
+ *                      index, start from sampled rows instead: every 64th position of every string, taken from the locate table of
+ *                      grlgpu_fm_locate (built by pointer jumping when no call built it before, and then shared by both calls).
+ *                      GRLGPU_FLAG_FORCE_WALK / _JUMP force one path. A walk from row k always ends (the LF cycle of k holds the
+ *                      separator row LF^-1(k)), so only the sampled path can meet a run list that is not a BWT.
+ * GRLGPU_ERR_ARG: cell_bytes not in {1,2,4,8}, a null array with n_req > 0, some str_id >= N, or cap_cells < n_cells
+ * (info->n_cells then holds the number needed, and device_ms / extract_ms the time spent, nothing is written). GRLGPU_ERR_STATE: no index loaded. GRLGPU_ERR_LIMIT: n_req >= 2^32.
+ * GRLGPU_ERR_ILL_FORMED: the call needed the locate table and the run list is not a BWT. n_req = 0 is accepted. */
+typedef struct {
+    uint64_t n_req, n_cells;     /* requests; cells written (or needed, when cap_cells is too small) */
+    uint32_t path;               /* 0 walk per request, 1 from the samples */
+    uint32_t jump_rounds;        /* pointer-jumping rounds when this call built the locate table, else 0 */
+    float device_ms, extract_ms; /* CUDA events on the context's stream: whole call (copies included) / the extraction */
+} grlgpu_fm_extract_t;
+int grlgpu_fm_extract(grlgpu_ctx* ctx, const uint32_t* str_id, const uint32_t* from, const uint32_t* len, uint64_t n_req,
+                      int cell_bytes, uint64_t* out_off /* n_req + 1 */, void* out, uint64_t cap_cells, grlgpu_fm_extract_t* info);
 
 /* digest of the last round's level artefacts, computed on the device before they are fetched: four sums mod 2^64
  * {rules weighted by rank, hocc marks weighted by rank, sum of the preliminary-BWT run lengths, runs weighted by symbol}.
