@@ -54,6 +54,11 @@ class FmQuery(C.Structure):
                [(k, C.c_float) for k in ("device_ms", "search_ms", "locate_ms")]
 
 
+class FmApprox(C.Structure):
+    _fields_ = [(k, C.c_uint64) for k in ("n_pat", "n_pat_syms", "n_hits", "n_occ", "n_lf")] + [(k, C.c_uint32) for k in ("path", "jump_rounds")] + \
+               [(k, C.c_float) for k in ("device_ms", "search_ms", "locate_ms")]
+
+
 class FmExtract(C.Structure):
     _fields_ = [(k, C.c_uint64) for k in ("n_req", "n_cells")] + [(k, C.c_uint32) for k in ("path", "jump_rounds")] + \
                [(k, C.c_float) for k in ("device_ms", "extract_ms")]
@@ -129,6 +134,8 @@ def lib_gpu():
         L.grlgpu_fm_load.argtypes = [vp, vp, u64, C.POINTER(FmInfo)]
         L.grlgpu_fm_count.argtypes = [vp, vp, vp, u64, C.c_int, vp, C.POINTER(FmQuery)]
         L.grlgpu_fm_locate.argtypes = [vp, vp, vp, u64, C.c_int, vp, vp, vp, u64, C.POINTER(FmQuery)]
+        L.grlgpu_fm_approx_count.argtypes = [vp, vp, vp, u64, C.c_int, C.c_uint32, vp, vp, vp, u64, C.POINTER(FmApprox)]
+        L.grlgpu_fm_approx_locate.argtypes = [vp, vp, vp, u64, C.c_int, C.c_uint32, vp, vp, vp, vp, u64, C.POINTER(FmApprox)]
         L.grlgpu_fm_extract.argtypes = [vp, vp, vp, vp, u64, C.c_int, vp, vp, u64, C.POINTER(FmExtract)]
         L.grlgpu_fm_drop.argtypes = [vp]
         L.grlgpu_selftest_scan.argtypes = [vp, u64, vp, vp]
@@ -379,6 +386,44 @@ class GrlGpu:
                                                    n_occ, C.byref(info)), info)
         return occ_off, str_id[:n_occ], str_pos[:n_occ], d
 
+    def fm_approx_count(self, patterns, k: int):
+        """Search with at most k <= 3 mismatches (substitutions) -> (hit_off, sp, ep, mm, info): pattern q's hits are
+        [hit_off[q], hit_off[q + 1]) of the uint64 arrays sp, ep and the uint8 array mm; a hit is one distinct string Q within
+        Hamming distance mm of the pattern that occurs, at the rows [sp, ep), listed by ascending sp. info is the dict of
+        grlgpu_fm_approx_t (n_occ = the sum of ep - sp). The hits are written into a guessed capacity; when it is short, a second
+        call writes them, and device_ms / search_ms are the sums of both calls."""
+        cells, off, k = _fm_approx_args(patterns, k)
+        n_pat = off.size - 1
+        hit_off = np.zeros(n_pat + 1, np.uint64)
+        cap, first = max(1024, 4 * n_pat), None
+        while True:
+            sp_ep, mm, info = np.zeros(2 * cap, np.uint64), np.zeros(cap, np.uint8), FmApprox()
+            rc = self._L.grlgpu_fm_approx_count(self._h, _ptr(cells), _ptr(off), n_pat, cells.dtype.itemsize, k, _ptr(hit_off), _ptr(sp_ep), _ptr(mm), cap,
+                                                C.byref(info))
+            if first is not None or rc != -1 or info.n_hits <= cap:
+                break
+            first, cap = {f: getattr(info, f) for f, _ in FmApprox._fields_}, int(info.n_hits)
+        d = self._fm_call(rc, info)
+        if first:
+            d["device_ms"] += first["device_ms"]
+            d["search_ms"] += first["search_ms"]
+        n = d["n_hits"]
+        return hit_off, sp_ep[0:2 * n:2].copy(), sp_ep[1:2 * n:2].copy(), mm[:n].copy(), d
+
+    def fm_approx_locate(self, patterns, k: int):
+        """Every occurrence with at most k <= 3 mismatches -> (occ_off, str_id, str_pos, mm, info): pattern q's occurrences are
+        [occ_off[q], occ_off[q + 1]) of str_id (string k), str_pos (offset p) and mm (mismatches d), in row order. The output is
+        sized by a fm_approx_count call."""
+        cells, off, k = _fm_approx_args(patterns, k)
+        n_pat = off.size - 1
+        n_occ = int(self.fm_approx_count((cells, off), k)[4]["n_occ"])
+        occ_off = np.zeros(n_pat + 1, np.uint64)
+        str_id, str_pos, mm = np.zeros(max(n_occ, 1), np.uint32), np.zeros(max(n_occ, 1), np.uint32), np.zeros(max(n_occ, 1), np.uint8)
+        info = FmApprox()
+        d = self._fm_call(self._L.grlgpu_fm_approx_locate(self._h, _ptr(cells), _ptr(off), n_pat, cells.dtype.itemsize, k, _ptr(occ_off), _ptr(str_id),
+                                                          _ptr(str_pos), _ptr(mm), n_occ, C.byref(info)), info)
+        return occ_off, str_id[:n_occ], str_pos[:n_occ], mm[:n_occ], d
+
     def fm_extract(self, str_id, start=0, length=None, cell_bytes: int = 1):
         """Substrings of the indexed strings (see _fm_requests for the forms accepted) -> (out_off, cells, info): request q is
         S_k[start .. min(start + length, |S_k|)) with k = str_id[q] (to the end of the string when length is None), the cells
@@ -559,6 +604,15 @@ def _fm_patterns(patterns) -> tuple:
     if (np.diff(off.astype(np.int64)) <= 0).any():
         raise GrlGpuError(-1, "patterns: every pattern must have at least one cell (offsets strictly increasing)")
     return np.ascontiguousarray(cells), np.ascontiguousarray(off)
+
+
+def _fm_approx_args(patterns, k) -> tuple:
+    """checks of fm_approx_count / fm_approx_locate, before the library is called -> (cells, uint64 offsets, k): the patterns as
+    _fm_patterns takes them, k an integer from 0 to 3"""
+    if isinstance(k, (bool, np.bool_)) or not isinstance(k, (int, np.integer)) or not 0 <= int(k) <= 3:
+        raise GrlGpuError(-1, "approximate search: k must be an integer from 0 to 3")
+    cells, off = _fm_patterns(patterns)
+    return cells, off, int(k)
 
 
 _FM_EXTRACT_DIRECT_CAP = 1 << 26   # fm_extract: cells allocated up front from the given lengths; beyond, the library sizes the output

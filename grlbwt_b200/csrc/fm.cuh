@@ -14,6 +14,8 @@
 //            L_k, writing the cells below e backwards through InvStage. A string longer than B switches the call to samples: the
 //            row at every FM_EXTRACT_SAMPLE-th position of every string, taken from the locate table (built here when no locate
 //            built it) and kept for every later call; the walk then starts at the first sample at or after e.
+//   approx   count / locate with at most k <= 3 substitutions: one thread per pattern, a depth-first backward search over at most
+//            k + 1 frames (fm_approx_kernel), hits appended to a pool, sorted by (pattern, sp); locate runs on the hits' intervals
 // Convention of reverse_bwt and grlgpu_invert: the separator is the smallest symbol of a non-empty record, N its count, strings in
 // input order. A pattern containing the separator or a symbol outside the directory has no occurrence; every empty interval is
 // reported as sp = ep = 0 (the host tool fm_query does the same). Positions and symbols are 32-bit, as for the inversion.
@@ -63,6 +65,116 @@ __global__ void __launch_bounds__(INV_THREADS) fm_count_kernel(FmView x, const C
     sp_ep[2 * q] = sp;
     sp_ep[2 * q + 1] = ep;
 }
+// approximate search (DESIGN.md §12, "Approximate search"): one thread per pattern, depth-first over the substitutions, hits
+// appended to a pool of `cap` entries through counters[0] (which keeps counting past cap). Frame j holds the state after j
+// substitutions: t cells of the pattern are still to match (cells 0 .. t - 1), [sp, ep) is the interval of the suffix matched so
+// far, [ra, rb) the runs holding it, cur the next substitution to try at cell t - 1 (a run of [ra, rb) when they are fewer than
+// the directory's symbols, else a directory index). Exact steps move a frame's own t down; a substitution pushes frame j + 1.
+constexpr u32 FM_APPROX_MAX_K = 3;
+struct FmFrame { u32 t, sp, ep, cur, ra, rb; };
+__device__ __forceinline__ FmFrame fm_frame(const FmView& x, u32 t, u32 sp, u32 ep, bool subst) {
+    if (!subst || t == 0) return FmFrame{t, sp, ep, 0, 0, 0};  // no substitution will be tried: the runs are not needed
+    return FmFrame{t, sp, ep, 0, ind_upper_bound(x.start, x.n_runs + 1, sp) - 1, ind_upper_bound(x.start, x.n_runs + 1, ep - 1)};
+}
+template <class CellT>
+__global__ void __launch_bounds__(INV_THREADS) fm_approx_kernel(FmView x, const CellT* __restrict__ pat, const u64* __restrict__ pat_off, u64 n_pat, u32 kmax,
+                                                                u64 cap, u64* __restrict__ key, u32* __restrict__ slot, u64* __restrict__ ep_d, u64* __restrict__ cnt,
+                                                                u64* counters /* [0] hits, [1] LF_c evaluations */) {
+    const u64 q = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= n_pat) return;
+    const CellT* P = pat + pat_off[q];
+    const u64 m = pat_off[q + 1] - pat_off[q];
+    u64 hits = 0, lf = 0;
+    FmFrame f[FM_APPROX_MAX_K + 1];
+    int j = 0;
+    if (m < x.n) f[0] = fm_frame(x, (u32)m, 0, x.n, kmax > 0);
+    else j = -1;  // a window inside a string has fewer cells than the BWT has rows
+    // Each pass either emits a hit and pops, tries one substitution (at most sigma per cell and frame), takes one exact step (at
+    // most m per frame) or pops: at most kmax + 1 <= 4 frames live, so the loop ends after O(m * sigma) passes per frame pushed.
+    while (j >= 0) {
+        FmFrame& F = f[j];
+        if (F.t == 0) {  // the whole pattern is matched with j substitutions
+            const u64 s = atomicAdd((unsigned long long*)counters, 1ull);
+            if (s < cap) { key[s] = (q << 32) | F.sp; slot[s] = (u32)s; ep_d[s] = ((u64)j << 32) | F.ep; }
+            hits++;
+            j--;
+            continue;
+        }
+        const u64 own = (u64)P[F.t - 1];
+        if ((u32)j < kmax) {  // substitutions at cell t - 1: symbols other than the separator and the cell's own
+            bool found = false;
+            u32 csp = 0, cep = 0;
+            if (F.rb - F.ra < x.n_dir) {  // the symbols of the runs holding [sp, ep), each tried at its first run there
+                while (!found && F.ra + F.cur < F.rb) {  // at most rb - ra < sigma candidates
+                    const u32 r = F.ra + F.cur++, c = x.sym[r];
+                    if (c == x.sep || (u64)c == own) continue;
+                    const u32 first = x.F[r] + (max(F.sp, x.start[r]) - x.start[r]);  // LF_c(sp) when r is c's first run in [sp, ep)
+                    if (F.rb - F.ra == 1) {  // one run: LF_c = F + the offset in the run, no search
+                        csp = first;
+                        cep = x.F[r] + (F.ep - x.start[r]);
+                        lf += 2;
+                        found = true;
+                        continue;
+                    }
+                    const u32 d = fm_dir_find(x, c);
+                    csp = fm_lf_c(x, d, F.sp);
+                    lf++;
+                    if (csp != first) continue;  // c has an earlier run in the interval, where it was tried
+                    cep = fm_lf_c(x, d, F.ep);
+                    lf++;
+                    found = true;  // non-empty: run r holds c inside [sp, ep)
+                }
+            } else {
+                for (; !found && F.cur < x.n_dir; F.cur++) {  // at most sigma candidates
+                    const u32 c = x.dir_sym[F.cur];
+                    if (c == x.sep || (u64)c == own) continue;
+                    csp = fm_lf_c(x, F.cur, F.sp);
+                    cep = fm_lf_c(x, F.cur, F.ep);
+                    lf += 2;
+                    found = csp < cep;
+                }
+            }
+            if (found) {
+                f[j + 1] = fm_frame(x, F.t - 1, csp, cep, (u32)j + 1 < kmax);
+                j++;
+                continue;
+            }
+        }
+        // no substitution left at this cell: the exact step
+        const u32 d = fm_dir_find(x, own);
+        if (d == x.n_dir) { j--; continue; }
+        const u32 sp = fm_lf_c(x, d, F.sp), ep = fm_lf_c(x, d, F.ep);
+        lf += 2;
+        if (sp >= ep) { j--; continue; }
+        F = fm_frame(x, F.t - 1, sp, ep, (u32)j < kmax);
+    }
+    cnt[q] = hits;
+    atomicAdd((unsigned long long*)counters + 1, (unsigned long long)lf);
+}
+// hits in (pattern, sp) order: slot s of the pool -> sp_ep[2i], sp_ep[2i + 1], mm[i]
+static __global__ void __launch_bounds__(INV_THREADS) fm_approx_gather_kernel(const u64* __restrict__ key, const u32* __restrict__ slot, const u64* __restrict__ ep_d, u64 n_hits,
+                                                                              u64* __restrict__ sp_ep, u8* __restrict__ mm) {
+    const u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_hits) return;
+    const u64 e = ld_gather8(ep_d + slot[i]);
+    sp_ep[2 * i] = (u32)key[i];
+    sp_ep[2 * i + 1] = (u32)e;
+    mm[i] = (u8)(e >> 32);
+}
+// approximate locate: occurrence o takes the d of its hit; pattern q's occurrences start where its first hit's do
+static __global__ void __launch_bounds__(INV_THREADS) fm_approx_occ_mm_kernel(const u64* __restrict__ hit_occ, u64 n_hits, const u8* __restrict__ hit_mm, u64 n_occ,
+                                                                              u8* __restrict__ occ_mm) {
+    const u64 o = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    if (o >= n_occ) return;
+    u64 lo = 0, hi = n_hits;  // last h with hit_occ[h] <= o
+    while (hi - lo > 1) { const u64 mid = (lo + hi) >> 1; if (hit_occ[mid] <= o) lo = mid; else hi = mid; }
+    occ_mm[o] = hit_mm[lo];
+}
+static __global__ void __launch_bounds__(INV_THREADS) fm_approx_occ_off_kernel(const u64* __restrict__ hit_occ, const u64* __restrict__ hit_off, u64 n_pat, u64* __restrict__ occ_off) {
+    const u64 q = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    if (q <= n_pat) occ_off[q] = hit_occ[hit_off[q]];
+}
+
 static __global__ void __launch_bounds__(INV_THREADS) fm_occ_count_kernel(const u64* __restrict__ sp_ep, u64 n_pat, u64* __restrict__ cnt) {
     const u64 q = (u64)blockIdx.x * blockDim.x + threadIdx.x;
     if (q < n_pat) cnt[q] = sp_ep[2 * q + 1] - sp_ep[2 * q];
@@ -244,6 +356,48 @@ inline u32 fm_build_doc(FmIndex& x, u32* flag, cudaStream_t st, const char* who)
     return rounds;
 }
 
+// locate of every row of n_iv > 0 device intervals d_se (sp, ep per interval): d_occ receives the n_iv + 1 occurrence offsets, d_id /
+// d_pos the occurrences, interval by interval in row order; info->n_occ, path and jump_rounds are set. Errors: GRLGPU_ERR_ARG when
+// cap_occ < n_occ (info->n_occ holds the number needed), GRLGPU_ERR_ILL_FORMED on an LF cycle without separator.
+template <class Info>
+u64 fm_locate_rows(grlgpu_ctx* c, const u64* d_se, u64 n_iv, u64 cap_occ, DevBuf<u64>& d_occ, DevBuf<u32>& d_id, DevBuf<u32>& d_pos, Timer& t_loc, Info* info) {
+    cudaStream_t st = c->st;
+    FmIndex& x = *c->fm;
+    d_occ.alloc(n_iv + 1, st);
+    {
+        DevBuf<u64> cnt(n_iv, st);
+        GRL_LAUNCH("fm_occ_count", n_iv * 24, fm_occ_count_kernel, grid_for(n_iv, INV_THREADS), INV_THREADS, 0, st, d_se, n_iv, cnt.p);
+        exclusive_scan<u64, u64>(cnt.p, d_occ.p, n_iv, d_occ.p + n_iv, st);
+    }
+    const u64 n_occ = d2h_scalar(d_occ.p + n_iv, st);
+    info->n_occ = n_occ;
+    if (n_occ > cap_occ) throw Error(GRLGPU_ERR_ARG, "locate: the occurrences need a capacity of " + std::to_string(n_occ));
+    t_loc.start();
+    d_id.alloc(n_occ, st);
+    d_pos.alloc(n_occ, st);
+    DevBuf<u32> flag(1, st);
+    const bool force_walk = (c->flags & GRLGPU_FLAG_FORCE_WALK) != 0, force_jump = (c->flags & GRLGPU_FLAG_FORCE_JUMP) != 0 && !force_walk;
+    bool walk = n_occ && !force_jump && (force_walk || !x.doc_ready);  // once built, the table answers every call
+    if (walk) {  // rows off a cycle reach a separator row within n LF steps and a row < N within n psi steps: the bound n never overflows
+        const u64 B = force_walk ? x.t.n : inv_walk_bound(x.t.n);
+        flag.zero();
+        GRL_LAUNCH("fm_locate_walk", n_occ * (8 + 8 + 8 * 2) + (u64)n_occ * 32 * 16, fm_locate_walk_kernel, grid_for(n_occ, INV_THREADS), INV_THREADS, 0, st, x.t.E.p, x.psi.p,
+                   (u32)x.t.N, x.t.sep, d_se, d_occ.p, n_iv, n_occ, (u32)B, d_id.p, d_pos.p, flag.p);
+        if (d2h_scalar(flag.p, st)) {
+            if (force_walk) throw Error(GRLGPU_ERR_ILL_FORMED, "locate: a walk of n steps met no separator (an LF cycle without separator)");
+            walk = false;
+        }
+    }
+    info->path = (walk || !n_occ) ? 0 : 1;
+    if (n_occ && !walk) {
+        if (!x.doc_ready) info->jump_rounds = fm_build_doc(x, flag.p, st, "locate");
+        GRL_LAUNCH("fm_locate_table", n_occ * (8 + 8 + 8 + 32), fm_locate_table_kernel, grid_for(n_occ, INV_THREADS), INV_THREADS, 0, st, x.doc.p, d_se, d_occ.p, n_iv, n_occ,
+                   d_id.p, d_pos.p);
+    }
+    t_loc.stop();
+    return n_occ;
+}
+
 // count (str_id == nullptr) or locate of n_pat > 0 checked patterns on the loaded index
 inline void fm_query(grlgpu_ctx* c, const void* pat, const uint64_t* pat_off, u64 n_pat, int pat_bytes, uint64_t* sp_ep, uint64_t* occ_off, u32* str_id, u32* str_pos, u64 cap_occ,
                      grlgpu_fm_query_t* info) {
@@ -281,36 +435,9 @@ inline void fm_query(grlgpu_ctx* c, const void* pat, const uint64_t* pat_off, u6
         info->device_ms = t_all.ms();  // waits for the copy
         return;
     }
-    DevBuf<u64> d_occ(n_pat + 1, st);
-    {
-        DevBuf<u64> cnt(n_pat, st);
-        GRL_LAUNCH("fm_occ_count", n_pat * 24, fm_occ_count_kernel, grid_for(n_pat, INV_THREADS), INV_THREADS, 0, st, d_se.p, n_pat, cnt.p);
-        exclusive_scan<u64, u64>(cnt.p, d_occ.p, n_pat, d_occ.p + n_pat, st);
-    }
-    const u64 n_occ = d2h_scalar(d_occ.p + n_pat, st);
-    info->n_occ = n_occ;
-    if (n_occ > cap_occ) throw Error(GRLGPU_ERR_ARG, "locate: the occurrences need a capacity of " + std::to_string(n_occ));
-    t_loc.start();
-    DevBuf<u32> d_id(n_occ, st), d_pos(n_occ, st), flag(1, st);
-    const bool force_walk = (c->flags & GRLGPU_FLAG_FORCE_WALK) != 0, force_jump = (c->flags & GRLGPU_FLAG_FORCE_JUMP) != 0 && !force_walk;
-    bool walk = n_occ && !force_jump && (force_walk || !x.doc_ready);  // once built, the table answers every call
-    if (walk) {  // rows off a cycle reach a separator row within n LF steps and a row < N within n psi steps: the bound n never overflows
-        const u64 B = force_walk ? x.t.n : inv_walk_bound(x.t.n);
-        flag.zero();
-        GRL_LAUNCH("fm_locate_walk", n_occ * (8 + 8 + 8 * 2) + (u64)n_occ * 32 * 16, fm_locate_walk_kernel, grid_for(n_occ, INV_THREADS), INV_THREADS, 0, st, x.t.E.p, x.psi.p,
-                   (u32)x.t.N, x.t.sep, d_se.p, d_occ.p, n_pat, n_occ, (u32)B, d_id.p, d_pos.p, flag.p);
-        if (d2h_scalar(flag.p, st)) {
-            if (force_walk) throw Error(GRLGPU_ERR_ILL_FORMED, "locate: a walk of n steps met no separator (an LF cycle without separator)");
-            walk = false;
-        }
-    }
-    info->path = (walk || !n_occ) ? 0 : 1;
-    if (n_occ && !walk) {
-        if (!x.doc_ready) info->jump_rounds = fm_build_doc(x, flag.p, st, "locate");
-        GRL_LAUNCH("fm_locate_table", n_occ * (8 + 8 + 8 + 32), fm_locate_table_kernel, grid_for(n_occ, INV_THREADS), INV_THREADS, 0, st, x.doc.p, d_se.p, d_occ.p, n_pat, n_occ,
-                   d_id.p, d_pos.p);
-    }
-    t_loc.stop();
+    DevBuf<u64> d_occ;
+    DevBuf<u32> d_id, d_pos;
+    const u64 n_occ = fm_locate_rows(c, d_se.p, n_pat, cap_occ, d_occ, d_id, d_pos, t_loc, info);
     GRL_CUDA(cudaMemcpyAsync(occ_off, d_occ.p, (n_pat + 1) * 8, cudaMemcpyDeviceToHost, st));
     if (n_occ) {
         GRL_CUDA(cudaMemcpyAsync(str_id, d_id.p, n_occ * 4, cudaMemcpyDeviceToHost, st));
@@ -401,5 +528,133 @@ inline void fm_extract(grlgpu_ctx* c, const u32* str_id, const u32* from, const 
     if (n_cells) GRL_CUDA(cudaMemcpyAsync(out, dout.p, n_cells * w, cudaMemcpyDeviceToHost, st));
     t_all.stop();
     info->extract_ms = t_ext.ms();
+    info->device_ms = t_all.ms();  // waits for the copies
+}
+
+// approximate search: the first pool holds max(FM_APPROX_POOL_MIN, 4 n_pat) hits; a search that finds more runs once more with
+// the exact size. 20 bytes per pool entry, 12 more per hit for the sort.
+constexpr u64 FM_APPROX_POOL_MIN = 1ull << 16;
+
+// backtracking search of 0 < n_pat < 2^32 checked patterns with at most kmax substitutions: the hits in (pattern, sp) order in
+// d_se (sp, ep per hit) and d_mm (d per hit), per-pattern hit offsets in d_hoff (n_pat + 1); info->n_pat(_syms), n_hits and n_lf
+// are set. Returns the number of hits (GRLGPU_ERR_LIMIT from 2^32 hits).
+inline u64 fm_approx_search(grlgpu_ctx* c, const void* pat, const uint64_t* pat_off, u64 n_pat, int pat_bytes, u32 kmax, DevBuf<u64>& d_se, DevBuf<u8>& d_mm,
+                            DevBuf<u64>& d_hoff, grlgpu_fm_approx_t* info) {
+    cudaStream_t st = c->st;
+    FmIndex& x = *c->fm;
+    const u64 n_syms = pat_off[n_pat];
+    info->n_pat = n_pat;
+    info->n_pat_syms = n_syms;
+    d_hoff.alloc(n_pat + 1, st);
+    if (x.t.n == 0) {  // no rows: no hits
+        d_hoff.zero();
+        return 0;
+    }
+    DevBuf<u8> d_pat(n_syms * pat_bytes, st);
+    DevBuf<u64> d_off(n_pat + 1, st), cnt(n_pat, st), counters(2, st);
+    GRL_CUDA(cudaMemcpyAsync(d_pat.p, pat, n_syms * pat_bytes, cudaMemcpyHostToDevice, st));
+    GRL_CUDA(cudaMemcpyAsync(d_off.p, pat_off, (n_pat + 1) * 8, cudaMemcpyHostToDevice, st));
+    const FmView v = fm_view(x);
+    DevBuf<u64> key, ep_d;
+    DevBuf<u32> slot;
+    u64 cap = std::max(FM_APPROX_POOL_MIN, 4 * n_pat), h[2] = {0, 0};
+    for (int pass = 0; pass < 2; pass++) {  // the second pass only when the first pool was too small, with the exact size
+        key.alloc(cap, st);
+        ep_d.alloc(cap, st);
+        slot.alloc(cap, st);
+        counters.zero();
+        // bytes known only from the LF_c count read back below: added to this launch's record then
+        switch (pat_bytes) {
+            case 1: GRL_LAUNCH("fm_approx", 0, (fm_approx_kernel<u8>), grid_for(n_pat, INV_THREADS), INV_THREADS, 0, st, v, (const u8*)d_pat.p, d_off.p, n_pat, kmax, cap, key.p, slot.p, ep_d.p, cnt.p, counters.p); break;
+            case 2: GRL_LAUNCH("fm_approx", 0, (fm_approx_kernel<u16>), grid_for(n_pat, INV_THREADS), INV_THREADS, 0, st, v, (const u16*)d_pat.p, d_off.p, n_pat, kmax, cap, key.p, slot.p, ep_d.p, cnt.p, counters.p); break;
+            case 4: GRL_LAUNCH("fm_approx", 0, (fm_approx_kernel<u32>), grid_for(n_pat, INV_THREADS), INV_THREADS, 0, st, v, (const u32*)d_pat.p, d_off.p, n_pat, kmax, cap, key.p, slot.p, ep_d.p, cnt.p, counters.p); break;
+            default: GRL_LAUNCH("fm_approx", 0, (fm_approx_kernel<u64>), grid_for(n_pat, INV_THREADS), INV_THREADS, 0, st, v, (const u64*)d_pat.p, d_off.p, n_pat, kmax, cap, key.p, slot.p, ep_d.p, cnt.p, counters.p); break;
+        }
+        d2h_small(h, counters.p, sizeof(h), st);
+        // per LF_c evaluation two binary searches (run starts, c's slice), one 32 B sector per probe, as fm_count; the hits' stores
+        if (g_prof && g_prof->timing && !g_prof->pending.empty()) g_prof->pending.back().bytes = n_pat * 24 + n_syms * pat_bytes + h[1] * 64 * 32 + std::min(h[0], cap) * 20;
+        if (h[0] >> 32) throw Error(GRLGPU_ERR_LIMIT, "approximate search: 2^32 hits or more");
+        if (h[0] <= cap) break;
+        cap = h[0];
+    }
+    const u64 n_hits = h[0];
+    info->n_hits = n_hits;
+    info->n_lf = h[1];
+    exclusive_scan<u64, u64>(cnt.p, d_hoff.p, n_pat, d_hoff.p + n_pat, st);
+    {
+        DevBuf<u64> key_alt(n_hits, st);
+        DevBuf<u32> slot_alt(n_hits, st);
+        u64 *kp = key.p, *ka = key_alt.p;
+        u32 *vp = slot.p, *va = slot_alt.p;
+        radix_sort_pairs(&kp, &vp, &ka, &va, n_hits, 32 + bit_width64(n_pat - 1), st);
+        d_se.alloc(2 * n_hits, st);
+        d_mm.alloc(n_hits, st);
+        GRL_LAUNCH("fm_approx_gather", n_hits * (8 + 4 + 32 + 16 + 1), fm_approx_gather_kernel, grid_for(n_hits, INV_THREADS), INV_THREADS, 0, st, kp, vp, ep_d.p, n_hits, d_se.p, d_mm.p);
+    }
+    return n_hits;
+}
+
+// approximate count: the hits of 0 < n_pat < 2^32 checked patterns with at most kmax substitutions
+inline void fm_approx_count(grlgpu_ctx* c, const void* pat, const uint64_t* pat_off, u64 n_pat, int pat_bytes, u32 kmax, uint64_t* hit_off, uint64_t* sp_ep, uint8_t* hit_mm,
+                            u64 cap_hits, grlgpu_fm_approx_t* info) {
+    cudaStream_t st = c->st;
+    Timer t_all(st), t_search(st);
+    t_all.start();
+    t_search.start();
+    DevBuf<u64> d_se, d_hoff;
+    DevBuf<u8> d_mm;
+    const u64 n_hits = fm_approx_search(c, pat, pat_off, n_pat, pat_bytes, kmax, d_se, d_mm, d_hoff, info);
+    t_search.stop();
+    if (n_hits > cap_hits) {  // the times of the search already run
+        t_all.stop();
+        info->search_ms = t_search.ms();
+        info->device_ms = t_all.ms();
+        throw Error(GRLGPU_ERR_ARG, "approximate count: the hits need a capacity of " + std::to_string(n_hits));
+    }
+    GRL_CUDA(cudaMemcpyAsync(hit_off, d_hoff.p, (n_pat + 1) * 8, cudaMemcpyDeviceToHost, st));
+    if (n_hits) {
+        GRL_CUDA(cudaMemcpyAsync(sp_ep, d_se.p, 2 * n_hits * 8, cudaMemcpyDeviceToHost, st));
+        GRL_CUDA(cudaMemcpyAsync(hit_mm, d_mm.p, n_hits, cudaMemcpyDeviceToHost, st));
+    }
+    t_all.stop();
+    info->search_ms = t_search.ms();
+    info->device_ms = t_all.ms();  // waits for the copies
+    for (u64 i = 0; i < n_hits; i++) info->n_occ += sp_ep[2 * i + 1] - sp_ep[2 * i];
+}
+
+// approximate locate: every occurrence of every hit, with the d of its hit; pattern q's occurrences in row order
+inline void fm_approx_locate(grlgpu_ctx* c, const void* pat, const uint64_t* pat_off, u64 n_pat, int pat_bytes, u32 kmax, uint64_t* occ_off, u32* str_id, u32* str_pos,
+                             uint8_t* occ_mm, u64 cap_occ, grlgpu_fm_approx_t* info) {
+    cudaStream_t st = c->st;
+    Timer t_all(st), t_search(st), t_loc(st);
+    t_all.start();
+    t_search.start();
+    DevBuf<u64> d_se, d_hoff;
+    DevBuf<u8> d_mm;
+    const u64 n_hits = fm_approx_search(c, pat, pat_off, n_pat, pat_bytes, kmax, d_se, d_mm, d_hoff, info);
+    t_search.stop();
+    if (n_hits == 0) {
+        memset(occ_off, 0, (n_pat + 1) * 8);
+        t_all.stop();
+        info->search_ms = t_search.ms();
+        info->device_ms = t_all.ms();
+        return;
+    }
+    DevBuf<u64> d_occ;
+    DevBuf<u32> d_id, d_pos;
+    const u64 n_occ = fm_locate_rows(c, d_se.p, n_hits, cap_occ, d_occ, d_id, d_pos, t_loc, info);
+    DevBuf<u8> d_omm(n_occ, st);
+    DevBuf<u64> d_qoff(n_pat + 1, st);
+    GRL_LAUNCH("fm_approx_occ_mm", n_occ * (1 + 32 * 2) + n_hits, fm_approx_occ_mm_kernel, grid_for(n_occ, INV_THREADS), INV_THREADS, 0, st, d_occ.p, n_hits, d_mm.p, n_occ, d_omm.p);
+    GRL_LAUNCH("fm_approx_occ_off", (n_pat + 1) * (8 + 32 + 8), fm_approx_occ_off_kernel, grid_for(n_pat + 1, INV_THREADS), INV_THREADS, 0, st, d_occ.p, d_hoff.p, n_pat, d_qoff.p);
+    GRL_CUDA(cudaMemcpyAsync(occ_off, d_qoff.p, (n_pat + 1) * 8, cudaMemcpyDeviceToHost, st));
+    if (n_occ) {
+        GRL_CUDA(cudaMemcpyAsync(str_id, d_id.p, n_occ * 4, cudaMemcpyDeviceToHost, st));
+        GRL_CUDA(cudaMemcpyAsync(str_pos, d_pos.p, n_occ * 4, cudaMemcpyDeviceToHost, st));
+        GRL_CUDA(cudaMemcpyAsync(occ_mm, d_omm.p, n_occ, cudaMemcpyDeviceToHost, st));
+    }
+    t_all.stop();
+    info->search_ms = t_search.ms();
+    info->locate_ms = t_loc.ms();
     info->device_ms = t_all.ms();  // waits for the copies
 }

@@ -1686,6 +1686,30 @@ int grlgpu_fm_locate(grlgpu_ctx* ctx, const void* pat, const uint64_t* pat_off, 
     return guarded(ctx, [&] { fm_query(ctx, pat, pat_off, n_pat, pat_bytes, nullptr, occ_off, str_id, str_pos, cap_occ, info); });
 }
 
+int grlgpu_fm_approx_count(grlgpu_ctx* ctx, const void* pat, const uint64_t* pat_off, uint64_t n_pat, int pat_bytes, uint32_t max_mismatches, uint64_t* hit_off,
+                           uint64_t* sp_ep, uint8_t* hit_mm, uint64_t cap_hits, grlgpu_fm_approx_t* info) {
+    if (!ctx || !info) return GRLGPU_ERR_ARG;
+    memset(info, 0, sizeof(*info));
+    if (const int rc = fm_patterns_ok(pat, pat_off, n_pat, pat_bytes)) return rc;
+    if (max_mismatches > FM_APPROX_MAX_K || (n_pat && !hit_off) || (cap_hits && (!sp_ep || !hit_mm))) return GRLGPU_ERR_ARG;
+    if (!ctx->fm) return GRLGPU_ERR_STATE;
+    if (n_pat >> 32) return GRLGPU_ERR_LIMIT;
+    if (n_pat == 0) return GRLGPU_OK;
+    return guarded(ctx, [&] { fm_approx_count(ctx, pat, pat_off, n_pat, pat_bytes, max_mismatches, hit_off, sp_ep, hit_mm, cap_hits, info); });
+}
+
+int grlgpu_fm_approx_locate(grlgpu_ctx* ctx, const void* pat, const uint64_t* pat_off, uint64_t n_pat, int pat_bytes, uint32_t max_mismatches, uint64_t* occ_off,
+                            uint32_t* str_id, uint32_t* str_pos, uint8_t* occ_mm, uint64_t cap_occ, grlgpu_fm_approx_t* info) {
+    if (!ctx || !info) return GRLGPU_ERR_ARG;
+    memset(info, 0, sizeof(*info));
+    if (const int rc = fm_patterns_ok(pat, pat_off, n_pat, pat_bytes)) return rc;
+    if (max_mismatches > FM_APPROX_MAX_K || (n_pat && !occ_off) || (cap_occ && (!str_id || !str_pos || !occ_mm))) return GRLGPU_ERR_ARG;
+    if (!ctx->fm) return GRLGPU_ERR_STATE;
+    if (n_pat >> 32) return GRLGPU_ERR_LIMIT;
+    if (n_pat == 0) return GRLGPU_OK;
+    return guarded(ctx, [&] { fm_approx_locate(ctx, pat, pat_off, n_pat, pat_bytes, max_mismatches, occ_off, str_id, str_pos, occ_mm, cap_occ, info); });
+}
+
 int grlgpu_fm_extract(grlgpu_ctx* ctx, const uint32_t* str_id, const uint32_t* from, const uint32_t* len, uint64_t n_req, int cell_bytes, uint64_t* out_off, void* out,
                       uint64_t cap_cells, grlgpu_fm_extract_t* info) {
     if (!ctx || !info) return GRLGPU_ERR_ARG;

@@ -76,13 +76,21 @@ inline void read_requests(const std::string& path, uint64_t n_strings, std::vect
     }
 }
 
-// one output line: the count, then " k:p" per occurrence in row order
+// one output line: the count, then " k:p" per occurrence in row order, or " k:p:d" with the mismatches d of each (search with -k)
 template <class T>
-inline void put_line(std::string& out, uint64_t count, const T* k, const T* p) {
+inline void put_line(std::string& out, uint64_t count, const T* k, const T* p, const uint8_t* d = nullptr) {
     out += std::to_string(count);
     if (k)
-        for (uint64_t o = 0; o < count; o++) { out += ' '; out += std::to_string(k[o]); out += ':'; out += std::to_string(p[o]); }
+        for (uint64_t o = 0; o < count; o++) {
+            out += ' '; out += std::to_string(k[o]); out += ':'; out += std::to_string(p[o]);
+            if (d) { out += ':'; out += std::to_string(d[o]); }
+        }
     out += '\n';
+}
+// the -k argument of the search tools: 0 to 3 mismatches
+inline uint32_t parse_mismatches(const char* s) {
+    if (s[0] < '0' || s[0] > '3' || s[1]) throw std::runtime_error(std::string("-k takes 0, 1, 2 or 3 mismatches, not \"") + s + "\"");
+    return (uint32_t)(s[0] - '0');
 }
 inline void flush_out(std::string& out, bool force) {
     if (!force && out.size() < (1u << 20)) return;

@@ -113,6 +113,64 @@ struct RlBwt {
         }
         return {sp, ep};
     }
+    // search with at most k substitutions: every distinct string Q with Hamming(P, Q) <= k that occurs, as its rows [sp, ep) and
+    // d = Hamming(P, Q), by ascending sp. A depth-first backward search over k + 1 frames, frame d the state after d substitutions
+    // (cells 0 .. t - 1 still to match, the interval so far, the next symbol to substitute), as the device search does. A pattern
+    // cell that is the separator or an absent symbol never matches; substitutions use every symbol but the separator.
+    struct Hit { uint64_t sp, ep; uint32_t d; };
+    std::vector<Hit> approx_count(const uint64_t* P, size_t m, uint32_t k) const {
+        // the candidates of a frame: the symbols of the runs [sp, ep) spans when they are fewer than the alphabet (narrow intervals
+        // of large alphabets), else every symbol
+        struct Frame { size_t t; uint64_t sp, ep; size_t cur; std::vector<uint64_t> cand; };
+        auto candidates = [&](uint64_t sp, uint64_t ep) {
+            const size_t a = (size_t)(std::upper_bound(start.begin(), start.end(), sp) - start.begin()) - 1;
+            const size_t b = (size_t)(std::lower_bound(start.begin(), start.end(), ep) - start.begin());
+            if (b - a >= c_sym.size()) return c_sym;
+            std::vector<uint64_t> c(runs.sym.begin() + (long)a, runs.sym.begin() + (long)b);
+            std::sort(c.begin(), c.end());
+            c.erase(std::unique(c.begin(), c.end()), c.end());
+            return c;
+        };
+        std::vector<Hit> hits;
+        if (m >= n) return hits;  // a window inside a string has fewer cells than the BWT has rows
+        std::vector<Frame> f;
+        f.push_back({m, 0, n, 0, k ? candidates(0, n) : std::vector<uint64_t>()});
+        while (!f.empty()) {
+            Frame& F = f.back();
+            const uint32_t d = (uint32_t)(f.size() - 1);
+            if (F.t == 0) {
+                hits.push_back({F.sp, F.ep, d});
+                f.pop_back();
+                continue;
+            }
+            const uint64_t own = P[F.t - 1];
+            if (d < k) {
+                uint64_t sp = 0, ep = 0;
+                while (F.cur < F.cand.size() && sp == ep) {
+                    const uint64_t c = F.cand[F.cur++];
+                    if (c == sep || c == own) continue;
+                    sp = C.at(c) + rank(c, F.sp);
+                    ep = C.at(c) + rank(c, F.ep);
+                }
+                if (sp < ep) {
+                    const size_t t = F.t - 1;
+                    f.push_back({t, sp, ep, 0, d + 1 < k && t ? candidates(sp, ep) : std::vector<uint64_t>()});
+                    continue;
+                }
+            }
+            const auto it = C.find(own);
+            if (own == sep || it == C.end()) { f.pop_back(); continue; }
+            const uint64_t sp = it->second + rank(own, F.sp), ep = it->second + rank(own, F.ep);
+            if (sp >= ep) { f.pop_back(); continue; }
+            F.t--;
+            F.sp = sp;
+            F.ep = ep;
+            F.cur = 0;
+            F.cand = d < k && F.t ? candidates(sp, ep) : std::vector<uint64_t>();
+        }
+        std::sort(hits.begin(), hits.end(), [](const Hit& a, const Hit& b) { return a.sp < b.sp; });
+        return hits;
+    }
     // psi(j) = LF^-1(j): the c of F row j, then the run of c that holds its (j - C[c])-th occurrence
     uint64_t psi(uint64_t j) const {
         const size_t d = (size_t)(std::upper_bound(c_val.begin(), c_val.end(), j) - c_val.begin()) - 1;

@@ -222,6 +222,34 @@ int grlgpu_fm_locate(grlgpu_ctx* ctx, const void* pat, const uint64_t* pat_off, 
                      uint32_t* str_id, uint32_t* str_pos, uint64_t cap_occ, grlgpu_fm_query_t* info);
 int grlgpu_fm_drop(grlgpu_ctx* ctx);
 
+/* search with mismatches on the loaded index (the host tool fm_query -k is the general path and the same answers). An occurrence
+ * of P with d mismatches is a pair (k, p) such that the window S_k[p .. p + m) lies inside string k and differs from P in exactly
+ * d <= max_mismatches positions (Hamming distance). A pattern cell that is the separator or a symbol absent from the BWT never
+ * matches; substitutions use the symbols of the BWT other than the separator. A hit is one distinct string Q with
+ * Hamming(P, Q) <= max_mismatches that occurs: its rows [sp, ep) and its d. Hits of one pattern are disjoint and listed by
+ * ascending sp, so its occurrences are listed in row order. max_mismatches = 0 gives the answers of grlgpu_fm_count / _locate
+ * (without the empty intervals).
+ *   grlgpu_fm_approx_count   pattern q's hits are hit_off[q] .. hit_off[q + 1] (n_pat + 1 entries): sp_ep[2h], sp_ep[2h + 1] and
+ *                            hit_mm[h] = d. One thread per pattern runs a depth-first backward search over at most
+ *                            max_mismatches + 1 frames, pruning every empty interval.
+ *   grlgpu_fm_approx_locate  every occurrence of every hit: occ_off[q] .. occ_off[q + 1] are pattern q's, str_id = k, str_pos = p,
+ *                            occ_mm = d, in row order; the locate paths, flags and table of grlgpu_fm_locate.
+ * GRLGPU_ERR_ARG: the pattern checks of grlgpu_fm_count, max_mismatches > 3, a null array, or cap_hits < n_hits / cap_occ < n_occ
+ * (info->n_hits / n_occ then hold the number needed; nothing is written). GRLGPU_ERR_STATE: no index loaded. GRLGPU_ERR_LIMIT:
+ * n_pat >= 2^32 or 2^32 hits or more. GRLGPU_ERR_ILL_FORMED: locate only, as grlgpu_fm_locate. n_pat = 0 is accepted. */
+typedef struct {
+    uint64_t n_pat, n_pat_syms;     /* patterns and their cells */
+    uint64_t n_hits;                /* hits (written, or needed when cap_hits is too small) */
+    uint64_t n_occ;                 /* sum of ep - sp over the hits (locate: written, or needed when cap_occ is too small) */
+    uint64_t n_lf;                  /* LF_c evaluations of the search */
+    uint32_t path, jump_rounds;     /* locate, as grlgpu_fm_query_t */
+    float device_ms, search_ms, locate_ms; /* CUDA events on the context's stream: whole call (copies included) / search / locate */
+} grlgpu_fm_approx_t;
+int grlgpu_fm_approx_count(grlgpu_ctx* ctx, const void* pat, const uint64_t* pat_off, uint64_t n_pat, int pat_bytes, uint32_t max_mismatches,
+                           uint64_t* hit_off /* n_pat + 1 */, uint64_t* sp_ep /* 2 * cap_hits */, uint8_t* hit_mm, uint64_t cap_hits, grlgpu_fm_approx_t* info);
+int grlgpu_fm_approx_locate(grlgpu_ctx* ctx, const void* pat, const uint64_t* pat_off, uint64_t n_pat, int pat_bytes, uint32_t max_mismatches,
+                            uint64_t* occ_off /* n_pat + 1 */, uint32_t* str_id, uint32_t* str_pos, uint8_t* occ_mm, uint64_t cap_occ, grlgpu_fm_approx_t* info);
+
 /* extract from the loaded index (the host tool fm_extract is the general path and writes the same cells):
  *   grlgpu_fm_extract  substrings of the indexed strings: request q = (str_id[q], from[q], len[q]) yields S_k[from .. e) with
  *                      k = str_id[q], e = min(from + len, L_k) (computed in 64 bits, so len = UINT32_MAX means "to the end");
