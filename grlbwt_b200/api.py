@@ -140,6 +140,8 @@ def lib_gpu():
         L.grlgpu_fm_drop.argtypes = [vp]
         L.grlgpu_selftest_scan.argtypes = [vp, u64, vp, vp]
         L.grlgpu_selftest_sort.argtypes = [vp, vp, u64, C.c_int]
+        L.grlgpu_selftest_scan_same.argtypes = [vp, u64, C.c_int, u64, C.c_int, vp, vp]
+        L.grlgpu_selftest_sort32.argtypes = [vp, vp, u64, C.c_int, C.c_int]
         L.grlgpu_selftest_compact.argtypes = [vp, vp, u64, vp, vp]
         L.grlgpu_selftest_ipc_rendezvous.argtypes = [C.c_char_p, C.c_int, C.c_int, C.c_int]
         _gpu = L
@@ -734,6 +736,28 @@ def selftest_scan(a: np.ndarray):
 def selftest_sort(keys: np.ndarray, vals: np.ndarray, n_bits: int):
     k, v = np.ascontiguousarray(keys, np.uint64).copy(), np.ascontiguousarray(vals, np.uint32).copy()
     rc = lib_gpu().grlgpu_selftest_sort(_ptr(k), _ptr(v), k.size, n_bits)
+    if rc != 0:
+        raise GrlGpuError(rc, lib_gpu().grlgpu_strerror(rc).decode())
+    return k, v
+
+
+def selftest_scan_same(a: np.ndarray, elem_offset: int = 0, in_place: bool = False):
+    """exclusive scan of a uint32 (mod 2^32) or uint64 array into its own type -> (out, total); the device arrays start elem_offset
+    elements into their allocation"""
+    a = np.ascontiguousarray(a)
+    if a.dtype not in (np.uint32, np.uint64):
+        raise GrlGpuError(-1, "selftest_scan_same: uint32 or uint64 input")
+    out, tot = np.zeros(a.size, a.dtype), np.zeros(1, a.dtype)
+    rc = lib_gpu().grlgpu_selftest_scan_same(_ptr(a), a.size, a.dtype.itemsize, elem_offset, int(in_place), _ptr(out), _ptr(tot))
+    if rc != 0:
+        raise GrlGpuError(rc, lib_gpu().grlgpu_strerror(rc).decode())
+    return out, int(tot[0])
+
+
+def selftest_sort32(keys: np.ndarray, vals: np.ndarray, n_bits: int = 32, partition_shift: int = -1):
+    """(uint32 key, uint32 value) pairs: sorted on the low n_bits, or one partition pass on the digit at partition_shift (>= 0)"""
+    k, v = np.ascontiguousarray(keys, np.uint32).copy(), np.ascontiguousarray(vals, np.uint32).copy()
+    rc = lib_gpu().grlgpu_selftest_sort32(_ptr(k), _ptr(v), k.size, n_bits, partition_shift)
     if rc != 0:
         raise GrlGpuError(rc, lib_gpu().grlgpu_strerror(rc).decode())
     return k, v

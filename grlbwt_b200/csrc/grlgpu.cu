@@ -436,6 +436,14 @@ void dict_offsets(Round& R) {
     R.max_len = hmx[1];
 }
 
+// A round's level values go up to A + 3 + tot + 1 with tot <= nE (exact_par_phase.cpp:19-20), and its sort codes up to A + 1.
+// The round refuses an input for which A + nE + 8 exceeds 2^64: that keeps every one of them, and the sums below, inside u64.
+inline void check_level_range(u64 A, u64 nE) {
+    if (A > ~0ull - 7 - nE) throw Error(GRLGPU_ERR_LIMIT, "symbols too close to 2^64: the alphabet plus the round's dictionary exceeds 64 bits");
+}
+// 64-bit level symbols when A + nE + 8 >= 2^32 (written so that it does not wrap: check_level_range holds)
+inline bool level_is_wide(u64 A, u64 nE) { return A + nE + 7 >= 0xffffffffull; }
+
 template <class CellT, bool FIRST, class SymT>
 void stage_gather(Round& R) {
     grlgpu_ctx* c = R.c;
@@ -779,9 +787,8 @@ void run_round_t(grlgpu_ctx* c, grlgpu_round_t* out) {
     t_text.stop();
     t_dict.start();
     const u64 A = c->alphabet;
-    // rule values go up to A + 3 + tot + 1 with tot <= nE
-    const bool wide = (A + R.nE + 8) >= (1ull << 32);
-    if (wide) { stage_gather<CellT, FIRST, u64>(R); stage_dict<u64>(R); }
+    check_level_range(A, R.nE);
+    if (level_is_wide(A, R.nE)) { stage_gather<CellT, FIRST, u64>(R); stage_dict<u64>(R); }
     else { stage_gather<CellT, FIRST, u32>(R); stage_dict<u32>(R); }
     t_dict.stop();
     if (c->flags & GRLGPU_FLAG_KEEP_DICT) {
@@ -851,6 +858,7 @@ void compute_stats(grlgpu_ctx* c) {
         s.max_sym_freq = m;
     } else { s.min_sym = h.min_sym; s.max_sym = h.max_sym; }
     if (s.sep_sym != s.min_sym) throw Error(GRLGPU_ERR_ILL_FORMED, "the collection is ill formed: the last symbol is not the smallest symbol");
+    if (s.max_sym == ~0ull) throw Error(GRLGPU_ERR_LIMIT, "symbol 2^64 - 1: the alphabet max_sym + 1 does not fit 64 bits");
     // longest string: positions of the separators -> adjacent differences
     {
         const u64 n_words = div_up(c->n, 32);
@@ -1795,6 +1803,36 @@ int grlgpu_selftest_sort(uint64_t* keys, uint32_t* vals, uint64_t n, int n_bits)
         radix_sort_pairs(&kp, &vp, &kap, &vap, n, n_bits, st);
         GRL_CUDA(cudaStreamSynchronize(st));
         GRL_CUDA(cudaMemcpy(keys, kp, n * 8, cudaMemcpyDeviceToHost));
+        GRL_CUDA(cudaMemcpy(vals, vp, n * 4, cudaMemcpyDeviceToHost));
+    });
+}
+int grlgpu_selftest_scan_same(const void* in, uint64_t n, int elem_bytes, uint64_t elem_offset, int in_place, void* out_exclusive, void* total) {
+    if ((elem_bytes != 4 && elem_bytes != 8) || (n && (!in || !out_exclusive)) || !total) return GRLGPU_ERR_ARG;
+    return guarded(nullptr, [&] {
+        cudaStream_t st = nullptr;
+        const u64 nb = n * (u64)elem_bytes, ob = elem_offset * (u64)elem_bytes;
+        DevBuf<u8> din(ob + nb + 1, st), dout(ob + nb + 1, st), tot(8, st);
+        GRL_CUDA(cudaMemcpy(din.p + ob, in, nb, cudaMemcpyHostToDevice));
+        u8* o = in_place ? din.p + ob : dout.p + ob;
+        if (elem_bytes == 4) exclusive_scan<u32, u32>((const u32*)(din.p + ob), (u32*)o, n, (u32*)tot.p, st);
+        else exclusive_scan<u64, u64>((const u64*)(din.p + ob), (u64*)o, n, (u64*)tot.p, st);
+        GRL_CUDA(cudaStreamSynchronize(st));
+        GRL_CUDA(cudaMemcpy(out_exclusive, o, nb, cudaMemcpyDeviceToHost));
+        GRL_CUDA(cudaMemcpy(total, tot.p, elem_bytes, cudaMemcpyDeviceToHost));
+    });
+}
+int grlgpu_selftest_sort32(uint32_t* keys, uint32_t* vals, uint64_t n, int n_bits, int partition_shift) {
+    if (n && (!keys || !vals)) return GRLGPU_ERR_ARG;
+    return guarded(nullptr, [&] {
+        cudaStream_t st = nullptr;
+        DevBuf<u32> k(n, st), ka(n, st), v(n, st), va(n, st);
+        GRL_CUDA(cudaMemcpy(k.p, keys, n * 4, cudaMemcpyHostToDevice));
+        GRL_CUDA(cudaMemcpy(v.p, vals, n * 4, cudaMemcpyHostToDevice));
+        u32 *kp = k.p, *kap = ka.p, *vp = v.p, *vap = va.p;
+        if (partition_shift >= 0) radix_partition_u32(&kp, &vp, &kap, &vap, n, partition_shift, st);
+        else radix_sort_pairs_u32(&kp, &vp, &kap, &vap, n, n_bits, st);
+        GRL_CUDA(cudaStreamSynchronize(st));
+        GRL_CUDA(cudaMemcpy(keys, kp, n * 4, cudaMemcpyDeviceToHost));
         GRL_CUDA(cudaMemcpy(vals, vp, n * 4, cudaMemcpyDeviceToHost));
     });
 }

@@ -916,11 +916,11 @@ void mg2_round_t(grlgpu_ctx* c, Comm& cm, grlgpu_round_t* out) {
     clk.lap("M owner dedup");
     // ---- D .. E4: entries of my phrases, ranking by key range, rules by rank range ----
     const u64 A = c->alphabet;
+    check_level_range(A, nE_g);  // every rank has the same A and nE_g: all of them refuse together
     P.sym_bits = bit_width64(A + 1);
     P.K = std::max(1, 64 / P.sym_bits);
     P.spare = P.sym_bits * P.K < 64 ? 64 - P.sym_bits * P.K : 0;
-    const bool wide = (A + nE_g + 8) >= (1ull << 32);  // rule values go up to A + 3 + tot + 1 with tot <= nE
-    if (wide) { mg2_gather<CellT, FIRST, u64>(c, P); clk.lap("D entries"); mg2_rank<u64>(c, cm, P, S); }
+    if (level_is_wide(A, nE_g)) { mg2_gather<CellT, FIRST, u64>(c, P); clk.lap("D entries"); mg2_rank<u64>(c, cm, P, S); }
     else { mg2_gather<CellT, FIRST, u32>(c, P); clk.lap("D entries"); mg2_rank<u32>(c, cm, P, S); }
     clk.lap("(rank stages)");
     // ---- E5: metasymbols back to the ranks that saw the phrases, then the local rewrite ----

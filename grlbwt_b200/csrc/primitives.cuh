@@ -237,7 +237,8 @@ struct BitmapCompactor {
 };
 
 // ------------------------------------------------------------------------------------------------
-// LSD radix sort of (u64 or u32 key, u32 value) pairs on key bits [0, n_bits), 8 bits per pass, stable.
+// LSD radix sort of (u64 or u32 key, u32 value) pairs on key bits [0, n_bits), 8 bits per pass, stable. n_bits is rounded up
+// to whole 8-bit digits; key bits above those are carried unsorted.
 // Per pass: per-tile digit histogram -> exclusive scan of the digit-major table -> ranked scatter
 // through shared memory (writes of one digit from one tile are contiguous).
 // ------------------------------------------------------------------------------------------------

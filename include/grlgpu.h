@@ -25,7 +25,8 @@ enum grlgpu_status {
     GRLGPU_ERR_CUDA = -3,       /* CUDA runtime error / no device */
     GRLGPU_ERR_NOMEM = -4,      /* device memory exhausted */
     GRLGPU_ERR_STATE = -5,      /* call out of order (no text, phase already finished, ...) */
-    GRLGPU_ERR_LIMIT = -6       /* dictionary of one round exceeds 2^32 symbols or the table 2^31 slots */
+    GRLGPU_ERR_LIMIT = -6       /* dictionary of one round exceeds 2^32 symbols or the table 2^31 slots; symbol 2^64 - 1, or
+                                   alphabet + dictionary symbols + 8 above 2^64 */
 };
 
 /* flags of grlgpu_create */
@@ -375,6 +376,12 @@ int grlgpu_profile_entry(grlgpu_ctx* ctx, int index, char* name, int name_cap, u
 /* self-test hooks for the device primitives the path is built from (host buffers in / out) */
 int grlgpu_selftest_scan(const uint32_t* in, uint64_t n, uint64_t* out_exclusive, uint64_t* total);
 int grlgpu_selftest_sort(uint64_t* keys, uint32_t* vals, uint64_t n, int n_bits);
+/* exclusive scan with input and output of one type (elem_bytes 4: uint32_t, wrapping mod 2^32; 8: uint64_t). The device arrays start
+ * elem_offset elements into their allocation (an odd offset makes them not 16-byte aligned); in_place != 0 scans the input array over itself */
+int grlgpu_selftest_scan_same(const void* in, uint64_t n, int elem_bytes, uint64_t elem_offset, int in_place, void* out_exclusive, void* total);
+/* (uint32_t key, uint32_t value) pairs: partition_shift < 0 sorts on the low n_bits (radix_sort_pairs_u32, whole 8-bit digits), else one
+ * stable partition pass on the digit at partition_shift (radix_partition_u32) */
+int grlgpu_selftest_sort32(uint32_t* keys, uint32_t* vals, uint64_t n, int n_bits, int partition_shift);
 int grlgpu_selftest_compact(const uint32_t* bits, const uint32_t* prev_bits, uint64_t n_bits, uint64_t* out, uint64_t* count);
 /* the shared-memory rendezvous of the "ipc" backend WITHOUT its device windows (runs on a box without a GPU): `rounds` barriers and small
  * all-gathers of varying size between `world` processes that all pass the same `session`; GRLGPU_OK when every byte arrived intact */
