@@ -64,6 +64,11 @@ class FmExtract(C.Structure):
                [(k, C.c_float) for k in ("device_ms", "extract_ms")]
 
 
+class FmLcp(C.Structure):
+    _fields_ = [(k, C.c_uint64) for k in ("n", "n_irreducible", "sum_irreducible")] + [(k, C.c_uint32) for k in ("path", "jump_rounds")] + \
+               [(k, C.c_float) for k in ("device_ms", "sa_ms", "lcp_ms")]
+
+
 class BwtResult(C.Structure):
     _fields_ = [("n_runs", C.c_uint64), ("sb", C.c_uint64), ("fb", C.c_uint64), ("syms", C.POINTER(C.c_uint64)),
                 ("lens", C.POINTER(C.c_uint64)), ("n_rounds", C.c_uint64), ("h2d_ms", C.c_double), ("par_phase_ms", C.c_double),
@@ -137,6 +142,7 @@ def lib_gpu():
         L.grlgpu_fm_approx_count.argtypes = [vp, vp, vp, u64, C.c_int, C.c_uint32, vp, vp, vp, u64, C.POINTER(FmApprox)]
         L.grlgpu_fm_approx_locate.argtypes = [vp, vp, vp, u64, C.c_int, C.c_uint32, vp, vp, vp, vp, u64, C.POINTER(FmApprox)]
         L.grlgpu_fm_extract.argtypes = [vp, vp, vp, vp, u64, C.c_int, vp, vp, u64, C.POINTER(FmExtract)]
+        L.grlgpu_fm_lcp.argtypes = [vp, vp, u64, C.POINTER(FmLcp)]
         L.grlgpu_fm_drop.argtypes = [vp]
         L.grlgpu_selftest_scan.argtypes = [vp, u64, vp, vp]
         L.grlgpu_selftest_sort.argtypes = [vp, vp, u64, C.c_int]
@@ -453,6 +459,18 @@ class GrlGpu:
             d["jump_rounds"] = max(d["jump_rounds"], sizing["jump_rounds"])
         n = d["n_cells"]
         return out_off, (cells[:n].copy() if n < cap // 2 else cells[:n]), d   # lengths past the strings: do not keep the whole allocation
+
+    def fm_lcp(self):
+        """LCP array of the loaded index -> (lcp, info): lcp is a uint32 array of n entries in row order, lcp[j] the number of
+        leading cells the suffixes of rows j - 1 and j share (a separator never matches, so rows j < N have 0; lcp[0] = 0), and
+        info the dict of grlgpu_fm_lcp_t. A first call without an array reads n."""
+        info = FmLcp()
+        rc = self._L.grlgpu_fm_lcp(self._h, None, 0, C.byref(info))
+        if rc != -1 or info.n == 0:   # no rows, or an error other than the missing array
+            return np.zeros(0, np.uint32), self._fm_call(rc, info)
+        lcp = np.empty(int(info.n), np.uint32)
+        d = self._fm_call(self._L.grlgpu_fm_lcp(self._h, _ptr(lcp), lcp.size, C.byref(info)), info)
+        return lcp, d
 
     def fm_drop(self):
         """Frees this context's FM-index"""

@@ -16,6 +16,9 @@
 //            built it) and kept for every later call; the walk then starts at the first sample at or after e.
 //   approx   count / locate with at most k <= 3 substitutions: one thread per pattern, a depth-first backward search over at most
 //            k + 1 frames (fm_approx_kernel), hits appended to a pool, sorted by (pattern, sp); locate runs on the hits' intervals
+//   lcp      LCP array of every row: SA and the text T from the walk per string (or the locate table), then one warp per
+//            irreducible row (a run head or a separator symbol) compares T at SA[j] and SA[j - 1]; the other rows follow from
+//            PLCP[i] + i = PLCP[i - 1] + (i - 1), filled in by a max-scan over text positions, and are gathered back to rows
 // Convention of reverse_bwt and grlgpu_invert: the separator is the smallest symbol of a non-empty record, N its count, strings in
 // input order. A pattern containing the separator or a symbol outside the directory has no occurrence; every empty interval is
 // reported as sp = ep = 0 (the host tool fm_query does the same). Positions and symbols are 32-bit, as for the inversion.
@@ -292,6 +295,89 @@ __global__ void __launch_bounds__(INV_THREADS) fm_extract_write_kernel(const u64
         r = inv_lf(x);
     }
     sg.flush();
+}
+
+// ---- LCP (DESIGN.md §12, "LCP"): row j's suffix is S_k[p .. L_k) $_k, string k occupies T[o_k .. o_k + L_k] with o_k = off[k] + k
+// (off = exclusive scan of L), its separator last; a separator cell never matches ----
+// walk path: string k from row k (position L_k) down to position 0, writing SA of every row it meets and its cells of T
+static __global__ void __launch_bounds__(INV_THREADS) fm_lcp_walk_kernel(const u64* __restrict__ E, u32 N, u32 sep, const u32* __restrict__ len, const u32* __restrict__ off,
+                                                                         u32* __restrict__ SA, u32* __restrict__ T) {
+    const u32 k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= N) return;
+    const u32 L = len[k], o = off[k] + k;
+    InvStage<u32> sg{(u8*)T, (u64)o * 4, ((u64)o + L + 1) * 4};
+    sg.put((u64)o + L, sep);
+    SA[k] = o + L;
+    u32 r = k;
+    for (u32 p = L; p > 0; p--) {  // L steps, counted by the count pass
+        const u64 e = ld_gather8(E + r);
+        r = inv_lf(e);
+        sg.put((u64)o + p - 1, inv_sym(e));  // the row at position p holds S_k[p - 1]
+        SA[r] = o + p - 1;
+    }
+    sg.flush();
+}
+// table path: L_k = the offset of row k < N ($_k) in the locate table
+static __global__ void __launch_bounds__(INV_THREADS) fm_lcp_len_kernel(const u64* __restrict__ doc, u32 N, u32* __restrict__ len) {
+    const u32 k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k < N) len[k] = (u32)doc[k];
+}
+// table path: one thread per row, (k, p) from the locate table
+static __global__ void __launch_bounds__(INV_THREADS) fm_lcp_table_kernel(const u64* __restrict__ E, const u64* __restrict__ doc, u32 n, u32 N, u32 sep,
+                                                                          const u32* __restrict__ off, u32* __restrict__ SA, u32* __restrict__ T) {
+    const u32 j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= n) return;
+    const u64 t = doc[j];
+    const u32 k = (u32)(t >> 32), p = (u32)t, i = ld_gather4(off + k) + k + p;
+    SA[j] = i;
+    if (p) T[i - 1] = inv_sym(E[j]);
+    if (j < N) T[i] = sep;
+}
+// irreducible rows: j >= N whose BWT symbol is the separator or differs from row j - 1's, one bit each (bits[j / 32]); every other
+// row j >= N has LCP[LF(j)] = 1 + LCP[j]. The rows j < N ($_k) store PLCP 0 as a[SA[j]] = SA[j] (a is zero on entry).
+static __global__ void __launch_bounds__(INV_THREADS) fm_lcp_flags_kernel(const u64* __restrict__ E, const u32* __restrict__ SA, u32 n, u32 N, u32 sep, u32* __restrict__ bits,
+                                                                          u32* __restrict__ a) {
+    const u32 j = blockIdx.x * blockDim.x + threadIdx.x;
+    bool irr = false;
+    if (j < N) {
+        const u32 i = SA[j];
+        a[i] = i;
+    } else if (j < n) {
+        const u32 c = inv_sym(E[j]);
+        irr = c == sep || c != inv_sym(E[j - 1]);
+    }
+    const u32 m = __ballot_sync(0xffffffffu, irr);
+    if (lane_id() == 0 && j < n) bits[j >> 5] = m;
+}
+// one warp per irreducible row j (grid-stride): LCE of T[SA[j] ..] and T[SA[j - 1] ..], 32 cells a step, the first mismatch or
+// separator found by a ballot; a[SA[j]] = LCE + SA[j]; the LCEs summed into *sum, one atomic per warp
+static __global__ void __launch_bounds__(INV_THREADS) fm_lcp_lce_kernel(const u32* __restrict__ rows, u64 n_rows, const u32* __restrict__ SA, const u32* __restrict__ T, u32 n,
+                                                                        u32 sep, u32* __restrict__ a, u64* sum) {
+    const u32 lane = lane_id();
+    const u64 warps = ((u64)gridDim.x * blockDim.x) >> 5;
+    u64 tot = 0;
+    for (u64 w = ((u64)blockIdx.x * blockDim.x + threadIdx.x) >> 5; w < n_rows; w += warps) {  // warp-uniform
+        const u32 j = rows[w], x = SA[j], y = SA[j - 1];
+        u32 l = 0;
+        for (;;) {  // both strings end in a separator: at most min of their remaining lengths / 32 + 1 steps
+            const u32 px = x + l + lane, py = y + l + lane;  // x + l, y + l < n < 2^32 - 16 while the loop runs
+            const u32 cx = px < n ? T[px] : sep, cy = py < n ? T[py] : sep;
+            const u32 stop = __ballot_sync(0xffffffffu, cx != cy || cx == sep);
+            if (stop) { l += __ffs(stop) - 1; break; }
+            l += 32;
+        }
+        if (lane == 0) a[x] = x + l;
+        tot += l;
+    }
+    if (lane == 0 && tot) atomicAdd(sum, tot);
+}
+// M[i + 1] = max(a[0 .. i]) = PLCP[i] + i: LCP[j] = PLCP[SA[j]] for j >= N, 0 below
+static __global__ void __launch_bounds__(INV_THREADS) fm_lcp_gather_kernel(const u32* __restrict__ SA, const u32* __restrict__ M, u32 n, u32 N, u32* __restrict__ lcp) {
+    const u32 j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= n) return;
+    if (j < N) { lcp[j] = 0; return; }
+    const u32 i = SA[j];
+    lcp[j] = ld_gather4(M + i + 1) - i;
 }
 
 inline FmView fm_view(const FmIndex& x) {
@@ -657,4 +743,75 @@ inline void fm_approx_locate(grlgpu_ctx* c, const void* pat, const uint64_t* pat
     info->search_ms = t_search.ms();
     info->locate_ms = t_loc.ms();
     info->device_ms = t_all.ms();  // waits for the copies
+}
+
+// LCP of every row of the loaded index (n > 0) into the host array lcp (n entries, checked by the caller)
+inline void fm_lcp(grlgpu_ctx* c, u32* lcp, grlgpu_fm_lcp_t* info) {
+    cudaStream_t st = c->st;
+    FmIndex& x = *c->fm;
+    const u32 n = (u32)x.t.n, N = (u32)x.t.N, sep = x.t.sep;
+    Timer t_all(st), t_sa(st), t_lcp(st);
+    t_all.start();
+    t_sa.start();
+    // ---- 1: SA and T (T holds n + 1 cells: it receives the max-scan of step 4) ----
+    DevBuf<u32> SA(n, st), T((u64)n + 1, st), a((u64)n + 1, st), flag(1, st);
+    {
+        DevBuf<u32> len(N, st), off((u64)N + 1, st);
+        const bool force_walk = (c->flags & GRLGPU_FLAG_FORCE_WALK) != 0, force_jump = (c->flags & GRLGPU_FLAG_FORCE_JUMP) != 0 && !force_walk;
+        bool walk = !force_jump && (force_walk || !x.doc_ready);  // once built, the locate table answers
+        if (walk) {  // a walk from row k ends within n steps: the bound n never overflows
+            const u64 B = force_walk ? n : inv_walk_bound(n);
+            flag.zero();
+            GRL_LAUNCH("inv_walk_count", (u64)N * 4 + (u64)(n - N) * 32, inv_walk_count_kernel, grid_for(N, INV_THREADS), INV_THREADS, 0, st, x.t.E.p, (const u32*)nullptr, N, sep,
+                       (u32)B, len.p, flag.p);
+            walk = d2h_scalar(flag.p, st) == 0;
+        }
+        info->path = walk ? 0 : 1;
+        if (walk) {
+            exclusive_scan<u32, u32>(len.p, off.p, N, off.p + N, st);
+            if ((u64)d2h_scalar(off.p + N, st) + N != n) throw Error(GRLGPU_ERR_ILL_FORMED, "lcp: the strings do not cover the BWT (an LF cycle without separator)");
+            GRL_LAUNCH("fm_lcp_walk", (u64)N * 8 + (u64)n * (32 + 32 + 4), fm_lcp_walk_kernel, grid_for(N, INV_THREADS), INV_THREADS, 0, st, x.t.E.p, N, sep, len.p, off.p, SA.p, T.p);
+        } else {
+            if (!x.doc_ready) info->jump_rounds = fm_build_doc(x, flag.p, st, "lcp");
+            GRL_LAUNCH("fm_lcp_len", (u64)N * (8 + 4), fm_lcp_len_kernel, grid_for(N, INV_THREADS), INV_THREADS, 0, st, x.doc.p, N, len.p);
+            exclusive_scan<u32, u32>(len.p, off.p, N, off.p + N, st);
+            GRL_LAUNCH("fm_lcp_table", (u64)n * (8 + 8 + 4 + 32 + 32) + (u64)N * 32, fm_lcp_table_kernel, grid_for(n, INV_THREADS), INV_THREADS, 0, st, x.t.E.p, x.doc.p, n, N,
+                       sep, off.p, SA.p, T.p);
+        }
+    }
+    t_sa.stop();
+    t_lcp.start();
+    // ---- 2: irreducible rows; the separator rows' PLCP 0 into a ----
+    a.zero();
+    DevBuf<u32> bits(div_up(n, 32), st), rows;
+    GRL_LAUNCH("fm_lcp_flags", (u64)n * 8 + n / 8 + (u64)N * (4 + 32), fm_lcp_flags_kernel, grid_for(n, INV_THREADS), INV_THREADS, 0, st, x.t.E.p, SA.p, n, N, sep, bits.p, a.p);
+    BitmapCompactor bc;
+    const u64 n_irr = bc.count(bits.p, n, st);
+    rows.alloc(n_irr, st);
+    bc.write<u32>(nullptr, rows.p);
+    bits.release();
+    // ---- 3: one warp per irreducible row ----
+    DevBuf<u64> sum(1, st);
+    sum.zero();
+    if (n_irr) {
+        const u64 blocks = std::min<u64>(div_up(n_irr, INV_THREADS / 32), (u64)c->n_sm * (2048 / INV_THREADS));  // one wave of full SMs at most
+        // bytes known only from the LCE sum read back below: added to this launch's record then
+        GRL_LAUNCH("fm_lcp_lce", 0, fm_lcp_lce_kernel, (unsigned)blocks, INV_THREADS, 0, st, rows.p, n_irr, SA.p, T.p, n, sep, a.p, sum.p);
+    }
+    const u64 sum_irr = d2h_scalar(sum.p, st);
+    // per row its index, two SA gathers, and per 32-cell step two 128 B segments of T; the a store
+    if (n_irr && g_prof && g_prof->timing && !g_prof->pending.empty()) g_prof->pending.back().bytes = n_irr * (4 + 2 * 32 + 32) + (sum_irr / 32 + n_irr) * 2 * 128;
+    info->n_irreducible = n_irr;
+    info->sum_irreducible = sum_irr;
+    rows.release();
+    // ---- 4: inclusive max over text positions: T[i + 1] = max(a[0 .. i]) = PLCP[i] + i ----
+    exclusive_scan<u32, u32, ScanMax>(a.p, T.p, (u64)n + 1, (u32*)nullptr, st);
+    // ---- 5: back to rows, into a ----
+    GRL_LAUNCH("fm_lcp_gather", (u64)n * (4 + 4) + (u64)(n - N) * 32, fm_lcp_gather_kernel, grid_for(n, INV_THREADS), INV_THREADS, 0, st, SA.p, T.p, n, N, a.p);
+    t_lcp.stop();
+    GRL_CUDA(cudaMemcpyAsync(lcp, a.p, (u64)n * 4, cudaMemcpyDeviceToHost, st));
+    t_all.stop();
+    info->sa_ms = t_sa.ms();
+    info->lcp_ms = t_lcp.ms();
+    info->device_ms = t_all.ms();  // waits for the copy
 }

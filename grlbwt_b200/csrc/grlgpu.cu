@@ -1735,6 +1735,17 @@ int grlgpu_fm_extract(grlgpu_ctx* ctx, const uint32_t* str_id, const uint32_t* f
     return guarded(ctx, [&] { fm_extract(ctx, str_id, from, len, (u32)n_req, cell_bytes, out_off, out, cap_cells, info); });
 }
 
+int grlgpu_fm_lcp(grlgpu_ctx* ctx, uint32_t* lcp, uint64_t cap, grlgpu_fm_lcp_t* info) {
+    if (!ctx || !info) return GRLGPU_ERR_ARG;
+    memset(info, 0, sizeof(*info));
+    if (!ctx->fm) return GRLGPU_ERR_STATE;
+    const u64 n = ctx->fm->t.n;
+    info->n = n;
+    if (n && (!lcp || cap < n)) return GRLGPU_ERR_ARG;
+    if (n == 0) return GRLGPU_OK;
+    return guarded(ctx, [&] { fm_lcp(ctx, lcp, info); });
+}
+
 int grlgpu_fm_drop(grlgpu_ctx* ctx) {
     if (!ctx) return GRLGPU_ERR_ARG;
     return guarded(ctx, [&] { ctx->fm.reset(); });

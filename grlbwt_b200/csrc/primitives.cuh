@@ -2,17 +2,65 @@
 // LSD radix sort of (u64 or u32 key, u32 value) pairs and its one-digit partition, max-reduction.
 // All are plain multi-kernel formulations (no inter-CTA spin waits), HBM-bound, grid sized from the data.
 #pragma once
+#include <type_traits>
 #include "util.cuh"
 
 namespace grl {
 
 // ------------------------------------------------------------------------------------------------
-// Exclusive scan: out[i] = sum_{j<i} in[j]  (TOut accumulates). Works in place (in == out).
+// Exclusive scan: out[i] = op_{j<i} in[j]  (TOut accumulates; op is the sum unless Op says otherwise). Works in place (in == out).
 // ------------------------------------------------------------------------------------------------
 constexpr int SCAN_THREADS = 256;
 constexpr int SCAN_ITEMS = 8;
 constexpr int SCAN_TILE = SCAN_THREADS * SCAN_ITEMS;
 
+// scan operators: associative, with identity 0 on the unsigned types they are used with
+struct ScanSum {
+    template <class T>
+    __device__ __forceinline__ static T apply(T a, T b) { return a + b; }
+};
+struct ScanMax {
+    template <class T>
+    __device__ __forceinline__ static T apply(T a, T b) { return a > b ? a : b; }
+};
+template <class Op, class T>
+__device__ __forceinline__ T warp_inclusive_op(T v) {
+    const u32 l = lane_id();
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const T x = __shfl_up_sync(0xffffffffu, v, o);
+        if (l >= (u32)o) v = Op::apply(v, x);
+    }
+    return v;
+}
+// block_exclusive_sum (util.cuh) for any scan operator: the sum keeps its own code; other operators take the exclusive prefix of a
+// lane from its neighbour's inclusive one, since they cannot subtract
+template <class Op, class T>
+__device__ __forceinline__ T block_exclusive_op(T v, T* smem, T& total) {
+    if constexpr (std::is_same<Op, ScanSum>::value) {
+        return block_exclusive_sum<T>(v, smem, total);
+    } else {
+        const u32 l = lane_id(), w = threadIdx.x >> 5, nw = (blockDim.x + 31) >> 5;
+        const T inc = warp_inclusive_op<Op>(v);
+        T ex = __shfl_up_sync(0xffffffffu, inc, 1);
+        if (l == 0) ex = T(0);
+        if (l == 31) smem[w] = inc;
+        __syncthreads();
+        if (w == 0) {
+            const T x = l < nw ? smem[l] : T(0);
+            const T xi = warp_inclusive_op<Op>(x);
+            T xe = __shfl_up_sync(0xffffffffu, xi, 1);
+            if (l == 0) xe = T(0);
+            smem[l] = xe;  // exclusive prefix of warp totals
+            if (l == 31) smem[32] = xi;
+        }
+        __syncthreads();
+        const T res = Op::apply(smem[w], ex);
+        total = smem[32];
+        __syncthreads();
+        return res;
+    }
+}
 // a thread's SCAN_ITEMS consecutive items move as 16-byte vectors when the whole run exists and the array is 16-byte aligned
 template <class T>
 __device__ __forceinline__ void scan_load(const T* in, u64 base, u64 n, bool vec, T (&v)[SCAN_ITEMS]) {
@@ -47,7 +95,7 @@ __device__ __forceinline__ void scan_store(T* out, u64 base, u64 n, bool vec, co
     }
 }
 
-template <class TIn, class TOut>
+template <class TIn, class TOut, class Op = ScanSum>
 __global__ void __launch_bounds__(SCAN_THREADS) scan_tile_sums_kernel(const TIn* __restrict__ in, TOut* __restrict__ partial, u64 n, bool vec) {
     __shared__ TOut sm[33];
     const u64 base = (u64)blockIdx.x * SCAN_TILE + (u64)threadIdx.x * SCAN_ITEMS;
@@ -55,14 +103,14 @@ __global__ void __launch_bounds__(SCAN_THREADS) scan_tile_sums_kernel(const TIn*
     scan_load<TIn>(in, base, n, vec, x);
     TOut s = 0;
 #pragma unroll
-    for (int i = 0; i < SCAN_ITEMS; i++) s += (TOut)x[i];
+    for (int i = 0; i < SCAN_ITEMS; i++) s = Op::apply(s, (TOut)x[i]);
     TOut tot;
-    block_exclusive_sum<TOut>(s, sm, tot);
+    block_exclusive_op<Op, TOut>(s, sm, tot);
     if (threadIdx.x == 0) partial[blockIdx.x] = tot;
 }
 
 // single block scans a short array (n <= any size, loops tile by tile), writes the grand total
-template <class TIn, class TOut>
+template <class TIn, class TOut, class Op = ScanSum>
 __global__ void __launch_bounds__(SCAN_THREADS) scan_single_block_kernel(const TIn* in, TOut* out, u64 n, TOut* total) {
     __shared__ TOut sm[33];
     TOut carry = 0;
@@ -73,21 +121,21 @@ __global__ void __launch_bounds__(SCAN_THREADS) scan_single_block_kernel(const T
 #pragma unroll
         for (int i = 0; i < SCAN_ITEMS; i++) {
             v[i] = (base + i < n) ? (TOut)in[base + i] : TOut(0);
-            s += v[i];
+            s = Op::apply(s, v[i]);
         }
         TOut tot;
-        TOut ex = block_exclusive_sum<TOut>(s, sm, tot) + carry;
+        TOut ex = Op::apply(block_exclusive_op<Op, TOut>(s, sm, tot), carry);
 #pragma unroll
         for (int i = 0; i < SCAN_ITEMS; i++) {
             if (base + i < n) out[base + i] = ex;
-            ex += v[i];
+            ex = Op::apply(ex, v[i]);
         }
-        carry += tot;
+        carry = Op::apply(carry, tot);
     }
     if (threadIdx.x == 0 && total) *total = carry;
 }
 
-template <class TIn, class TOut>
+template <class TIn, class TOut, class Op = ScanSum>
 __global__ void __launch_bounds__(SCAN_THREADS) scan_apply_kernel(const TIn* in, TOut* out, const TOut* __restrict__ tile_prefix, u64 n, bool vec) {
     __shared__ TOut sm[33];
     const u64 base = (u64)blockIdx.x * SCAN_TILE + (u64)threadIdx.x * SCAN_ITEMS;
@@ -95,31 +143,31 @@ __global__ void __launch_bounds__(SCAN_THREADS) scan_apply_kernel(const TIn* in,
     scan_load<TIn>(in, base, n, vec, x);
     TOut s = 0;
 #pragma unroll
-    for (int i = 0; i < SCAN_ITEMS; i++) s += (TOut)x[i];
+    for (int i = 0; i < SCAN_ITEMS; i++) s = Op::apply(s, (TOut)x[i]);
     TOut tot;
-    TOut ex = block_exclusive_sum<TOut>(s, sm, tot) + tile_prefix[blockIdx.x];
+    TOut ex = Op::apply(block_exclusive_op<Op, TOut>(s, sm, tot), tile_prefix[blockIdx.x]);
     TOut v[SCAN_ITEMS];
 #pragma unroll
     for (int i = 0; i < SCAN_ITEMS; i++) {
         v[i] = ex;
-        ex += (TOut)x[i];
+        ex = Op::apply(ex, (TOut)x[i]);
     }
     scan_store<TOut>(out, base, n, vec, v);
 }
 
-// total_dev (optional, device pointer) receives the sum of all inputs.
-template <class TIn, class TOut>
+// total_dev (optional, device pointer) receives the op of all inputs (the sum, or with ScanMax the maximum).
+template <class TIn, class TOut, class Op = ScanSum>
 void exclusive_scan(const TIn* in, TOut* out, u64 n, TOut* total_dev, cudaStream_t st) {
     if (n <= (u64)SCAN_TILE * 4) {
-        GRL_LAUNCH("scan_single_block", n * (sizeof(TIn) + sizeof(TOut)), (scan_single_block_kernel<TIn, TOut>), 1, SCAN_THREADS, 0, st, in, out, n, total_dev);
+        GRL_LAUNCH("scan_single_block", n * (sizeof(TIn) + sizeof(TOut)), (scan_single_block_kernel<TIn, TOut, Op>), 1, SCAN_THREADS, 0, st, in, out, n, total_dev);
         return;
     }
     const u64 tiles = div_up(n, SCAN_TILE);
     DevBuf<TOut> partial(tiles, st);
     const bool vec = (((uintptr_t)in | (uintptr_t)out) & 15) == 0;
-    GRL_LAUNCH("scan_tile_sums", n * sizeof(TIn), (scan_tile_sums_kernel<TIn, TOut>), (unsigned)tiles, SCAN_THREADS, 0, st, in, partial.p, n, vec);
-    exclusive_scan<TOut, TOut>(partial.p, partial.p, tiles, total_dev, st);
-    GRL_LAUNCH("scan_apply", n * (sizeof(TIn) + sizeof(TOut)), (scan_apply_kernel<TIn, TOut>), (unsigned)tiles, SCAN_THREADS, 0, st, in, out, partial.p, n, vec);
+    GRL_LAUNCH("scan_tile_sums", n * sizeof(TIn), (scan_tile_sums_kernel<TIn, TOut, Op>), (unsigned)tiles, SCAN_THREADS, 0, st, in, partial.p, n, vec);
+    exclusive_scan<TOut, TOut, Op>(partial.p, partial.p, tiles, total_dev, st);
+    GRL_LAUNCH("scan_apply", n * (sizeof(TIn) + sizeof(TOut)), (scan_apply_kernel<TIn, TOut, Op>), (unsigned)tiles, SCAN_THREADS, 0, st, in, out, partial.p, n, vec);
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -202,6 +202,57 @@ struct RlBwt {
         std::reverse(s.begin(), s.end());
         return s;
     }
+    // ---- LCP (fm_lcp) ----
+    // SA of every row and the text T (each string followed by the separator, strings in order): string k is walked by LF from
+    // row k (position L_k) down to position 0. A run list that is not a BWT leaves rows on no string's walk.
+    void sa_and_text(std::vector<uint32_t>& SA, std::vector<uint64_t>& T) const {
+        if (n >= 0xfffffff0ull) throw std::runtime_error("the BWT has 2^32 symbols or more (LCP values are written as 32-bit)");
+        SA.assign(n, 0);
+        T.assign(n, 0);
+        std::vector<uint64_t> F(runs.size());  // lf() with C[c] + before[k] looked up once per run
+        for (size_t q = 0; q < runs.size(); q++) F[q] = C.at(runs.sym[q]) + before[q];
+        const auto step = [&](uint64_t i) -> std::pair<uint64_t, uint64_t> {
+            const size_t q = (size_t)(std::upper_bound(start.begin(), start.end(), i) - start.begin()) - 1;
+            return {runs.sym[q], F[q] + (i - start[q])};
+        };
+        std::vector<uint64_t> rows, syms;
+        uint64_t o = 0;
+        for (uint64_t k = 0; k < n_strings; k++) {
+            rows.assign(1, k);
+            syms.clear();
+            for (auto e = step(k); e.first != sep; e = step(e.second)) {  // at most n steps: the LF cycle of row k holds a separator row
+                syms.push_back(e.first);
+                rows.push_back(e.second);
+                if (o + rows.size() > n) throw std::runtime_error("the file is ill formed (the strings do not cover the BWT)");
+            }
+            const uint64_t L = syms.size();
+            for (uint64_t t = 0; t <= L; t++) SA[rows[t]] = (uint32_t)(o + L - t);  // rows[t] is at position L - t
+            for (uint64_t t = 0; t < L; t++) T[o + L - 1 - t] = syms[t];
+            T[o + L] = sep;
+            o += L + 1;
+        }
+        if (o != n) throw std::runtime_error("the file is ill formed (the strings do not cover the BWT: an LF cycle without separator)");
+    }
+    // LCP of every row: Kärkkäinen's Phi algorithm on the text, a separator never matching (itself included)
+    std::vector<uint32_t> lcp() const {
+        std::vector<uint32_t> SA, P;
+        std::vector<uint64_t> T;
+        sa_and_text(SA, T);
+        P.assign(n, 0);
+        for (uint64_t j = 1; j < n; j++) P[SA[j]] = SA[j - 1];  // Phi; position SA[0] holds a separator and keeps 0
+        uint64_t l = 0;
+        for (uint64_t i = 0; i < n; i++) {  // P[i] becomes PLCP[i]; l grows by at most n in total and drops by one per position
+            if (T[i] == sep) { P[i] = 0; l = 0; continue; }
+            const uint64_t q = P[i];
+            while (T[i + l] == T[q + l] && T[i + l] != sep) l++;  // both strings end in a separator
+            P[i] = (uint32_t)l;
+            if (l) l--;
+        }
+        std::vector<uint32_t> out(n);
+        for (uint64_t j = 0; j < n; j++) out[j] = j < n_strings ? 0 : P[SA[j]];
+        return out;
+    }
+
     // the cells [from, e) of S_k[from .. e) in a string of length L: e = min(from + len, L) without overflow, empty when from >= L
     static std::pair<uint64_t, uint64_t> clamp(uint64_t L, uint64_t from, uint64_t len) {
         if (from >= L) return {0, 0};

@@ -275,6 +275,26 @@ typedef struct {
 int grlgpu_fm_extract(grlgpu_ctx* ctx, const uint32_t* str_id, const uint32_t* from, const uint32_t* len, uint64_t n_req,
                       int cell_bytes, uint64_t* out_off /* n_req + 1 */, void* out, uint64_t cap_cells, grlgpu_fm_extract_t* info);
 
+/* LCP array of the loaded index (the host tool fm_lcp is the general path and writes the same values). Row j's suffix is
+ * S_k[p .. L_k) followed by $_k, where (k, p) is the row's locate entry; rows j < N are the $_k rows. lcp[0] = 0 and, for j >= 1,
+ * lcp[j] = the number of leading cells shared by the suffixes of rows j - 1 and j, where a separator never matches (itself
+ * included): rows j < N have 0, no value crosses a string's end, and the values do not depend on how separators are tie-broken.
+ *   grlgpu_fm_lcp  writes n values in row order. SA and the text come from a walk per string (the count pass of grlgpu_fm_extract,
+ *                  bound B = max(4096, n / 2048)) or from the locate table of grlgpu_fm_locate: the table answers when it exists, when a
+ *                  string is longer than B (built here by pointer jumping, then kept for every later call) or under
+ *                  GRLGPU_FLAG_FORCE_JUMP; GRLGPU_FLAG_FORCE_WALK walks with bound n. Only the rows that start a BWT run or hold the
+ *                  separator (irreducible) compare text; every other row follows from its LF successor.
+ * GRLGPU_ERR_ARG: a null lcp with n > 0, or cap < n (info->n then holds n, nothing is written). GRLGPU_ERR_STATE: no index loaded.
+ * GRLGPU_ERR_ILL_FORMED: the run list is not a BWT (its LF has a cycle without separator), through either path. */
+typedef struct {
+    uint64_t n;                 /* rows: entries written (or needed, when cap is too small) */
+    uint64_t n_irreducible;     /* rows whose LCP was found by comparing cells */
+    uint64_t sum_irreducible;   /* sum of those rows' LCP values */
+    uint32_t path, jump_rounds; /* 0 walk per string, 1 the locate table; rounds when this call built the table, else 0 */
+    float device_ms, sa_ms, lcp_ms; /* CUDA events: whole call incl. the copy out / SA + text / irreducible rows, scan and gather */
+} grlgpu_fm_lcp_t;
+int grlgpu_fm_lcp(grlgpu_ctx* ctx, uint32_t* lcp /* n */, uint64_t cap, grlgpu_fm_lcp_t* info);
+
 /* digest of the last round's level artefacts, computed on the device before they are fetched: four sums mod 2^64
  * {rules weighted by rank, hocc marks weighted by rank, sum of the preliminary-BWT run lengths, runs weighted by symbol}.
  * The sums of the per-rank slices of a multi-GPU level add up to the single-GPU value, so bench.py can check that 1, 2,
